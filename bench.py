@@ -18,6 +18,10 @@ candidate noise in pinned HOST memory (H2D inside the timed region) and the
 scores + winning noise read back (D2H).  `roofline` is the tcgen05 tap-GEMM
 family, timed launch by launch with CUDA events; `cpu_baseline` is the CPU port
 of the reference path (oracle/) on this box's host cores.
+
+`--dump-outputs DIR` writes what the last timed step returned (the winning noise, its score, every candidate's
+score and the winner's index) as DIR/<name>.npy.  The weights, candidates and step noise are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -34,6 +38,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: the benchmark writes nothing into it
 
 import torch  # noqa: E402
 
@@ -319,6 +324,9 @@ def run_ours(args):
             best_noise, best_score = step_resident()
         e1.record()
         barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, best_noise=best_noise, best_score=best_score, scores=rs.last_scores,
+                     best_index=rs.last_index)
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -400,6 +408,15 @@ def run_ours(args):
 
 
 PRECISION = "16bit"     # --precision: "16bit" (tensor-core path, the headline) or "fp32" (CUDA-core parity path)
+
+
+def dump_outputs(out_dir, **values):
+    """One .npy per value: tensors keep float32, Python scalars (score, index) are stored as float64."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in values.items():
+        a = v.detach().cpu().numpy().astype(np.float32) if torch.is_tensor(v) else np.asarray(v, dtype=np.float64)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def build_workload(key, dev):
@@ -561,7 +578,7 @@ def profile_tapgemm(plan, dev, pk):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3, help="timed searches (at least 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="A", choices=sorted(WORKLOADS), help="A = BASELINE.json configs[1] (default)")
@@ -575,7 +592,13 @@ def main():
                     help="skip the one-search measurements of workloads C and E appended to the default line")
     ap.add_argument("--precision", default="16bit", choices=["16bit", "fp32"],
                     help="16bit = tensor-core path (default, the headline number); fp32 = CUDA-core parity path")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed search's results as DIR/<name>.npy (our arm only)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     global PRECISION
     PRECISION = args.precision
     if args.candidates is None:
