@@ -89,6 +89,39 @@ int its_philox_normal(float* out, const float* base, int32_t base_bcast,
 int its_step_advance(int32_t* t_dev, int32_t delta, void* stream);
 
 /* ------------------------------------------------------------------------
+ * its_ddpm_step with the x0 prediction of search over paths (Ma et al.): the same
+ * state update as its_ddpm_step (same kernel body, same bits), and, when x0_out
+ * != NULL, from the same mixed eps and the input state x_t:
+ *   x0_out = clip(r1[t]*x_t - r2[t]*eps, -1, 1)            (NaN stays NaN)
+ * i.e. torch.clip(sqrt(1/abar_t)*x_t - sqrt(1/abar_t - 1)*eps, -1, 1) in fp32 with
+ * separately rounded mul / mul / sub.  x0_coef is a device table [T][2] of fp32
+ * {sqrt(1/abar), sqrt(1/abar - 1)} formed in fp64 from abar = cumprod(1 - betas)
+ * (Diffusion.py:57-60).  The candidate base is read from *cand_dev (device int64),
+ * so one captured step graph serves every round and chunk of a search.
+ * ---------------------------------------------------------------------- */
+int its_ddpm_step_x0(float* x, float* x0_out, const float* eps_c,
+                     const float* eps_u, const float* noise,
+                     int64_t noise_t_stride, int64_t n_img, int64_t n_per_img,
+                     const float* coef, const float* x0_coef,
+                     const int32_t* t_dev, double w, uint64_t seed,
+                     const int64_t* cand_dev, int32_t* nan_flag,
+                     int32_t clip_last, void* stream);
+
+/* Children of one search-over-paths round, q(x_s' | x_s) applied to survivors:
+ *   out[i] = a * x[parent[(child0 + i) / m]] + b * z[i],   i < n_child
+ * torch: a * x[parents] + b * z  (fp32, separately rounded mul / mul / add).
+ * x is [n_parent][n_per], parent a device int32 array of n_sel survivor indices
+ * (its_topk_first's idx_out as is), m children per survivor.  z == NULL draws z
+ * from Philox (seed, cand_id0 + child0 + i, tag), the stream its_philox_normal
+ * gives unit cand_id0 + child0 + i; otherwise z is [n_child][n_per].  A parent
+ * index outside [0, n_parent) yields a NaN child.                           */
+int its_path_expand(float* out, const float* x, const int32_t* parent,
+                    int32_t n_sel, int32_t m, int64_t child0, int64_t n_child,
+                    int64_t n_parent, int64_t n_per, float a, float b,
+                    const float* z, uint64_t seed, int64_t cand_id0,
+                    int32_t tag, void* stream);
+
+/* ------------------------------------------------------------------------
  * Sinusoidal time embedding  emb[b,2i]=sin(t*f_i), emb[b,2i+1]=cos(t*f_i)
  * (Model.py:76-88; the table form ModelCondition.py:27-34 gives the same
  * values for integer t).  t comes from t_idx[b] (int64, host-API path) or, when

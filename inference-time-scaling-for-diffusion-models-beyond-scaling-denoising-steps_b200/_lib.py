@@ -22,7 +22,7 @@ SYMBOLS = [
     "its_group_norm_apply", "its_conv_stats_parts", "its_set_pdl", "its_attention_fused", "its_head_patches",
     "its_attention_flash", "its_attention_group", "its_conv_gn_sync_words",
     "its_f32_nchw_to_nhwc", "its_f32_conv2d", "its_f32_group_norm", "its_f32_attention",
-    "its_topk_first",
+    "its_topk_first", "its_ddpm_step_x0", "its_path_expand",
 ]
 
 
@@ -84,6 +84,8 @@ def lib() -> C.CDLL:
     L.its_abi_sizeof.argtypes = [i32]
     L.its_set_pdl.argtypes = [i32]
     L.its_ddpm_step.argtypes = [vp, vp, vp, vp, i64, i64, i64, vp, vp, f64, u64, i64, vp, i32, vp]
+    L.its_ddpm_step_x0.argtypes = [vp, vp, vp, vp, vp, i64, i64, i64, vp, vp, vp, f64, u64, vp, vp, i32, vp]
+    L.its_path_expand.argtypes = [vp, vp, vp, i32, i32, i64, i64, i64, i64, f32, f32, vp, u64, i64, i32, vp]
     L.its_philox_normal.argtypes = [vp, vp, i32, f32, i64, i64, u64, i64, i32, vp]
     L.its_step_advance.argtypes = [vp, i32, vp]
     L.its_time_embed.argtypes = [vp, vp, vp, vp, i32, i32, vp]

@@ -54,6 +54,9 @@ class SamplerBase(nn.Module):
         self.use_cuda_graph = True
         self._coef_cache: Dict = {}
         self._traj: Dict = {}
+        self._x0_cache: Dict = {}
+        self._seg: Dict = {}
+        self.segment_captures = 0   # step graphs captured by `segment` (one per plan and noise mode)
 
     # ----------------------------------------------------------- public seam --
     def predict_xt_prev_mean_from_eps(self, x_t, t, eps):
@@ -84,6 +87,16 @@ class SamplerBase(nn.Module):
             tab = torch.stack([self.coeff1.float().to(dev), self.coeff2.float().to(dev), torch.sqrt(var),
                                torch.zeros_like(var)], dim=1).contiguous()
             self._coef_cache = {key: tab}
+        return tab
+
+    def _x0_table(self, dev) -> torch.Tensor:
+        """[T][2] fp32 {sqrt(1/abar), sqrt(1/abar - 1)}, formed in fp64 from abar = cumprod(1 - betas)."""
+        key = (str(dev), self.T, self.betas.data_ptr())
+        tab = self._x0_cache.get(key)
+        if tab is None:
+            abar = torch.cumprod(1. - self.betas.cpu(), dim=0)     # sequential fp64 product, as _init_schedule
+            tab = torch.stack([torch.sqrt(1. / abar), torch.sqrt(1. / abar - 1.)], dim=1).float().to(dev).contiguous()
+            self._x0_cache = {key: tab}
         return tab
 
     def _sample(self, x_T: torch.Tensor, labels: Optional[torch.Tensor], *, noise=None, seed=None,
@@ -187,3 +200,101 @@ class SamplerBase(nn.Module):
             raise AssertionError("nan in tensor.")
         self.last_launches_per_step = plan.n_launches + 2
         return plan.x_in.clone()
+
+    def segment(self, x: torch.Tensor, labels: Optional[torch.Tensor] = None, *, t_start: int, t_stop: int,
+                seed: int, cand_id0: int = 0, noise: Optional[torch.Tensor] = None, x0: bool = False,
+                check_nan: bool = True) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+        """Steps time_step = t_start ... t_stop of the ancestral loop from state `x` (the x_t that step t_start
+        takes), as `forward(x, t_start=..., t_stop=...)` computes them, bit for bit; the state after step 0 is
+        clipped.  Returns (state after step t_stop, x0 prediction of step t_stop or None).  With `x0` the last
+        step also yields clip(sqrt(1/abar)*x_t - sqrt(1/abar - 1)*eps, -1, 1) from that step's (guidance-mixed)
+        eps: no extra UNet evaluation.  The candidate base `cand_id0` is written to device memory before the
+        steps run, so the captured step graph is kept per (plan, noise mode, x0) and replayed for every call
+        with the same seed and guidance weight (`segment_captures` counts the captures)."""
+        _lib.require_cuda()
+        L = _lib.lib()
+        if x.device.type != "cuda":
+            raise RuntimeError("its_b200 samplers run on CUDA only (no CPU fallback)")
+        if not (0 <= int(t_stop) <= int(t_start) < self.T):
+            raise ValueError(f"segment needs 0 <= t_stop <= t_start < T={self.T}; got t_start={t_start} t_stop={t_stop}")
+        with torch.cuda.device(x.device):
+            return self._segment_on_device(L, x, labels, int(t_start), int(t_stop), int(seed), int(cand_id0),
+                                           noise, bool(x0), check_nan)
+
+    def _segment_on_device(self, L, x, labels, first, t_stop, seed, cand_id0, noise, want_x0, check_nan):
+        net = self._unet()
+        if net.head.weight.device != x.device:
+            raise RuntimeError(f"x lives on {x.device} but the UNet on {net.head.weight.device}")
+        if self.guided:
+            if getattr(net, "is_conditional", False) and self.T > net.time_embedding.timembedding[0].num_embeddings:
+                raise IndexError("index out of range in self")
+            net.check_indices(None, labels)
+        B, Cc, H, W = x.shape
+        plan = net.plan(2 * B if self.guided else B, H, W, n_img_in=B, uniform_t=True, impl=getattr(net, "impl", None))
+        coef = self._coef_table(x.device)
+        x0tab = self._x0_table(x.device)
+        n_per = Cc * H * W
+        key = (id(plan), noise is not None, tuple(noise.shape) if noise is not None else None, want_x0)
+        tr = self._seg.get(key)
+        if tr is not None and tr.plan is not plan:
+            tr = None             # the plan was rebuilt: never replay its graph
+        if tr is None:
+            tr = _Trajectory()
+            tr.plan = plan
+            tr.nan_flag = torch.zeros(1, dtype=torch.int32, device=x.device)
+            tr.cand_dev = torch.zeros(1, dtype=torch.int64, device=x.device)
+            tr.x0_buf = torch.empty_like(x, dtype=torch.float32) if want_x0 else None
+            tr.seed_args = None
+            if noise is not None:
+                tr.noise_buf = torch.empty(noise.shape, dtype=torch.float32, device=x.device)
+            live = list(net._plans.values())   # drop graphs of plans the net has since rebuilt
+            self._seg = {k: v for k, v in self._seg.items() if any(v.plan is p for p in live)}
+            self._seg[key] = tr
+        with torch.no_grad():
+            plan.x_in.copy_(x)
+            plan.t_dev.fill_(first)
+            tr.cand_dev.fill_(cand_id0)
+            tr.nan_flag.zero_()
+            if self.guided:
+                lab = labels.reshape(-1).to(device=x.device, dtype=torch.int64)
+                plan.labels.copy_(torch.cat([lab, torch.zeros_like(lab)]))
+                plan.run_label_ops()
+            if noise is not None:
+                if noise.shape[0] != self.T or tuple(noise.shape[1:]) != tuple(x.shape):
+                    raise ValueError("injected noise must be [T, *x.shape]; entry t is used at time_step t")
+                tr.noise_buf.copy_(noise)
+        eps_c = plan.eps.data_ptr()
+        eps_u = plan.eps[B:].data_ptr() if self.guided else None
+        w = float(getattr(self, "w", 0.0))
+        noise_ptr = tr.noise_buf.data_ptr() if noise is not None else None
+        stride = B * n_per if noise is not None else 0
+        x0_ptr = tr.x0_buf.data_ptr() if want_x0 else None
+
+        def step():
+            plan.run()
+            s = _lib.stream_ptr()
+            _lib.check(L.its_ddpm_step_x0(plan.x_in.data_ptr(), x0_ptr, eps_c, eps_u, noise_ptr, stride, B, n_per,
+                                          coef.data_ptr(), x0tab.data_ptr(), plan.t_dev.data_ptr(), w, seed,
+                                          tr.cand_dev.data_ptr(), tr.nan_flag.data_ptr(), 1, s), "its_ddpm_step_x0")
+            _lib.check(L.its_step_advance(plan.t_dev.data_ptr(), -1, s), "its_step_advance")
+
+        t_cur = first
+        graph_key = (None, w) if noise is not None else (seed, w)
+        if self.use_cuda_graph and (tr.graph is None or tr.seed_args != graph_key) and first > t_stop:
+            step()                # a real step, and the lazy kernel attribute setup outside of capture
+            t_cur -= 1
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):
+                step()
+            tr.graph, tr.seed_args = g, graph_key
+            self.segment_captures += 1
+        graph_ok = self.use_cuda_graph and tr.graph is not None and tr.seed_args == graph_key
+        while t_cur >= t_stop:
+            if graph_ok:
+                tr.graph.replay()
+            else:
+                step()
+            t_cur -= 1
+        if check_nan and int(tr.nan_flag.item()) != 0:
+            raise AssertionError("nan in tensor.")
+        return plan.x_in.clone(), (tr.x0_buf.clone() if want_x0 else None)

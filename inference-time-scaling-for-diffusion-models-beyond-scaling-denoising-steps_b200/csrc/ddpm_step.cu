@@ -48,17 +48,34 @@ int set_error(int code, const char* fmt, ...) {
   return code;
 }
 
+// clip to [-1, 1] that keeps NaN (torch.clip semantics), so a diverged x0 prediction never ranks
+__device__ __forceinline__ float clip1_keep_nan(float v) { return v != v ? v : fminf(fmaxf(v, -1.f), 1.f); }
+
 // One thread handles 4 consecutive elements of one image (n_per_img % 4 == 0),
 // which is also one Philox counter.  Grid-stride over quads.
+// kX0 = false: its_ddpm_step (the trailing three arguments are unused).  kX0 = true: its_ddpm_step_x0 — the
+// candidate base is read from *cand_dev and, when x0_out != NULL, the x0 prediction of the same mixed eps,
+// clip(r1[t]*x - r2[t]*eps, -1, 1) with {r1, r2} = x0_coef[t], is written to x0_out.
+template <bool kX0>
 __global__ void __launch_bounds__(256) ddpm_step_kernel(
     float* __restrict__ x, const float* __restrict__ eps_c, const float* __restrict__ eps_u,
     const float* __restrict__ noise, long long noise_t_stride, long long n_img, long long quads_per_img,
     const float* __restrict__ coef, const int* __restrict__ t_dev, float w, float opw, uint64_t seed,
-    long long cand_id0, int* __restrict__ nan_flag, int clip_last) {
+    long long cand_id0, int* __restrict__ nan_flag, int clip_last, float* __restrict__ x0_out,
+    const float* __restrict__ x0_coef, const long long* __restrict__ cand_dev) {
   pdl_prologue();
   const int t = *t_dev;
   const float4 cf = *reinterpret_cast<const float4*>(coef + 4 * (long long)t);
   const float c1 = cf.x, c2 = cf.y, sigma = (t > 0) ? cf.z : 0.0f;
+  float r1 = 0.f, r2 = 0.f;
+  if constexpr (kX0) {
+    cand_id0 = *cand_dev;
+    if (x0_out != nullptr) {
+      const float2 r = *reinterpret_cast<const float2*>(x0_coef + 2 * (long long)t);
+      r1 = r.x;
+      r2 = r.y;
+    }
+  }
   const bool last = (t == 0) && clip_last;
   const long long total = n_img * quads_per_img;
   if (noise != nullptr) noise += (long long)t * noise_t_stride;
@@ -78,6 +95,16 @@ __global__ void __launch_bounds__(256) ddpm_step_kernel(
       e.y = __fsub_rn(__fmul_rn(opw, e.y), __fmul_rn(w, u.y));
       e.z = __fsub_rn(__fmul_rn(opw, e.z), __fmul_rn(w, u.z));
       e.w = __fsub_rn(__fmul_rn(opw, e.w), __fmul_rn(w, u.w));
+    }
+    if constexpr (kX0) {
+      if (x0_out != nullptr) {
+        float4 p;
+        p.x = clip1_keep_nan(__fsub_rn(__fmul_rn(r1, xv.x), __fmul_rn(r2, e.x)));
+        p.y = clip1_keep_nan(__fsub_rn(__fmul_rn(r1, xv.y), __fmul_rn(r2, e.y)));
+        p.z = clip1_keep_nan(__fsub_rn(__fmul_rn(r1, xv.z), __fmul_rn(r2, e.z)));
+        p.w = clip1_keep_nan(__fsub_rn(__fmul_rn(r1, xv.w), __fmul_rn(r2, e.w)));
+        reinterpret_cast<float4*>(x0_out)[q] = p;
+      }
     }
     float z[4] = {0.f, 0.f, 0.f, 0.f};
     if (t > 0) {
@@ -125,6 +152,42 @@ __global__ void __launch_bounds__(256) philox_normal_kernel(
   }
 }
 
+// Children of the path search: out[i] = a * x[parent[(child0 + i) / m]] + b * z[i], one float4 per thread,
+// separately rounded mul / mul / add.  z is injected or Philox (seed, cand_id0 + child0 + i, tag, quad), the
+// stream its_philox_normal gives unit cand_id0 + child0 + i.  An out-of-range parent index gives a NaN child.
+__global__ void __launch_bounds__(256) path_expand_kernel(
+    float* __restrict__ out, const float* __restrict__ x, const int* __restrict__ parent, int m, long long child0,
+    long long n_child, long long n_parent, long long quads_per, float a, float b, const float* __restrict__ z,
+    uint64_t seed, long long cand_id0, uint32_t tag) {
+  pdl_prologue();
+  const long long total = n_child * quads_per;
+  for (long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x; q < total;
+       q += (long long)gridDim.x * blockDim.x) {
+    const long long c = q / quads_per;
+    const uint32_t quad = (uint32_t)(q - c * quads_per);
+    const long long p = __ldg(parent + (child0 + c) / m);
+    float4 o;
+    if (p < 0 || p >= n_parent) {
+      o = make_float4(__int_as_float(0x7fffffff), __int_as_float(0x7fffffff), __int_as_float(0x7fffffff),
+                      __int_as_float(0x7fffffff));
+    } else {
+      const float4 xv = __ldg(reinterpret_cast<const float4*>(x) + p * quads_per + quad);
+      float zz[4];
+      if (z != nullptr) {
+        const float4 zv = __ldg(reinterpret_cast<const float4*>(z) + q);
+        zz[0] = zv.x; zz[1] = zv.y; zz[2] = zv.z; zz[3] = zv.w;
+      } else {
+        philox_normal4(seed, (uint64_t)(cand_id0 + child0 + c), tag, quad, zz);
+      }
+      o.x = __fadd_rn(__fmul_rn(a, xv.x), __fmul_rn(b, zz[0]));
+      o.y = __fadd_rn(__fmul_rn(a, xv.y), __fmul_rn(b, zz[1]));
+      o.z = __fadd_rn(__fmul_rn(a, xv.z), __fmul_rn(b, zz[2]));
+      o.w = __fadd_rn(__fmul_rn(a, xv.w), __fmul_rn(b, zz[3]));
+    }
+    reinterpret_cast<float4*>(out)[q] = o;
+  }
+}
+
 __global__ void step_advance_kernel(int* t_dev, int delta) {
   pdl_prologue();
   *t_dev += delta;
@@ -167,10 +230,45 @@ extern "C" int its_ddpm_step(float* x, const float* eps_c, const float* eps_u, c
               "its_ddpm_step: n_per_img=%lld must be a positive multiple of 4", (long long)n_per_img);
   ITS_REQUIRE(noise_t_stride % 4 == 0, "its_ddpm_step: noise_t_stride must be a multiple of 4");
   const long long quads = n_per_img / 4;
-  ITS_LAUNCH(its::ddpm_step_kernel, dim3(its::grid_for(n_img * quads, 256)), dim3(256), 0, its::as_stream(stream), 
+  ITS_LAUNCH(its::ddpm_step_kernel<false>, dim3(its::grid_for(n_img * quads, 256)), dim3(256), 0, its::as_stream(stream), 
       x, eps_c, eps_u, noise, noise_t_stride, n_img, quads, coef, t_dev, (float)w, (float)(1.0 + w), seed,
       cand_id0,
-      nan_flag, clip_last);
+      nan_flag, clip_last, (float*)nullptr, (const float*)nullptr, (const long long*)nullptr);
+  ITS_CHECK_LAUNCH();
+  return ITS_OK;
+}
+
+extern "C" int its_ddpm_step_x0(float* x, float* x0_out, const float* eps_c, const float* eps_u, const float* noise,
+                                int64_t noise_t_stride, int64_t n_img, int64_t n_per_img, const float* coef,
+                                const float* x0_coef, const int32_t* t_dev, double w, uint64_t seed,
+                                const int64_t* cand_dev, int32_t* nan_flag, int32_t clip_last, void* stream) {
+  ITS_REQUIRE(x && eps_c && coef && t_dev && cand_dev && nan_flag, "its_ddpm_step_x0: null pointer");
+  ITS_REQUIRE(x0_out == nullptr || x0_coef != nullptr, "its_ddpm_step_x0: null pointer (x0_coef with x0_out)");
+  ITS_REQUIRE(n_img > 0 && n_per_img > 0 && n_per_img % 4 == 0,
+              "its_ddpm_step_x0: n_per_img=%lld must be a positive multiple of 4", (long long)n_per_img);
+  ITS_REQUIRE(noise_t_stride % 4 == 0, "its_ddpm_step_x0: noise_t_stride must be a multiple of 4");
+  const long long quads = n_per_img / 4;
+  ITS_LAUNCH(its::ddpm_step_kernel<true>, dim3(its::grid_for(n_img * quads, 256)), dim3(256), 0,
+      its::as_stream(stream), x, eps_c, eps_u, noise, noise_t_stride, n_img, quads, coef, t_dev, (float)w,
+      (float)(1.0 + w), seed, (long long)0, nan_flag, clip_last, x0_out, x0_coef, (const long long*)cand_dev);
+  ITS_CHECK_LAUNCH();
+  return ITS_OK;
+}
+
+extern "C" int its_path_expand(float* out, const float* x, const int32_t* parent, int32_t n_sel, int32_t m,
+                               int64_t child0, int64_t n_child, int64_t n_parent, int64_t n_per, float a, float b,
+                               const float* z, uint64_t seed, int64_t cand_id0, int32_t tag, void* stream) {
+  ITS_REQUIRE(out && x && parent, "its_path_expand: null pointer");
+  ITS_REQUIRE(n_child > 0 && n_parent > 0 && n_per > 0 && n_per % 4 == 0,
+              "its_path_expand: n_child=%lld n_parent=%lld must be positive, n_per=%lld a positive multiple of 4",
+              (long long)n_child, (long long)n_parent, (long long)n_per);
+  ITS_REQUIRE(m >= 1 && n_sel >= 1 && child0 >= 0 && child0 + n_child <= (int64_t)n_sel * m,
+              "its_path_expand: children [%lld, %lld) exceed %d parents x %d children",
+              (long long)child0, (long long)(child0 + n_child), n_sel, m);
+  const long long quads = n_per / 4;
+  ITS_LAUNCH(its::path_expand_kernel, dim3(its::grid_for(n_child * quads, 256)), dim3(256), 0,
+      its::as_stream(stream), out, x, (const int*)parent, (int)m, (long long)child0, (long long)n_child,
+      (long long)n_parent, quads, a, b, z, seed, (long long)cand_id0, (uint32_t)tag);
   ITS_CHECK_LAUNCH();
   return ITS_OK;
 }

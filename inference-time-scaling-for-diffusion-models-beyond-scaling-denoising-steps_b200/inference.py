@@ -11,7 +11,8 @@ reference (SURVEY.md §8f rows 1 and 3), without Hydra.
     the sampler's step graph (`forward(..., t_start=a, t_stop=b)`), so tracking costs nothing between
     metric points.  Calculators are duck-typed (FID / IS / CLIP weights are third-party downloads the
     reference fetches at run time, SURVEY.md §8c): pass the reference's own objects, or None.
-  * run_search               — config-driven search (random / zero_order / path) with the kernel verifiers
+  * run_search               — config-driven search (random / zero_order / path / search_over_paths) with the
+                               kernel verifiers
   * save_image_grid          — torchvision.utils.save_image grid as the reference writes it (:621-628)
 
     python -m its_b200.inference config/inference_config.yaml T=1000 img_size=32 batch_size=64
@@ -275,10 +276,13 @@ def make_verifier(name: str):
 
 def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Optional[int] = None):
     """`search:` block of the config -> (best_noise, best_score, images of the best candidate).
-    Keys: algorithm (random | zero_order | path), verifier (oracle | self_supervised | aesthetic),
-    n_candidates / n_neighbors / n_iterations / lambda_radius / n_paths / injection_step / noise_scale
+    Keys: algorithm (random | zero_order | path | search_over_paths), verifier (oracle | self_supervised |
+    aesthetic), n_candidates / n_neighbors / n_iterations / lambda_radius / n_paths / injection_step / noise_scale
     (defaults: the reference constructors', search_algorithm.py:24,98-100,246-248), batch_size,
-    img_size.  With torch.distributed initialised the candidates are sharded over the ranks."""
+    img_size.  search_over_paths takes n_beams (4), n_children (4), start_step (800), delta_f (50) and
+    delta_b (100), and returns the winner's initial x_T with the images the search itself finished (the winner's
+    path is re-noised along the way: denoising its x_T again would not reproduce it).
+    With torch.distributed initialised the candidates are sharded over the ranks."""
     from .search import search_algorithm as S
     sc = dict(config.get("search") or {})
     algo = sc.get("algorithm", "random")
@@ -287,6 +291,13 @@ def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Op
     ver = make_verifier(sc.get("verifier", "oracle"))
     den = S.make_denoise_fn(sampler, labels, max_images=int(sc.get("max_images", 256)), seed=seed)
     dev = str(device)
+    if algo == "search_over_paths":
+        search = S.SearchOverPaths(n_beams=int(sc.get("n_beams", 4)), n_children=int(sc.get("n_children", 4)),
+                                   start_step=int(sc.get("start_step", 800)), delta_f=int(sc.get("delta_f", 50)),
+                                   delta_b=int(sc.get("delta_b", 100)))
+        images, score, _ = search.search(shape, den, ver.score, device=dev, verbose=False, seed=seed)
+        best = S.philox_normal((1,) + shape, search.last_seed, search.last_index, S.TAG_X_T, torch.device(device))[0]
+        return best, score, images
     if algo == "random":
         search = S.RandomSearch(n_candidates=int(sc.get("n_candidates", 4)))
         best, score = search.search(shape, den, ver.score, device=dev, verbose=False, seed=seed)
@@ -302,7 +313,7 @@ def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Op
                                   noise_scale=float(sc.get("noise_scale", 0.1)))
             best, score, _ = search.search(x0, den, ver.score, device=dev, verbose=False, seed=seed)
         else:
-            raise ValueError(f"search.algorithm {algo!r}: random | zero_order | path")
+            raise ValueError(f"search.algorithm {algo!r}: random | zero_order | path | search_over_paths")
     # the images of the winner: its own trajectory (the Philox stream of the candidate id it was scored under),
     # so that the returned images are the ones that produced the returned score
     images = None

@@ -21,12 +21,16 @@ the global best (:193-196), PathSearch is the reference's placeholder (perturb
 x_T, denoise fully, :307-316) unless `restart=True` is passed (opt-in extension:
 true mid-trajectory restart at `injection_step`).
 
+SearchOverPaths is not in the reference: it is the search over paths of Ma et al. (a beam of partial
+trajectories, re-noised and pruned by top-k on x0 predictions), in population mode only.
+
 GradientBasedSearch (:343-438) needs autograd through the whole trajectory: it is kept
 for arbitrary differentiable callables (callable mode only, the reference's loop); the
 kernel sampler is not differentiable and is refused with a clear error.
 """
 from __future__ import annotations
 
+import math
 from typing import Any, Callable, Dict, List, Optional, Sequence, Tuple
 
 import torch
@@ -38,6 +42,10 @@ from . import verifier as _ver
 TAG_X_T = X_T_TAG            # candidate x_T draws
 TAG_NEIGHBOR = X_T_TAG + 16  # + iteration
 TAG_PATH = X_T_TAG + 8
+TAG_FORWARD = X_T_TAG + 4    # SearchOverPaths re-noising draws, keyed by round and child
+# SearchOverPaths: image b of child c in round r (1-based; the initial paths are round 0) draws its step noise from
+# Philox candidate id r * ROUND_STRIDE + c * B + b
+ROUND_STRIDE = 1 << 40
 
 
 # ------------------------------------------------------------------ adapter --
@@ -86,9 +94,11 @@ class SamplerDenoiser:
         return self.denoise_candidates(noise.unsqueeze(0), i, labels=kwargs.get("labels"))[0]
 
     def denoise_candidates(self, cands: torch.Tensor, first_cand: int, *, labels=None,
-                           t_start: Optional[int] = None, seed: Optional[int] = None) -> torch.Tensor:
+                           t_start: Optional[int] = None, seed: Optional[int] = None, t_stop: int = 0,
+                           clip: bool = True) -> torch.Tensor:
         """cands [n, B, C, H, W] -> images [n, B, C, H, W]; candidate i is global
-        candidate first_cand + i (its Philox streams are keyed by that id)."""
+        candidate first_cand + i (its Philox streams are keyed by that id).  `t_stop` / `clip` end the loop
+        early as the sampler's own arguments do (the states step t_stop - 1 starts from)."""
         n, B = cands.shape[:2]
         guided = getattr(self.sampler, "guided", False)
         per_call = max(1, self.max_images // B)
@@ -98,6 +108,8 @@ class SamplerDenoiser:
             i1 = min(n, i0 + per_call)
             x = cands[i0:i1].reshape((i1 - i0) * B, *cands.shape[2:])
             kw: Dict[str, Any] = dict(seed=seed, cand_id0=(first_cand + i0) * B, t_start=t_start)
+            if t_stop or not clip:
+                kw.update(t_stop=t_stop, clip=clip)
             if self.step_noise is not None:
                 kw["noise"] = self.step_noise.repeat(1, i1 - i0, 1, 1, 1)
             if guided:
@@ -106,6 +118,31 @@ class SamplerDenoiser:
                 y = self.sampler(x, **kw)
             out[i0:i1] = y.view(i1 - i0, B, *cands.shape[2:])
         return out
+
+    def denoise_segment(self, states: torch.Tensor, first_cand: int, *, t_start: int, t_stop: int,
+                        cand_offset: int = 0, labels=None, seed: Optional[int] = None,
+                        x0: bool = True) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+        """states [n, B, C, H, W] at step t_start -> (states after step t_stop, x0 predictions of step t_stop or
+        None), in chunks of `max_images`.  Candidate i's per-step Philox streams are keyed by
+        cand_offset + (first_cand + i) * B + image; every chunk replays the sampler's one segment graph."""
+        n, B = states.shape[:2]
+        guided = getattr(self.sampler, "guided", False)
+        per_call = max(1, self.max_images // B)
+        out = torch.empty_like(states)
+        out_x0 = torch.empty_like(states) if x0 else None
+        seed = self.step_seed(seed)
+        for i0 in range(0, n, per_call):
+            i1 = min(n, i0 + per_call)
+            x = states[i0:i1].reshape((i1 - i0) * B, *states.shape[2:])
+            kw: Dict[str, Any] = dict(t_start=t_start, t_stop=t_stop, seed=seed,
+                                      cand_id0=cand_offset + (first_cand + i0) * B, x0=x0)
+            if self.step_noise is not None:
+                kw["noise"] = self.step_noise.repeat(1, i1 - i0, 1, 1, 1)
+            y, p = self.sampler.segment(x, self._labels_for(i1 - i0, labels) if guided else None, **kw)
+            out[i0:i1] = y.view(i1 - i0, B, *states.shape[2:])
+            if x0:
+                out_x0[i0:i1] = p.view(i1 - i0, B, *states.shape[2:])
+        return out, out_x0
 
 
 def make_denoise_fn(sampler, labels: Optional[torch.Tensor] = None, **kw) -> SamplerDenoiser:
@@ -140,17 +177,23 @@ def _shard(n: int, rank: int, world: int) -> Tuple[int, int]:
     return lo, min(n, lo + per)
 
 
-def _gather_scores(local: torch.Tensor, n: int) -> torch.Tensor:
+def _gather_states(local: torch.Tensor, n: int) -> torch.Tensor:
+    """All n rows of a population block-sharded by `_shard` ([n_local, ...] fp32 per rank), in global order on
+    every rank: one all_gather of equal-sized, padded blocks."""
     dist, rank, world = _dist()
     if dist is None:
         return local
     per = -(-n // world)
-    buf = torch.full((per,), float("nan"), dtype=torch.float32, device=local.device)
-    buf[: local.numel()] = local
+    buf = torch.full((per, *local.shape[1:]), float("nan"), dtype=torch.float32, device=local.device)
+    buf[: local.shape[0]] = local
     parts = [torch.empty_like(buf) for _ in range(world)]
-    dist.all_gather(parts, buf)                       # the path's only collective
+    dist.all_gather(parts, buf)
     sizes = [_shard(n, r, world)[1] - _shard(n, r, world)[0] for r in range(world)]
     return torch.cat([p[:k] for p, k in zip(parts, sizes)])
+
+
+def _gather_scores(local: torch.Tensor, n: int) -> torch.Tensor:
+    return _gather_states(local, n)                   # the only collective of RandomSearch / ZeroOrder / PathSearch
 
 
 def _shared_seed(seed: Optional[int], device) -> int:
@@ -193,9 +236,8 @@ def argmax_first(scores: torch.Tensor) -> Tuple[int, float]:
     return int(idx.item()), float(val.item())
 
 
-def topk_first(scores: torch.Tensor, k: int) -> Tuple[List[int], List[float]]:
-    """The k best (indices, values) under argmax_first's rule (strict '>', first index on ties, NaN never ranks);
-    indices are -1 past the number of eligible scores."""
+def _topk_device(scores: torch.Tensor, k: int) -> Tuple[torch.Tensor, torch.Tensor]:
+    """topk_first with the (int32 indices, fp32 values) left on the device."""
     _lib.require_cuda()
     s = scores.detach().to(torch.float32).contiguous()
     idx = torch.empty(k, dtype=torch.int32, device=s.device)
@@ -203,7 +245,36 @@ def topk_first(scores: torch.Tensor, k: int) -> Tuple[List[int], List[float]]:
     with torch.cuda.device(s.device):
         _lib.check(_lib.lib().its_topk_first(idx.data_ptr(), val.data_ptr(), s.data_ptr(), s.numel(), int(k),
                                              _lib.stream_ptr(s.device)), "its_topk_first")
+    return idx, val
+
+
+def topk_first(scores: torch.Tensor, k: int) -> Tuple[List[int], List[float]]:
+    """The k best (indices, values) under argmax_first's rule (strict '>', first index on ties, NaN never ranks);
+    indices are -1 past the number of eligible scores."""
+    idx, val = _topk_device(scores, k)
     return idx.tolist(), val.tolist()
+
+
+def path_expand(x: torch.Tensor, parent: torch.Tensor, m: int, child0: int, n_child: int, a: float, b: float, *,
+                z: Optional[torch.Tensor] = None, seed: int = 0, cand_id0: int = 0,
+                tag: int = TAG_FORWARD) -> torch.Tensor:
+    """[n_child, *x.shape[1:]]: child i = a * x[parent[(child0 + i) // m]] + b * z_i (fp32, separately rounded),
+    z_i = z[i] or the Philox unit cand_id0 + child0 + i of `philox_normal` under `tag`.  `parent` is a device int32
+    tensor (survivor indices into x, e.g. straight from the top-k kernel)."""
+    _lib.require_cuda()
+    xs = x.detach().to(torch.float32).contiguous()
+    par = parent.to(device=xs.device, dtype=torch.int32).contiguous()
+    out = torch.empty((n_child, *xs.shape[1:]), dtype=torch.float32, device=xs.device)
+    zz = None if z is None else z.to(device=xs.device, dtype=torch.float32).contiguous()
+    if zz is not None and zz.numel() != out.numel():
+        raise ValueError(f"z must hold {tuple(out.shape)} values, got {tuple(zz.shape)}")
+    with torch.cuda.device(xs.device):
+        _lib.check(_lib.lib().its_path_expand(out.data_ptr(), xs.data_ptr(), par.data_ptr(), par.numel(), int(m),
+                                              int(child0), int(n_child), xs.shape[0], out[0].numel(), float(a),
+                                              float(b), None if zz is None else zz.data_ptr(), int(seed),
+                                              int(cand_id0), int(tag), _lib.stream_ptr(xs.device)),
+                   "its_path_expand")
+    return out
 
 
 def _score_population(cands_local: torch.Tensor, lo: int, n_total: int, denoise: SamplerDenoiser, ver,
@@ -437,6 +508,156 @@ class PathSearch:
         if idx >= 0:
             best_score, best_noise, self.last_index = val, perturbed(idx, idx + 1)[0].clone(), idx
         return best_noise, best_score, history
+
+    def reset_nfes(self):
+        self.nfes = 0
+
+
+# --------------------------------------------------------- SearchOverPaths --
+def path_rounds(T: int, start_step: int, delta_f: int, delta_b: int) -> List[Tuple[int, int, int]]:
+    """Round schedule of search over paths: (s, s', e) per round.  A round starts from states at step s, re-noises
+    them to step s' = min(s + delta_f, T - 1) and denoises steps s' ... e = max(s' - delta_b + 1, 0); the next
+    round starts at e - 1.  The last round ends with step 0.  Raises ValueError for parameters outside
+    0 <= start_step <= T - 1, 0 <= delta_f < delta_b."""
+    T, s, delta_f, delta_b = int(T), int(start_step), int(delta_f), int(delta_b)
+    if T < 1:
+        raise ValueError(f"T={T} must be >= 1")
+    if not 0 <= s <= T - 1:
+        raise ValueError(f"start_step={s} outside [0, T-1={T - 1}]")
+    if delta_f < 0:
+        raise ValueError(f"delta_f={delta_f} must be >= 0")
+    if delta_b <= delta_f:
+        raise ValueError(f"delta_b={delta_b} must exceed delta_f={delta_f} (each round must make progress)")
+    rounds = []
+    while True:
+        sp = min(s + delta_f, T - 1)
+        e = max(sp - delta_b + 1, 0)
+        rounds.append((s, sp, e))
+        if e == 0:
+            return rounds
+        s = e - 1
+
+
+class SearchOverPaths:
+    """Search over paths (Ma et al., "Inference-Time Scaling for Diffusion Models beyond Scaling Denoising
+    Steps"): a beam of `n_beams` (N) partial trajectories.  Stage 0 denoises N initial x_T (Philox TAG_X_T keyed
+    by path id, as RandomSearch draws candidates, or `candidate_noise` [N, *noise_shape]) down to the state at
+    `start_step`.  Each round (`path_rounds`) re-noises every survivor `n_children` (M) times with q(x_s' | x_s)
+    (`delta_f` forward steps), denoises all N*M children `delta_b` steps, scores each on the x0 prediction of its
+    segment's last UNet evaluation (no extra evaluation) and keeps the N best (`topk_first`); the last round
+    ends at step 0 and returns the best finished sample (`argmax_first`).
+
+    Population mode only: an its_b200 `SamplerDenoiser` and a kernel verifier's `.score`.  Paths and children
+    are sharded over the ranks by global id; per round one score all_gather and one all_gather of the fp32
+    states.  Random streams depend on (seed, inputs) only: step noise of a child by (seed, round, child id),
+    re-noising by TAG_FORWARD, so results do not depend on rank count, `max_images` or batch.
+
+    `search(noise_shape, denoise_fn, verifier_fn, ...)` returns (best_images [B,C,H,W], best_score, history);
+    keyword extensions: `seed`, `labels`, `candidate_noise`, `forward_noise` ([rounds][N*M, *noise_shape]
+    injected re-noising draws).  `last_index` is the winner's initial path id, `last_seed` the search seed.
+    `nfes` counts UNet steps x candidates (the reference's classes count denoise_fn calls)."""
+
+    def __init__(self, n_beams: int = 4, n_children: int = 4, start_step: int = 800, delta_f: int = 50,
+                 delta_b: int = 100, verbose: bool = False):
+        self.n_beams = n_beams
+        self.n_children = n_children
+        self.start_step = start_step
+        self.delta_f = delta_f
+        self.delta_b = delta_b
+        self.verbose = verbose
+        self.nfes = 0
+
+    def search(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
+               device: str = 'cuda', verbose: Optional[bool] = None,
+               **kwargs) -> Tuple[torch.Tensor, float, Dict[str, Any]]:
+        cand_noise = kwargs.pop("candidate_noise", None)
+        fwd_noise = kwargs.pop("forward_noise", None)
+        seed = kwargs.pop("seed", None)
+        labels = kwargs.get("labels")
+        ver = _population_mode(denoise_fn, verifier_fn)
+        if ver is None:
+            raise ValueError("SearchOverPaths needs an its_b200 SamplerDenoiser and a kernel verifier's .score "
+                             "(population mode)")
+        N, M = int(self.n_beams), int(self.n_children)
+        if N < 1 or M < 1:
+            raise ValueError(f"n_beams={N} and n_children={M} must be >= 1")
+        smp = denoise_fn.sampler
+        T = smp.T
+        rounds = path_rounds(T, self.start_step, self.delta_f, self.delta_b)
+        if fwd_noise is not None and len(fwd_noise) < len(rounds):
+            raise ValueError(f"forward_noise has {len(fwd_noise)} rounds, the schedule {len(rounds)}")
+        dist, rank, world = _dist()
+        dev = torch.device(device)
+        seed = _shared_seed(seed, dev)
+        self.last_seed = seed
+        shape = tuple(noise_shape)
+        B = shape[0]
+        abar = torch.cumprod(1. - smp.betas.detach().double().cpu(), dim=0)
+        denoise_fn.reset_calls()
+        history: Dict[str, Any] = {'rounds': [], 'scores': [], 'survivors': []}
+        steps = 0                                     # UNet steps x candidates
+        with torch.no_grad():
+            # stage 0: N paths from x_T down to the states at step start_step
+            lo, hi = _shard(N, rank, world)
+            if cand_noise is not None:
+                local = cand_noise[lo:hi].to(dev, torch.float32)
+            elif hi > lo:
+                local = philox_normal((hi - lo,) + shape, seed, lo, TAG_X_T, dev)
+            else:
+                local = torch.empty((0,) + shape, device=dev)
+            s0 = rounds[0][0]
+            if s0 < T - 1 and hi > lo:
+                local = denoise_fn.denoise_candidates(local, lo, labels=labels, seed=seed, t_stop=s0 + 1, clip=False)
+            steps += N * (T - 1 - s0)
+            parents = _gather_states(local.contiguous(), N)
+            parent_idx = torch.arange(N, dtype=torch.int32, device=dev)
+            n_c = N * M
+            lo, hi = _shard(n_c, rank, world)
+            for r, (s, sp, e) in enumerate(rounds):
+                ratio = float(abar[sp] / abar[s])
+                a, b = math.sqrt(ratio), math.sqrt(1. - ratio)
+                if hi > lo:
+                    z = None if fwd_noise is None else fwd_noise[r][lo:hi]
+                    kids = path_expand(parents.reshape(parents.shape[0], -1), parent_idx, M, lo, hi - lo, a, b,
+                                       z=None if z is None else z.reshape(hi - lo, -1), seed=seed,
+                                       cand_id0=(r + 1) * ROUND_STRIDE, tag=TAG_FORWARD).view((hi - lo,) + shape)
+                    states, x0 = denoise_fn.denoise_segment(kids, lo, t_start=sp, t_stop=e, labels=labels, seed=seed,
+                                                            cand_offset=(r + 1) * ROUND_STRIDE, x0=True)
+                    judged = x0 if e > 0 else states   # the last round scores the finished, clipped samples
+                    local_scores = ver.score_candidates(judged.reshape(-1, *shape[1:]), B)
+                else:
+                    states = torch.empty((0,) + shape, device=dev)
+                    local_scores = torch.empty(0, dtype=torch.float32, device=dev)
+                steps += n_c * (sp - e + 1)
+                scores = _gather_scores(local_scores, n_c)
+                history['rounds'].append((s, sp, e))
+                history['scores'].append([float(v) for v in scores.tolist()])
+                parents = _gather_states(states.contiguous(), n_c)
+                if e > 0:
+                    parent_idx, _ = _topk_device(scores, N)
+                    ids = parent_idx.tolist()
+                    if min(ids) < 0:
+                        raise ValueError(f"round {r}: only {sum(i >= 0 for i in ids)} of {n_c} children have a "
+                                         f"score that can be ranked; {N} survivors are needed")
+                    history['survivors'].append(ids)
+                else:
+                    idx, best = argmax_first(scores)
+                    if idx < 0:
+                        raise ValueError(f"last round: none of the {n_c} finished samples has a score that can be "
+                                         "ranked")
+                    history['survivors'].append([idx])
+        # lineage of the winner: child id in every round, back to its initial path
+        child = idx
+        lineage = [child]
+        for ids in reversed(history['survivors'][:-1]):
+            child = ids[child // M]
+            lineage.append(child)
+        lineage.reverse()
+        history['lineage'] = {'path': lineage[0] // M, 'children': lineage}
+        history['unet_image_steps'] = steps * B * (2 if getattr(smp, "guided", False) else 1)
+        self.nfes += steps
+        self.last_index = lineage[0] // M
+        return parents[idx].clone(), best, history
 
     def reset_nfes(self):
         self.nfes = 0

@@ -1,7 +1,8 @@
 """Multi-GPU check of the three searches (BASELINE.json configs[3]): run under torchrun, one rank per GPU.
 Every rank must end with the same selection, and that selection must be bit-identical to the one the
 same rank computes alone over the whole population (candidate ids, Philox streams and summation orders
-do not depend on the number of ranks).  The only collective per round is the score all_gather.
+do not depend on the number of ranks).  The only collective per round is the score all_gather (search over
+paths adds one all_gather of the candidates' states per round).
 
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1 --master-port 29511 \
         scripts/search_multi_gpu.py
@@ -52,6 +53,9 @@ def run_all():
         ps = S.PathSearch(n_paths=5, injection_step=T // 2, noise_scale=0.1)
         pn, pscore, ph = ps.search(x0, den, ver.score, timesteps=T, device=str(dev), seed=23, restart=restart)
         out["path_restart" if restart else "path"] = (pn.clone(), pscore, torch.tensor(ph["scores"]))
+    sop = S.SearchOverPaths(n_beams=3, n_children=3, start_step=3 * T // 4, delta_f=T // 8, delta_b=T // 4)
+    si, ss, sh = sop.search(shape, den, ver.score, device=str(dev), seed=24)   # 9 children: ragged over 2 ranks
+    out["search_over_paths"] = (si.clone(), ss, torch.tensor(sh["scores"]))
     return out
 
 
