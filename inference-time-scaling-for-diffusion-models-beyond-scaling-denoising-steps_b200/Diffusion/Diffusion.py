@@ -26,11 +26,14 @@ class GaussianDiffusionSampler(SamplerBase):
 
     def forward(self, x_T, *, noise=None, seed=None, cand_id0=0, t_start=None, clip=True, t_stop=0):
         """Algorithm 2 (Diffusion.py:84-102): T fused steps on the device, then
-        clip to [-1, 1].  Extensions (keyword-only, defaults = reference
-        behaviour): `noise` [T, *x_T.shape] injects the per-step Gaussians (entry
-        t at time_step t, for parity runs); otherwise they come from the
-        in-kernel Philox stream `seed` keyed by candidate id `cand_id0 + b`;
-        `t_start` begins the loop at an intermediate step (search over paths) and
-        `t_stop` ends it early (metrics tracking), returning the unclipped x_{t_stop-1}."""
-        return self._sample(x_T, None, noise=noise, seed=seed, cand_id0=cand_id0, t_start=t_start, clip=clip,
-                            t_stop=t_stop)
+        clip to [-1, 1].  The steps replay the sampler's captured step graph,
+        which `segment` shares; the candidate base is read from device memory,
+        so a new `cand_id0` replays the same graph.  Extensions (keyword-only,
+        defaults = reference behaviour): `noise` [T, *x_T.shape] injects the
+        per-step Gaussians (entry t at time_step t, for parity runs); otherwise
+        they come from the in-kernel Philox stream `seed` keyed by candidate id
+        `cand_id0 + b`; `t_start` begins the loop at an intermediate step (search
+        over paths) and `t_stop` ends it early (metrics tracking), returning the
+        unclipped x_{t_stop-1}."""
+        return self._run(x_T, None, t_start=t_start, t_stop=t_stop, seed=seed, cand_id0=cand_id0, noise=noise,
+                         clip=clip, want_x0=False, check_nan=True)[0]

@@ -31,7 +31,8 @@ class GaussianDiffusionSampler(SamplerBase):
         return self.predict_xt_prev_mean_from_eps(x_t, t, eps=eps), var
 
     def forward(self, x_T, labels, *, noise=None, seed=None, cand_id0=0, t_start=None, clip=True, t_stop=0):
-        """Algorithm 2 with guidance (DiffusionCondition.py:89-105).  Keyword-only
-        extensions as in the unconditional sampler."""
-        return self._sample(x_T, labels, noise=noise, seed=seed, cand_id0=cand_id0, t_start=t_start, clip=clip,
-                            t_stop=t_stop)
+        """Algorithm 2 with guidance (DiffusionCondition.py:89-105), replaying the
+        sampler's captured step graph as the unconditional sampler does.
+        Keyword-only extensions as in the unconditional sampler."""
+        return self._run(x_T, labels, t_start=t_start, t_stop=t_stop, seed=seed, cand_id0=cand_id0, noise=noise,
+                         clip=clip, want_x0=False, check_nan=True)[0]

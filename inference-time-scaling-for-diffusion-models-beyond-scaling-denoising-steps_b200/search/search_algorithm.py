@@ -94,37 +94,21 @@ class SamplerDenoiser:
         return self.denoise_candidates(noise.unsqueeze(0), i, labels=kwargs.get("labels"))[0]
 
     def denoise_candidates(self, cands: torch.Tensor, first_cand: int, *, labels=None,
-                           t_start: Optional[int] = None, seed: Optional[int] = None, t_stop: int = 0,
-                           clip: bool = True) -> torch.Tensor:
+                           t_start: Optional[int] = None, seed: Optional[int] = None, t_stop: int = 0) -> torch.Tensor:
         """cands [n, B, C, H, W] -> images [n, B, C, H, W]; candidate i is global
-        candidate first_cand + i (its Philox streams are keyed by that id).  `t_stop` / `clip` end the loop
-        early as the sampler's own arguments do (the states step t_stop - 1 starts from)."""
-        n, B = cands.shape[:2]
-        guided = getattr(self.sampler, "guided", False)
-        per_call = max(1, self.max_images // B)
-        out = torch.empty_like(cands)
-        seed = self.step_seed(seed)
-        for i0 in range(0, n, per_call):
-            i1 = min(n, i0 + per_call)
-            x = cands[i0:i1].reshape((i1 - i0) * B, *cands.shape[2:])
-            kw: Dict[str, Any] = dict(seed=seed, cand_id0=(first_cand + i0) * B, t_start=t_start)
-            if t_stop or not clip:
-                kw.update(t_stop=t_stop, clip=clip)
-            if self.step_noise is not None:
-                kw["noise"] = self.step_noise.repeat(1, i1 - i0, 1, 1, 1)
-            if guided:
-                y = self.sampler(x, self._labels_for(i1 - i0, labels), **kw)
-            else:
-                y = self.sampler(x, **kw)
-            out[i0:i1] = y.view(i1 - i0, B, *cands.shape[2:])
-        return out
+        candidate first_cand + i (its Philox streams are keyed by that id).  `t_start` (default T-1) and `t_stop`
+        bound the loop as the sampler's own arguments do (a `t_stop` > 0 returns the states step t_stop - 1
+        starts from)."""
+        t_start = self.sampler.T - 1 if t_start is None else t_start
+        return self.denoise_segment(cands, first_cand, t_start=t_start, t_stop=t_stop, labels=labels, seed=seed,
+                                    x0=False)[0]
 
     def denoise_segment(self, states: torch.Tensor, first_cand: int, *, t_start: int, t_stop: int,
                         cand_offset: int = 0, labels=None, seed: Optional[int] = None,
                         x0: bool = True) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
         """states [n, B, C, H, W] at step t_start -> (states after step t_stop, x0 predictions of step t_stop or
         None), in chunks of `max_images`.  Candidate i's per-step Philox streams are keyed by
-        cand_offset + (first_cand + i) * B + image; every chunk replays the sampler's one segment graph."""
+        cand_offset + (first_cand + i) * B + image; every chunk replays the sampler's one step graph."""
         n, B = states.shape[:2]
         guided = getattr(self.sampler, "guided", False)
         per_call = max(1, self.max_images // B)
@@ -488,7 +472,8 @@ class PathSearch:
             T = smp.T
             if not (0 < self.injection_step < T):
                 raise ValueError("injection_step must lie in (0, T)")
-            base = _run_prefix(denoise_fn, initial_noise, self.injection_step, kwargs.get("labels"), seed)
+            base = denoise_fn.denoise_candidates(initial_noise.unsqueeze(0), 0, labels=kwargs.get("labels"), seed=seed,
+                                                 t_stop=self.injection_step)[0]
             t_start = self.injection_step - 1
 
         def perturbed(i0, i1):
@@ -607,7 +592,7 @@ class SearchOverPaths:
                 local = torch.empty((0,) + shape, device=dev)
             s0 = rounds[0][0]
             if s0 < T - 1 and hi > lo:
-                local = denoise_fn.denoise_candidates(local, lo, labels=labels, seed=seed, t_stop=s0 + 1, clip=False)
+                local = denoise_fn.denoise_candidates(local, lo, labels=labels, seed=seed, t_stop=s0 + 1)
             steps += N * (T - 1 - s0)
             parents = _gather_states(local.contiguous(), N)
             parent_idx = torch.arange(N, dtype=torch.int32, device=dev)
@@ -701,16 +686,3 @@ class GradientBasedSearch:
 
     def reset_nfes(self):
         self.nfes = 0
-
-
-def _run_prefix(denoise: SamplerDenoiser, x_T: torch.Tensor, stop_step: int, labels, seed=None) -> torch.Tensor:
-    """Run the pivot trajectory from T-1 down to `stop_step` inclusive as one device-resident segment
-    of the sampler's step graph and return the un-clipped state that step `stop_step - 1` starts from."""
-    smp = denoise.sampler
-    kw = dict(seed=denoise.step_seed(seed), cand_id0=0, t_stop=stop_step, clip=False)
-    if denoise.step_noise is not None:          # parity runs: the pivot's prefix uses the injected Gaussians too
-        kw["noise"] = denoise.step_noise
-    if getattr(smp, "guided", False):
-        lab = (labels if labels is not None else denoise.labels).reshape(-1).to(x_T.device, torch.int64)
-        return smp(x_T, lab, **kw)
-    return smp(x_T, **kw)

@@ -260,7 +260,7 @@ def test_path_expand_matches_torch(cuda_dev, built_lib):
 
 
 @pytest.mark.gpu
-def test_segment_uncut_equals_the_sampler(cuda_dev):
+def test_segment_uncut_equals_the_sampler_and_replays_its_graph(cuda_dev):
     cfg = SOP_CASES["u_sop"]
     net, _ = build_shell(cfg, cuda_dev)
     smp = _sampler(cfg, net, cuda_dev)
@@ -274,18 +274,39 @@ def test_segment_uncut_equals_the_sampler(cuda_dev):
     mid, _ = smp.segment(x_T, t_start=cfg["T"] - 1, t_stop=4, seed=19, cand_id0=6, x0=True)
     end, _ = smp.segment(mid, t_start=3, t_stop=0, seed=19, cand_id0=6, x0=True)
     assert torch.equal(end, whole)
-    assert smp.segment_captures == 2          # one graph per x0 mode
+    assert smp.graph_captures == 2            # one graph per x0 mode: segment(x0=False) replays forward's
 
 
 @pytest.mark.gpu
-def test_search_captures_the_step_graph_once(cuda_dev):
+def test_search_captures_stage_0_and_round_graphs_once(cuda_dev):
+    """One graph for stage 0 (N paths, steps 7 ... 5) and one for the rounds (N*M children); a second search
+    replays both."""
     cfg = SOP_CASES["u_sop"]
     net, _ = build_shell(cfg, cuda_dev)
     smp = _sampler(cfg, net, cuda_dev)
-    _, _, h, _ = _search(cfg, smp, cuda_dev, seed=4)
-    assert len(h["rounds"]) > 1 and smp.segment_captures == 1
-    _search(cfg, smp, cuda_dev, seed=4)
-    assert smp.segment_captures == 1
+    _, _, h, _ = _search(cfg, smp, cuda_dev, seed=4, start_step=4)
+    assert len(h["rounds"]) > 1 and smp.graph_captures == 2
+    _search(cfg, smp, cuda_dev, seed=4, start_step=4)
+    assert smp.graph_captures == 2
+
+
+@pytest.mark.gpu
+def test_chunks_and_serial_calls_capture_the_step_graph_once(cuda_dev):
+    """Chunks of a population and callable-mode candidates differ only in the candidate base: the step graph of
+    their batch size is captured once, and the images equal one unchunked call bit for bit."""
+    from its_b200.search import search_algorithm as S
+    cfg = SOP_CASES["u_sop"]
+    net, _ = build_shell(cfg, cuda_dev)
+    smp = _sampler(cfg, net, cuda_dev)
+    B = cfg["noise_shape"][0]
+    cands = _randn(5, (4,) + tuple(cfg["noise_shape"])).to(cuda_dev)
+    whole = S.make_denoise_fn(smp, max_images=4 * B, seed=11).denoise_candidates(cands, 0)
+    assert smp.graph_captures == 1
+    serial = S.make_denoise_fn(smp, max_images=B, seed=11)
+    got = torch.stack([serial(c) for c in cands])
+    assert torch.equal(got, whole) and smp.graph_captures == 2
+    chunked = S.make_denoise_fn(smp, max_images=B, seed=11).denoise_candidates(cands, 0)
+    assert torch.equal(chunked, whole) and smp.graph_captures == 2
 
 
 def _compare_with_oracle(h, ref_h, N, tol, strict):
