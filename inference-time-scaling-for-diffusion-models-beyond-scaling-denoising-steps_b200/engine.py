@@ -1,20 +1,28 @@
 """Execution plans: the UNet forward as a fixed list of libits_b200 kernel launches.
 
-A `UNetPlan` is built once per (model, batch, resolution).  It owns
-  * packed weights (bf16, K-major [Cout][taps*Cin], shortcut / dual-conv / sub-pixel
-    phases concatenated along K) rebuilt from the nn.Parameters of the shell
-    modules (which keep the reference's state-dict layout),
-  * every activation buffer (NHWC bf16; HBM is 180 GB, nothing is recycled inside
-    a step so that a step is a pure function of (x, t, labels)),
+A plan is built once per (model, batch, resolution).  It owns
+  * packed weights rebuilt from the nn.Parameters of the shell modules (which keep
+    the reference's state-dict layout),
+  * every activation buffer (nothing is recycled inside a step, so that a step is a
+    pure function of (x, t, labels); HBM is 180 GB),
   * the launch list.  All launches go to the caller's current stream, never
     synchronise or allocate, so a whole sampler step is captured into one CUDA
     graph and replayed T times with the step index living on the device.
+
+`PlanBase` walks the network once for every plan: input buffers, time-embedding
+chain, label chain, the down / middle / up path with its skip stack, the tail
+GroupNorm; it also owns the launch lists and run().  A subclass supplies the
+layers: `UNetPlan` here (16-bit operands on the tcgen05 tap-GEMM, NHWC bf16 / fp16
+activations, weights packed K-major [Cout][taps*Cin] with shortcut / dual-conv /
+sub-pixel phases concatenated along K), `engine_f32.UNetPlanF32` (fp32 CUDA-core
+kernels, the parity path).
 
 torch is used here for device memory and streams only; all arithmetic on the hot
 path is in the .so.
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 import math
 from typing import List, Optional, Sequence, Tuple
@@ -49,11 +57,18 @@ def taps_square(k: int, src: int = 0) -> List[Tuple[int, int, int]]:
     return [(src, ky - p, kx - p) for ky in range(k) for kx in range(k)]
 
 
-class UNetPlan:
-    """Launch plan of one UNet evaluation for n_img images of H x W."""
+class PlanBase:
+    """Launch plan of one UNet evaluation for n_img images of H x W: what every precision shares.
+
+    The constructor walks the network once (_build): input buffers, time-embedding chain, label chain, the
+    down / middle / up path with its skip stack, the tail GroupNorm.  The subclass emits the layers through
+    conv / group_norm / head_conv / _res_block / _attn_block / _down / _up / _tail_conv and sets its knobs in
+    _configure."""
+
+    ACT_DTYPE = BF16        # activation dtype of _new
 
     def __init__(self, model, n_img: int, H: int, W: int, *, n_img_in: Optional[int] = None,
-                 uniform_t: bool = False, impl: Optional[int] = None):
+                 uniform_t: bool = False, impl: Optional[int] = None, device=None):
         _lib.require_cuda()
         self.L = _lib.lib()
         self.model = model
@@ -61,61 +76,45 @@ class UNetPlan:
         self.n_img, self.H, self.W = int(n_img), int(H), int(W)
         self.n_img_in = int(n_img_in or n_img)
         self.uniform_t = uniform_t
-        self.dev = model.head.weight.device
+        self.dev = torch.device(device) if model is None else model.head.weight.device
         if self.dev.type != "cuda":
             raise RuntimeError("its_b200 UNet must live on a CUDA device (no CPU fallback); call .cuda()")
         self.impl_forced = impl
         self.keep: List[torch.Tensor] = []      # everything the launches point into
-        self.descs: List[ConvDesc] = []
         self.ops: List[Tuple] = []
         self.label_ops: List[Tuple] = []         # label embedding -> cond_proj of every ResBlock
-        self.n_label_launches = 0
         self.op_info: List[Tuple[str, int, int]] = []   # (kind, algorithmic flops, launches) per op
-        self.n_launches = 0
-        self.flops = 0                           # algorithmic 2*MAC of the tensor-core GEMMs + linears
-        with torch.no_grad():
-            self._build()
+        self.n_launches = self.n_label_launches = 0
+        self.flops = 0                           # algorithmic 2*MAC of the GEMMs, convolutions and linears
+        self.gn_bytes = 0                        # algorithmic bytes of the stand-alone 16-bit GroupNorm launches
+        self._to_label_ops = False
+        self.x_in = self.eps = self.t_dev = self.t_idx = self.labels = None
+        self.tproj = self.cproj = None           # every ResBlock's projected time / label embedding
+        # run() may run ops[:_n_time_ops] (the time chain) on a side stream, joined before ops[_join_at]
+        self.fork_time_chain = False
+        self._n_time_ops, self._join_at = 0, None
+        self._side = self._ev_fork = self._ev_join = None
+        self._configure()
+        if model is not None:
+            with torch.no_grad():
+                self._build()
 
-    @classmethod
-    def scratch(cls, device, n_img: int, impl: Optional[int] = None) -> "UNetPlan":
-        """A plan without a model: lets tests and micro-benchmarks append single
-        launches (conv / group_norm / linear) through the same descriptor builder."""
-        _lib.require_cuda()
-        self = cls.__new__(cls)
-        self.L = _lib.lib()
-        self.model, self.cond = None, False
-        self.n_img, self.H, self.W, self.n_img_in = int(n_img), 0, 0, int(n_img)
-        self.uniform_t, self.dev, self.impl_forced = False, torch.device(device), impl
-        self.keep, self.descs, self.ops, self.op_info = [], [], [], []
-        self.label_ops, self.n_label_launches = [], 0
-        self.n_launches, self.flops = 0, 0
-        self.gn_partials, self.tproj, self.cproj = None, None, None
-        self.ws, self.split_k = None, True
-        self.stats_of, self.schedule, self.fold_residual = {}, 0, True
-        self.ws_persist, self.sm_count, self.fused_attention = None, 148, True
-        self.head_on_tensor_cores = True
-        self.attn_v_mn = _os.environ.get("ITS_ATTN_VT", "0") != "1"
-        self.fork_time_chain, self._side = False, None
-        self.res_dtype = FP16 if (_os.environ.get("ITS_RESIDUAL_FP16", "0") == "1" and impl is None) else BF16
-        self.gn_dtype = FP16 if (FP16_GN and impl != 1) else BF16
-        self.prefused, self.n_gn_fused = {}, 0
-        self.gn_fusion = {"0": "off", "1": "all"}.get(_os.environ.get("ITS_GN_FUSION", "1"), "auto")   # scratch plans: all
-        return self
+    def _configure(self) -> None:
+        """Knobs and state of the subclass's layers."""
 
     # ------------------------------------------------------------ buffers --
-    def _new(self, shape: Sequence[int], dtype=BF16) -> torch.Tensor:
-        t = torch.empty(tuple(int(s) for s in shape), dtype=dtype, device=self.dev)
+    def _new(self, shape: Sequence[int], dtype=None) -> torch.Tensor:
+        t = torch.empty(tuple(int(s) for s in shape), dtype=dtype or self.ACT_DTYPE, device=self.dev)
         self.keep.append(t)
         return t
 
-    def _hold(self, t: torch.Tensor, dtype=None) -> torch.Tensor:
-        t = t.detach().to(device=self.dev, dtype=dtype or t.dtype).contiguous()
+    def _hold(self, t: torch.Tensor, dtype=torch.float32) -> torch.Tensor:
+        t = t.detach().to(device=self.dev, dtype=dtype).contiguous()
         self.keep.append(t)
         return t
 
     def _op(self, fn, *args, launches: int = 1, flops: int = 0, kind: str = "other"):
-        if getattr(self, "_into_label_ops", False):
-            # depends on the labels only (constant over a trajectory): see run_label_ops()
+        if self._to_label_ops:
             self.label_ops.append((fn, args))
             self.n_label_launches += launches
             return
@@ -123,6 +122,193 @@ class UNetPlan:
         self.op_info.append((kind, flops, launches))
         self.n_launches += launches
         self.flops += flops
+
+    @contextlib.contextmanager
+    def _label_ops(self):
+        """Launches appended inside depend on the labels only (constant over a trajectory): they go to
+        label_ops, which run_label_ops() enqueues."""
+        self._to_label_ops = True
+        try:
+            yield
+        finally:
+            self._to_label_ops = False
+
+    def linear(self, x: torch.Tensor, W: torch.Tensor, b: Optional[torch.Tensor], *, silu_in=False,
+               silu_out=False) -> torch.Tensor:
+        rows, K = x.shape
+        N = W.shape[0]
+        y = self._new((rows, N), torch.float32)
+        self._op(self.L.its_linear, y.data_ptr(), x.data_ptr(), W.data_ptr(), _ptr(b), rows, K, N,
+                 int(silu_in), int(silu_out), 0, flops=2 * rows * K * N, kind="linear")
+        return y
+
+    def _linear_of(self, x: torch.Tensor, lin, **kw) -> torch.Tensor:
+        return self.linear(x, self._hold(lin.weight), self._hold(lin.bias), **kw)
+
+    # -------------------------------------------------------------- build --
+    def _build(self):
+        m, L = self.model, self.L
+        B, H, W = self.n_img, self.H, self.W
+        ch = m.head.out_channels
+        self.x_in = self._new((self.n_img_in, 3, H, W), torch.float32)
+        self.t_dev = torch.zeros(1, dtype=torch.int32, device=self.dev)
+        self.t_idx = torch.zeros(B, dtype=torch.int64, device=self.dev)
+        self.labels = torch.zeros(B, dtype=torch.int64, device=self.dev) if self.cond else None
+        rows = 1 if self.uniform_t else B
+        t_idx_ptr = None if self.uniform_t else self.t_idx.data_ptr()
+        te = m.time_embedding
+        emb = self._new((rows, ch), torch.float32)
+        if self.cond:
+            table = self._hold(te.timembedding[0].weight)
+            self._op(L.its_embed_rows, emb.data_ptr(), table.data_ptr(), t_idx_ptr, self.t_dev.data_ptr(), rows,
+                     ch, table.shape[0])
+            lin1, lin2 = te.timembedding[1], te.timembedding[3]
+        else:
+            freq = self._hold(te.freq_coeffs)
+            self._op(L.its_time_embed, emb.data_ptr(), t_idx_ptr, self.t_dev.data_ptr(), freq.data_ptr(), rows, ch)
+            lin1, lin2 = te.timembedding[0], te.timembedding[2]
+        temb = self._linear_of(self._linear_of(emb, lin1, silu_out=True), lin2)
+        # every ResBlock's temb_proj (and cond_proj) as ONE linear over concatenated weights (Model.py:181-184)
+        blocks = [b for b in list(m.downblocks) + list(m.middleblocks) + list(m.upblocks) if hasattr(b, "temb_proj")]
+        offs, o = {}, 0
+        for rb in blocks:
+            offs[id(rb)] = o
+            o += rb.temb_proj[1].out_features
+
+        def proj(x, name):
+            w = torch.cat([getattr(rb, name)[1].weight.detach().float() for rb in blocks], 0)
+            b = torch.cat([getattr(rb, name)[1].bias.detach().float() for rb in blocks], 0)
+            return self.linear(x, self._hold(w), self._hold(b), silu_in=True)
+        self.tproj = proj(temb, "temb_proj")
+        # The time-embedding chain (embedding -> two linears -> every temb_proj) depends on t only; the head
+        # (patch gather, head GEMM, first GroupNorm) depends on x only.  run() may fork the chain onto a side
+        # stream and join before the first launch that adds the projected embedding (_join_at, set by conv).
+        self._n_time_ops = len(self.ops)
+        if self.cond:
+            # Everything from the label embedding to the per-ResBlock cond_proj vectors is a function of
+            # the labels alone (ModelCondition.py:216,131-135,154).  The labels of a trajectory never
+            # change, so the sampler runs these launches once per forward() instead of once per step;
+            # UNet.forward() runs them on every call.
+            with self._label_ops():
+                ce = m.cond_embedding.condEmbedding
+                ctab = self._hold(ce[0].weight)
+                cemb0 = self._new((B, ch), torch.float32)
+                self._op(L.its_embed_rows, cemb0.data_ptr(), ctab.data_ptr(), self.labels.data_ptr(), None, B, ch,
+                         ctab.shape[0])
+                cemb = self._linear_of(self._linear_of(cemb0, ce[1], silu_out=True), ce[3])
+                self.cproj = proj(cemb, "cond_proj")
+        # The GroupNorm -> Swish that the NEXT layer opens with, when that layer reads this layer's output alone
+        # (down path, middle, tail): the producing launch may apply it in its epilogue.  Up-path ResBlocks
+        # normalise the concatenation [h, skip] (their groups mix both tensors) and resampling convs read
+        # the raw tensor: nothing is passed there.
+        seq = list(m.downblocks) + list(m.middleblocks)
+
+        def opens_with(layer):
+            return (layer.block1[0], True) if hasattr(layer, "temb_proj") else None
+
+        next_gn = [opens_with(layer) for layer in seq[1:]] + [None]
+        h = self.head_conv(m.head.weight, m.head.bias, self.x_in, B, H, W, next_gn=opens_with(seq[0]))
+        hs = [h]
+        for i, layer in enumerate(seq):
+            if hasattr(layer, "temb_proj"):
+                h = self._res_block(layer, [h], offs[id(layer)], next_gn[i])
+            else:
+                h = self._down(layer, h, next_gn[i])
+            if i < len(m.downblocks):
+                hs.append(h)
+        ups = list(m.upblocks)
+        for i, layer in enumerate(ups):
+            if hasattr(layer, "temb_proj"):      # torch.cat([h, hs.pop()], 1)
+                tail_gn = (m.tail[0], True) if i == len(ups) - 1 else None
+                h = self._res_block(layer, [h, hs.pop()], offs[id(layer)], tail_gn)
+            else:
+                h = self._up(layer, h)
+        assert len(hs) == 0
+        a = self.group_norm([h], m.tail[0], silu=True)
+        self.eps = self._new((B, 3, H, W), torch.float32)
+        self._tail_conv(m.tail[2], a)
+
+    # ---------------------------------------------------------------- run --
+    @staticmethod
+    def _launch(ops, stream: int) -> None:
+        for fn, args in ops:
+            rc = fn(*args, stream)
+            if rc != 0:
+                _lib.check(rc, fn.__name__)
+
+    def run_label_ops(self) -> None:
+        """Enqueue the launches that depend on `self.labels` only (conditional net; no-op otherwise).
+        Must run after every change of the labels and before run()."""
+        self._launch(self.label_ops, _lib.stream_ptr(self.dev))
+
+    def run(self) -> None:
+        """Enqueue every launch on the current stream of the plan's device (graph-capturable).  With
+        fork_time_chain, the time-embedding chain runs on a side stream next to the head of the network
+        (fork / join by events, so the pair is two parallel branches of the captured step graph)."""
+        s = _lib.stream_ptr(self.dev)
+        n_time, join_at = self._n_time_ops, self._join_at
+        if not (self.fork_time_chain and n_time > 0 and join_at is not None and join_at > n_time):
+            self._launch(self.ops, s)
+            return
+        if self._side is None:
+            self._side = torch.cuda.Stream(device=self.dev)
+            self._ev_fork, self._ev_join = torch.cuda.Event(), torch.cuda.Event()
+        main = torch.cuda.current_stream()
+        self._ev_fork.record(main)
+        self._side.wait_event(self._ev_fork)
+        self._launch(self.ops[:n_time], self._side.cuda_stream)
+        self._ev_join.record(self._side)
+        self._launch(self.ops[n_time:join_at], s)
+        main.wait_event(self._ev_join)
+        self._launch(self.ops[join_at:], s)
+
+
+class UNetPlan(PlanBase):
+    """16-bit plan: tcgen05 tap-GEMMs (CUDA-core twins where a shape or `impl` asks for them)."""
+
+    @classmethod
+    def scratch(cls, device, n_img: int, impl: Optional[int] = None) -> "UNetPlan":
+        """A plan without a model: lets tests and micro-benchmarks append single
+        launches (conv / group_norm / linear) through the same descriptor builder."""
+        return cls(None, n_img, 0, 0, impl=impl, device=device)
+
+    def _configure(self) -> None:
+        """Every knob of a 16-bit plan.  A scratch plan (no model) differs from a model plan on purpose:
+          * gn_fusion: ITS_GN_FUSION defaults to 1 ("all": tests fuse wherever the tiling allows) and a forced
+            impl keeps it; a model plan defaults to "auto" and turns it "off" whenever impl is forced;
+          * schedule, fused_attention, head_on_tensor_cores, fork_time_chain: the defaults (0 / True / True /
+            False), whatever ITS_SCHEDULE, ITS_FUSED_ATTENTION, ITS_HEAD_TC and ITS_FORK_TIME say;
+          * res_dtype, gn_dtype: a model plan also needs a head width that is a multiple of 64, and for fp16
+            residuals also FP16_GN; its model's `residual_fp16` asks for them like ITS_RESIDUAL_FP16=1."""
+        m, impl, env = self.model, self.impl_forced, _os.environ.get
+        scratch = m is None
+        self.descs: List[ConvDesc] = []
+        self.gn_partials = self.ws = self.ws_persist = None     # workspaces, grown as layers need them
+        self.stats_of = {}          # raw tensor -> GroupNorm statistics its producing tap-GEMM left behind
+        self.prefused, self.n_gn_fused = {}, 0      # (tensor, GroupNorm) -> normalised tensor of a fused epilogue
+        self.split_k, self.fold_residual, self.sm_count = True, True, 148
+        self.attn_v_mn = env("ITS_ATTN_VT", "0") != "1"
+        # GroupNorm(+Swish) applied by the epilogue of the convolution that produces its input.  ITS_GN_FUSION:
+        # auto = where it was measured to pay (_fusion_pays), 1 = wherever the tiling allows it, 0 = never
+        # (every GroupNorm as its own its_group_norm_apply launch, the round-1 plan)
+        self.gn_fusion = {"0": "off", "1": "all"}.get(env("ITS_GN_FUSION", "1" if scratch else "auto"), "auto")
+        if impl is not None and not scratch:
+            self.gn_fusion = "off"
+        if scratch:
+            self.schedule, self.fused_attention, self.head_on_tensor_cores = 0, True, True
+        else:       # debugging switches (tests/parity triage): fall back to the simpler schedule of a stage
+            self.schedule = int(env("ITS_SCHEDULE", "0"))
+            self.fused_attention = env("ITS_FUSED_ATTENTION", "1") != "0"
+            self.head_on_tensor_cores = env("ITS_HEAD_TC", "1") != "0"
+            self.fork_time_chain = env("ITS_FORK_TIME", "1") != "0"
+        ch64 = scratch or m.head.out_channels % 64 == 0
+        # Opt-in: raw feature maps (residual stream, conv1 outputs) in IEEE fp16 instead of bf16 — 5x smaller
+        # error per evaluation (DESIGN.md section 5), but the residual stream follows |x_t|: only for trained
+        # checkpoints / schedules whose state stays far below fp16's 65504 (an overflow surfaces as the
+        # sampler's "nan in tensor." assertion).  Model attribute `residual_fp16` or ITS_RESIDUAL_FP16=1.
+        want16 = bool(getattr(m, "residual_fp16", False)) or env("ITS_RESIDUAL_FP16", "0") == "1"
+        self.res_dtype = FP16 if (want16 and impl is None and (scratch or (ch64 and FP16_GN))) else BF16
+        self.gn_dtype = FP16 if (FP16_GN and impl != 1 and ch64) else BF16
 
     # --------------------------------------------------------- primitives --
     def _impl_for(self, chans: Sequence[int], cout: int, out_nchw: bool = False) -> int:
@@ -255,7 +441,7 @@ class UNetPlan:
         d.out_fp16 = int(out.dtype == FP16) | (int(res is not None and res.dtype == FP16) << 1)
         d.Hout, d.Wout, d.out_scale, d.out_c_pitch, d.out_c_off = Hout, Wout, out_scale, out.shape[-1], 0
         d.bias = _ptr(bias)
-        if vec is not None and getattr(self, "_join_at", 0) is None:
+        if vec is not None and vec is self.tproj and self._join_at is None:
             self._join_at = len(self.ops)       # first consumer of the projected time embedding
         if vec is not None:
             d.vec, d.vec_stride, d.vec_off = vec.data_ptr(), (0 if vec.shape[0] == 1 else vec.shape[1]), vec_off
@@ -402,7 +588,7 @@ class UNetPlan:
             self._op(self.L.its_group_norm_apply, out.data_ptr(), x0.data_ptr(), C0, s0.data_ptr(), p0, _ptr(x1), C1,
                      _ptr(s1), p1, gamma.data_ptr(), beta.data_ptr(), B, HW, gn.num_groups, float(gn.eps),
                      int(silu), fmt, launches=1, kind="group_norm_apply")
-            self.gn_bytes = getattr(self, "gn_bytes", 0) + B * HW * Ct * 2 * 2
+            self.gn_bytes += B * HW * Ct * 2 * 2
             return out
         prow = max(1, 256 // (Ct // 8))
         # the split depends on (HW, C) only, never on the batch: a candidate's numbers are then
@@ -418,17 +604,8 @@ class UNetPlan:
                  self.gn_partials.data_ptr(), chunks,
                  f16 | (int(x0.dtype == FP16) << 1) | (int(x1 is not None and x1.dtype == FP16) << 2),
                  launches=1, kind="group_norm")
-        self.gn_bytes = getattr(self, "gn_bytes", 0) + B * HW * Ct * 2 * 2   # one read + one write, bf16
+        self.gn_bytes += B * HW * Ct * 2 * 2     # one read + one write, 16-bit
         return out
-
-    def linear(self, x: torch.Tensor, W: torch.Tensor, b: Optional[torch.Tensor], *, silu_in=False,
-               silu_out=False) -> torch.Tensor:
-        rows, K = x.shape
-        N = W.shape[0]
-        y = self._new((rows, N), torch.float32)
-        self._op(self.L.its_linear, y.data_ptr(), x.data_ptr(), W.data_ptr(), _ptr(b), rows, K, N,
-                 int(silu_in), int(silu_out), 0, flops=2 * rows * K * N, kind="linear")
-        return y
 
     # ------------------------------------------------------------- blocks --
     def _res_block(self, rb, xs: List[torch.Tensor], proj_off: int, next_gn=None) -> torch.Tensor:
@@ -475,76 +652,63 @@ class UNetPlan:
         wq, wk, wv = (m.weight.detach().float()[:, :, 0, 0] for m in (at.proj_q, at.proj_k, at.proj_v))
         bq, bk, bv = (m.bias.detach().float() for m in (at.proj_q, at.proj_k, at.proj_v))
         one = [(0, 0, 0)]
-        tensor_path = N > 64      # batched-GEMM formulation (tcgen05, or its CUDA-core twin when forced)
-        if tensor_path:
-            fused256 = N == 256 and Cc % 64 == 0 and Cc <= 384
-            flash = N % 128 == 0 and N > 256 and Cc in (64, 128)
-            if (fused256 or flash) and self._impl_for([Cc], Cc) == 0 and self.fused_attention and self.attn_v_mn:
+        on_tc = self._impl_for([Cc], Cc) == 0 and self.fused_attention
+        flops = 4 * B * N * N * Cc
+
+        def project(w, b, cout):    # 1x1 projection(s) of the normalised input
+            return self.conv([(a, Cc, 0, 1, False)], [(one, 0, 0, 0)], H, W, self._hold(w), cout, bias=self._hold(b),
+                             want_stats=False)
+        if N > 64:      # batched-GEMM formulation (tcgen05, or its CUDA-core twin when forced)
+            core = (("attention_fused", self.L.its_attention_fused) if N == 256 and Cc % 64 == 0 and Cc <= 384 else
+                    ("attention_flash", self.L.its_attention_flash) if N % 128 == 0 and N > 256 and Cc in (64, 128)
+                    else None)
+            fused = core is not None and on_tc
+            if fused and self.attn_v_mn:
                 # one projection launch for q|k|v; the attention core reads V as an MN-major B operand
                 # straight from that tensor (no V^T projection launch)
-                wqkv = self._hold(torch.cat([wq, wk, wv], 0), torch.float32)
-                bqk0 = self._hold(torch.cat([bq, bk, torch.zeros_like(bv)], 0), torch.float32)
-                qkv = self.conv([(a, Cc, 0, 1, False)], [(one, 0, 0, 0)], H, W, wqkv, 3 * Cc, bias=bqk0, want_stats=False)
+                qk = project(torch.cat([wq, wk, wv]), torch.cat([bq, bk, torch.zeros_like(bv)]), 3 * Cc)
+                vT = None
+            else:
+                qk = project(torch.cat([wq, wk]), torch.cat([bq, bk]), 2 * Cc)
+                # V^T[b] = Wv . a[b]^T : weights are the A operand, the image is the B operand
+                wv_img = self._hold(wv.reshape(1, 1, Cc, Cc), a.dtype)
+                vT = self.conv([(wv_img, Cc, 0, 1, True)], [(one, 0, 0, 0)], 1, Cc, a.view(B, N, Cc), N,
+                               w_batch_stride=N * Cc, out_shape=(B, 1, Cc, N), want_stats=False)
+            if fused:
+                # scores in TMEM, probabilities in shared memory: one launch for QK^T, softmax and PV; V's bias is
+                # added after the product (the rows of softmax(S) sum to one)
                 o = self._new((B, H, W, Cc))
-                bvh = self._hold(bv, torch.float32)     # added after the product: the rows of softmax(S) sum to one
-                self._op(self.L.its_attention_fused if fused256 else self.L.its_attention_flash, o.data_ptr(),
-                         qkv.data_ptr(), None, bvh.data_ptr(), B, N, Cc, scale, flops=4 * B * N * N * Cc,
-                         kind="attention_fused" if fused256 else "attention_flash")
-                wp = self._hold(at.proj.weight.detach().float()[:, :, 0, 0], torch.float32)
-                bp = self._hold(at.proj.bias, torch.float32)
-                return self.conv([(o, Cc, 0, 1, False)], [(one, 0, 0, 0)], H, W, wp, Cc, bias=bp, res=x, out_dtype=self.res_dtype,
-                                 fuse_gn=next_gn)
-            wqk = self._hold(torch.cat([wq, wk], 0), torch.float32)
-            bqk = self._hold(torch.cat([bq, bk], 0), torch.float32)
-            qk = self.conv([(a, Cc, 0, 1, False)], [(one, 0, 0, 0)], H, W, wqk, 2 * Cc, bias=bqk, want_stats=False)
-            # V^T[b] = Wv . a[b]^T : weights are the A operand, the image is the B operand
-            wv_img = self._hold(wv.reshape(1, 1, Cc, Cc), a.dtype)
-            vT = self.conv([(wv_img, Cc, 0, 1, True)], [(one, 0, 0, 0)], 1, Cc, a.view(B, N, Cc), N,
-                           w_batch_stride=N * Cc, out_shape=(B, 1, Cc, N), want_stats=False)
-            if (fused256 or flash) and self._impl_for([Cc], Cc) == 0 and self.fused_attention:
-                # scores in TMEM, probabilities in shared memory: one launch for QK^T, softmax and PV
-                o = self._new((B, H, W, Cc))
-                bvh = self._hold(bv, torch.float32)
-                self._op(self.L.its_attention_fused if fused256 else self.L.its_attention_flash, o.data_ptr(),
-                         qk.data_ptr(), vT.data_ptr(), bvh.data_ptr(), B, N, Cc, scale, flops=4 * B * N * N * Cc,
-                         kind="attention_fused" if fused256 else "attention_flash")
-                wp = self._hold(at.proj.weight.detach().float()[:, :, 0, 0], torch.float32)
-                bp = self._hold(at.proj.bias, torch.float32)
-                return self.conv([(o, Cc, 0, 1, False)], [(one, 0, 0, 0)], H, W, wp, Cc, bias=bp, res=x, out_dtype=self.res_dtype,
-                                 fuse_gn=next_gn)
-            # S = scale * Q K^T (fp32), per image
-            k_view = qk.view(B, N, 2 * Cc)[:, :, Cc:]
-            S = self.conv([(qk, Cc, 0, 1, False)], [(one, 0, 0, 0)], H, W, k_view, N, alpha=scale,
-                          out_fp32=True, w_batch_stride=N * 2 * Cc, w_pitch=2 * Cc)
-            P = self._new((B, H, W, N))
-            self._op(self.L.its_softmax_rows, P.data_ptr(), S.data_ptr(), B * N, N, kind="softmax")
-            bvh = self._hold(bv, torch.float32)
-            o = self.conv([(P, N, 0, 1, False)], [(one, 0, 0, 0)], H, W, vT.view(B, Cc, N), Cc, bias=bvh,
-                          w_batch_stride=Cc * N, want_stats=False)
-        elif (N in (32, 64) and Cc % 64 == 0 and Cc <= 512 and (Cc <= 256 or Cc % 128 == 0)
-              and self._impl_for([Cc], Cc) == 0 and self.fused_attention):
+                bvh = self._hold(bv)
+                self._op(core[1], o.data_ptr(), qk.data_ptr(), _ptr(vT), bvh.data_ptr(), B, N, Cc, scale,
+                         flops=flops, kind=core[0])
+            else:
+                # S = scale * Q K^T (fp32), per image
+                k_view = qk.view(B, N, 2 * Cc)[:, :, Cc:]
+                S = self.conv([(qk, Cc, 0, 1, False)], [(one, 0, 0, 0)], H, W, k_view, N, alpha=scale,
+                              out_fp32=True, w_batch_stride=N * 2 * Cc, w_pitch=2 * Cc)
+                P = self._new((B, H, W, N))
+                self._op(self.L.its_softmax_rows, P.data_ptr(), S.data_ptr(), B * N, N, kind="softmax")
+                bvh = self._hold(bv)
+                o = self.conv([(P, N, 0, 1, False)], [(one, 0, 0, 0)], H, W, vT.view(B, Cc, N), Cc, bias=bvh,
+                              w_batch_stride=Cc * N, want_stats=False)
+        elif N in (32, 64) and Cc % 64 == 0 and Cc <= 512 and (Cc <= 256 or Cc % 128 == 0) and on_tc:
             # small maps on the tensor cores: 128 / N images per tile, block-diagonal softmax mask.  (4x4 maps
             # stay on the CUDA-core kernel: at the design batch they are only 8 tiles, a latency-bound chain
             # of 13.6 us against 8.7 us for one CTA per query; the choice depends on the shape only, never on
             # the batch, so a candidate's numbers do not depend on what it is batched with.)
-            wqkv = self._hold(torch.cat([wq, wk, wv], 0), torch.float32)
-            bqk0 = self._hold(torch.cat([bq, bk, torch.zeros_like(bv)], 0), torch.float32)
-            qkv = self.conv([(a, Cc, 0, 1, False)], [(one, 0, 0, 0)], H, W, wqkv, 3 * Cc, bias=bqk0, want_stats=False)
+            qkv = project(torch.cat([wq, wk, wv]), torch.cat([bq, bk, torch.zeros_like(bv)]), 3 * Cc)
             o = self._new((B, H, W, Cc))
-            bvh = self._hold(bv, torch.float32)
+            bvh = self._hold(bv)
             self._op(self.L.its_attention_group, o.data_ptr(), qkv.data_ptr(), bvh.data_ptr(), B, N, Cc, scale,
-                     flops=4 * B * N * N * Cc, kind="attention_group")
+                     flops=flops, kind="attention_group")
         else:
-            wqkv = self._hold(torch.cat([wq, wk, wv], 0), torch.float32)
-            bqkv = self._hold(torch.cat([bq, bk, bv], 0), torch.float32)
-            qkv = self.conv([(a, Cc, 0, 1, False)], [(one, 0, 0, 0)], H, W, wqkv, 3 * Cc, bias=bqkv, want_stats=False)
+            qkv = project(torch.cat([wq, wk, wv]), torch.cat([bq, bk, bv]), 3 * Cc)
             o = self._new((B, H, W, Cc))
             self._op(self.L.its_attention_small, o.data_ptr(), qkv.data_ptr(), B, N, Cc, scale,
-                     flops=4 * B * N * N * Cc, kind="attention_small")
-        wp = self._hold(at.proj.weight.detach().float()[:, :, 0, 0], torch.float32)
-        bp = self._hold(at.proj.bias, torch.float32)
-        return self.conv([(o, Cc, 0, 1, False)], [(one, 0, 0, 0)], H, W, wp, Cc, bias=bp, res=x, out_dtype=self.res_dtype,
-                                 fuse_gn=next_gn)
+                     flops=flops, kind="attention_small")
+        wp, bp = self._hold(at.proj.weight.detach().float()[:, :, 0, 0]), self._hold(at.proj.bias)
+        return self.conv([(o, Cc, 0, 1, False)], [(one, 0, 0, 0)], H, W, wp, Cc, bias=bp, res=x,
+                         out_dtype=self.res_dtype, fuse_gn=next_gn)
 
     def _down(self, ds, x: torch.Tensor, next_gn=None) -> torch.Tensor:
         B, H, W, Cc = x.shape
@@ -626,170 +790,16 @@ class UNetPlan:
                  n_img_in, H, W, 3, ch, flops=2 * B * H * W * ch * 27, kind="conv_head")
         return h
 
-    # -------------------------------------------------------------- build --
-    def _build(self):
-        m, L = self.model, self.L
-        B, H, W = self.n_img, self.H, self.W
-        ch = m.head.out_channels
-        self.gn_partials = None
-        self.ws, self.split_k = None, True
-        self.stats_of, self.schedule, self.fold_residual = {}, 0, True
-        self.ws_persist, self.sm_count, self.fused_attention = None, 148, True
-        self.head_on_tensor_cores = True
-        # GroupNorm(+Swish) applied by the epilogue of the convolution that produces its input.  ITS_GN_FUSION:
-        # auto (default) = where it was measured to pay (_fusion_pays), 1 = wherever the tiling allows it,
-        # 0 = never (every GroupNorm as its own its_group_norm_apply launch, the round-1 plan)
-        self.prefused, self.n_gn_fused = {}, 0
-        self.gn_fusion = {"0": "off", "1": "all"}.get(_os.environ.get("ITS_GN_FUSION", "auto"), "auto")
-        if self.impl_forced is not None:
-            self.gn_fusion = "off"
-        # debugging switches (tests/parity triage): fall back to the simpler schedule of a stage
-        self.schedule = int(_os.environ.get("ITS_SCHEDULE", "0"))
-        self.fused_attention = _os.environ.get("ITS_FUSED_ATTENTION", "1") != "0"
-        self.head_on_tensor_cores = _os.environ.get("ITS_HEAD_TC", "1") != "0"
-        self.attn_v_mn = _os.environ.get("ITS_ATTN_VT", "0") != "1"
-        self.fork_time_chain = _os.environ.get("ITS_FORK_TIME", "1") != "0"
-        self._side = None
-        # Opt-in: raw feature maps (residual stream, conv1 outputs) in IEEE fp16 instead of bf16 — 5x smaller
-        # error per evaluation (DESIGN.md section 5), but the residual stream follows |x_t|: only for trained
-        # checkpoints / schedules whose state stays far below fp16's 65504 (an overflow surfaces as the
-        # sampler's "nan in tensor." assertion).  Model attribute `residual_fp16` or ITS_RESIDUAL_FP16=1.
-        want16 = bool(getattr(m, "residual_fp16", False)) or _os.environ.get("ITS_RESIDUAL_FP16", "0") == "1"
-        self.res_dtype = FP16 if (want16 and ch % 64 == 0 and self.impl_forced is None and FP16_GN) else BF16
-        self.gn_dtype = FP16 if (FP16_GN and ch % 64 == 0 and self.impl_forced != 1) else BF16
-        self.x_in = self._new((self.n_img_in, 3, H, W), torch.float32)
-        self.t_dev = torch.zeros(1, dtype=torch.int32, device=self.dev)
-        self.t_idx = torch.zeros(B, dtype=torch.int64, device=self.dev)
-        self.labels = torch.zeros(B, dtype=torch.int64, device=self.dev) if self.cond else None
-        rows = 1 if self.uniform_t else B
-        t_idx_ptr = None if self.uniform_t else self.t_idx.data_ptr()
-        te = m.time_embedding
-        emb = self._new((rows, ch), torch.float32)
-        if self.cond:
-            table = self._hold(te.timembedding[0].weight, torch.float32)
-            self._op(L.its_embed_rows, emb.data_ptr(), table.data_ptr(), t_idx_ptr, self.t_dev.data_ptr(), rows,
-                     ch, table.shape[0])
-            lin1, lin2 = te.timembedding[1], te.timembedding[3]
-        else:
-            freq = self._hold(te.freq_coeffs, torch.float32)
-            self._op(L.its_time_embed, emb.data_ptr(), t_idx_ptr, self.t_dev.data_ptr(), freq.data_ptr(), rows, ch)
-            lin1, lin2 = te.timembedding[0], te.timembedding[2]
-        hmid = self.linear(emb, self._hold(lin1.weight, torch.float32), self._hold(lin1.bias, torch.float32),
-                           silu_out=True)
-        temb = self.linear(hmid, self._hold(lin2.weight, torch.float32), self._hold(lin2.bias, torch.float32))
-        # every ResBlock's temb_proj (and cond_proj) as ONE linear over concatenated weights
-        blocks = [b for b in list(m.downblocks) + list(m.middleblocks) + list(m.upblocks) if hasattr(b, "temb_proj")]
-        offs, o = {}, 0
-        for rb in blocks:
-            offs[id(rb)] = o
-            o += rb.temb_proj[1].out_features
-        wt = self._hold(torch.cat([rb.temb_proj[1].weight.detach().float() for rb in blocks], 0), torch.float32)
-        bt = self._hold(torch.cat([rb.temb_proj[1].bias.detach().float() for rb in blocks], 0), torch.float32)
-        self.tproj = self.linear(temb, wt, bt, silu_in=True)
-        # The time-embedding chain (embedding -> two linears -> every temb_proj) depends on t only; the head
-        # (patch gather, head GEMM, first GroupNorm) depends on x only.  run() forks the chain onto a side
-        # stream and joins before the first launch that adds the projected embedding.
-        self._n_time_ops = len(self.ops)
-        self._join_at = None
-        self.cproj = None
-        if self.cond:
-            # Everything from the label embedding to the per-ResBlock cond_proj vectors is a function of
-            # the labels alone (ModelCondition.py:216,131-135,154).  The labels of a trajectory never
-            # change, so the sampler runs these launches once per forward() instead of once per step;
-            # UNet.forward() runs them on every call.
-            self._into_label_ops = True
-            ce = m.cond_embedding.condEmbedding
-            ctab = self._hold(ce[0].weight, torch.float32)
-            cemb0 = self._new((B, ch), torch.float32)
-            self._op(L.its_embed_rows, cemb0.data_ptr(), ctab.data_ptr(), self.labels.data_ptr(), None, B, ch,
-                     ctab.shape[0])
-            c1 = self.linear(cemb0, self._hold(ce[1].weight, torch.float32), self._hold(ce[1].bias, torch.float32),
-                             silu_out=True)
-            cemb = self.linear(c1, self._hold(ce[3].weight, torch.float32), self._hold(ce[3].bias, torch.float32))
-            wc = self._hold(torch.cat([rb.cond_proj[1].weight.detach().float() for rb in blocks], 0), torch.float32)
-            bc = self._hold(torch.cat([rb.cond_proj[1].bias.detach().float() for rb in blocks], 0), torch.float32)
-            self.cproj = self.linear(cemb, wc, bc, silu_in=True)
-            self._into_label_ops = False
-        # ---- head
-        # The GroupNorm -> Swish that the NEXT layer opens with, when that layer reads this layer's output alone
-        # (down path, middle, tail): the producing launch applies it in its epilogue.  Up-path ResBlocks
-        # normalise the concatenation [h, skip] (their groups mix both tensors) and resampling convs read
-        # the raw tensor: no fusion there.
-        seq = list(m.downblocks) + list(m.middleblocks)
-
-        def opens_with(layer):
-            return (layer.block1[0], True) if hasattr(layer, "temb_proj") else None
-
-        nxt = {id(a): opens_with(b) for a, b in zip(seq[:-1], seq[1:])}
-        ups = list(m.upblocks)
-        h = self.head_conv(m.head.weight, m.head.bias, self.x_in, B, H, W, next_gn=opens_with(seq[0]))
-        hs = [h]
-        for layer in m.downblocks:
-            if hasattr(layer, "temb_proj"):
-                h = self._res_block(layer, [h], offs[id(layer)], nxt.get(id(layer)))
-            else:
-                h = self._down(layer, h, nxt.get(id(layer)))
-            hs.append(h)
-        for layer in m.middleblocks:
-            h = self._res_block(layer, [h], offs[id(layer)], nxt.get(id(layer)))
-        for i, layer in enumerate(ups):
-            if hasattr(layer, "temb_proj"):
-                h = self._res_block(layer, [h, hs.pop()], offs[id(layer)], (m.tail[0], True) if i == len(ups) - 1 else None)
-            else:
-                h = self._up(layer, h)
-        assert len(hs) == 0
-        a = self.group_norm([h], m.tail[0], silu=True)
-        self.eps = self._new((B, 3, H, W), torch.float32)
-        ct = a.shape[3]
+    def _tail_conv(self, conv, a: torch.Tensor) -> None:
+        """Model.py:257-262: conv3x3(ch -> 3) of the tail GroupNorm's output into eps (NCHW fp32)."""
+        B, H, W, ct = a.shape
         if self._impl_for([ct], 3, True) == 0:
             # 3-channel tail on the tensor cores: N tile of 32 (rows 3..31 of the weight box are
             # TMA zero fill), epilogue writes NCHW fp32 directly (coalesced over pixels)
-            tw = self._hold(pack_conv_weight(m.tail[2].weight), torch.float32)
-            tb = self._hold(m.tail[2].bias, torch.float32)
+            tw, tb = self._hold(pack_conv_weight(conv.weight)), self._hold(conv.bias)
             self.conv([(a, ct, 0, 1, False)], [(taps_square(3), 0, 0, 0)], H, W, tw, 3, bias=tb, out=self.eps,
                       out_fp32=True, out_nchw=True)
         else:
-            tw, tb = self._hold(m.tail[2].weight, torch.float32), self._hold(m.tail[2].bias, torch.float32)
-            self._op(L.its_conv_tail, self.eps.data_ptr(), a.data_ptr(), tw.data_ptr(), tb.data_ptr(), B, a.shape[1],
-                     a.shape[2], ct, 3, flops=2 * B * H * W * 3 * 9 * ct, kind="conv_tail")
-
-    # ---------------------------------------------------------------- run --
-    def run_label_ops(self) -> None:
-        """Enqueue the launches that depend on `self.labels` only (conditional net; no-op otherwise).
-        Must run after every change of the labels and before run()."""
-        s = _lib.stream_ptr()
-        for fn, args in self.label_ops:
-            rc = fn(*args, s)
-            if rc != 0:
-                _lib.check(rc, fn.__name__)
-
-    def run(self) -> None:
-        """Enqueue every launch on the current stream (graph-capturable).  The time-embedding chain runs
-        on a side stream next to the head of the network (fork / join by events, so the pair is two
-        parallel branches of the captured step graph)."""
-        s = _lib.stream_ptr()
-        n_time = getattr(self, "_n_time_ops", 0)
-        join_at = getattr(self, "_join_at", None)
-        fork = self.fork_time_chain and n_time > 0 and join_at is not None and join_at > n_time
-        if fork:
-            if self._side is None:
-                self._side = torch.cuda.Stream(device=self.dev)
-                self._ev_fork, self._ev_join = torch.cuda.Event(), torch.cuda.Event()
-            main = torch.cuda.current_stream()
-            self._ev_fork.record(main)
-            self._side.wait_event(self._ev_fork)
-            s_side = self._side.cuda_stream
-            for fn, args in self.ops[:n_time]:
-                rc = fn(*args, s_side)
-                if rc != 0:
-                    _lib.check(rc, fn.__name__)
-            self._ev_join.record(self._side)
-        for i, (fn, args) in enumerate(self.ops):
-            if fork:
-                if i < n_time:
-                    continue
-                if i == join_at:
-                    torch.cuda.current_stream().wait_event(self._ev_join)
-            rc = fn(*args, s)
-            if rc != 0:
-                _lib.check(rc, fn.__name__)
+            tw, tb = self._hold(conv.weight), self._hold(conv.bias)
+            self._op(self.L.its_conv_tail, self.eps.data_ptr(), a.data_ptr(), tw.data_ptr(), tb.data_ptr(), B, H, W,
+                     ct, 3, flops=2 * B * H * W * 3 * 9 * ct, kind="conv_tail")

@@ -3,71 +3,27 @@
 The reference is fp32 end to end (Diffusion/Diffusion.py:74-99 over Model.py / ModelCondition.py) and north_star
 states 1e-4 on the samples for an fp32 mode.  This plan evaluates the UNet with the `its_f32_*` kernels of
 libits_b200 (csrc/fp32_path.cu): NHWC fp32 activations, fp32 weights, one launch per reference operation, in the
-reference's own order.  It has the interface of `engine.UNetPlan` (x_in / t_dev / t_idx / labels / eps, run(),
-run_label_ops(), graph-capturable launches on the caller's stream), so the samplers, the searches and the
-drivers use it unchanged.  It is the parity instrument and an independent on-device cross-check of the tcgen05
-plan — CUDA-core arithmetic, roughly two orders of magnitude slower than the 16-bit plan.
+reference's own order.  It is an `engine.PlanBase`, so the network walk, the time / label chains, the buffers
+(x_in / t_dev / t_idx / labels / eps) and run() / run_label_ops() are the ones of the 16-bit plan; only the layers
+differ.  The samplers, the searches and the drivers use it unchanged.  It is the parity instrument and an
+independent on-device cross-check of the tcgen05 plan — CUDA-core arithmetic, roughly two orders of magnitude
+slower than the 16-bit plan.
 """
 from __future__ import annotations
 
-from typing import List, Optional, Tuple
+from typing import List
 
 import torch
 
-from . import _lib
+from .engine import PlanBase, _ptr
 
 F32 = torch.float32
 
 
-class UNetPlanF32:
-    """Launch plan of one fp32 UNet evaluation for n_img images of H x W."""
+class UNetPlanF32(PlanBase):
+    """Launch plan of one fp32 UNet evaluation for n_img images of H x W (`impl` is ignored)."""
 
-    def __init__(self, model, n_img: int, H: int, W: int, *, n_img_in: Optional[int] = None,
-                 uniform_t: bool = False, impl: Optional[int] = None):
-        _lib.require_cuda()
-        self.L = _lib.lib()
-        self.model = model
-        self.cond = bool(getattr(model, "is_conditional", False))
-        self.n_img, self.H, self.W = int(n_img), int(H), int(W)
-        self.n_img_in = int(n_img_in or n_img)
-        self.uniform_t = uniform_t
-        self.dev = model.head.weight.device
-        if self.dev.type != "cuda":
-            raise RuntimeError("its_b200 UNet must live on a CUDA device (no CPU fallback); call .cuda()")
-        self.keep: List[torch.Tensor] = []
-        self.ops: List[Tuple] = []
-        self.label_ops: List[Tuple] = []
-        self.op_info: List[Tuple[str, int, int]] = []
-        self.n_launches = self.n_label_launches = 0
-        self.flops = 0
-        self._into_label_ops = False
-        with torch.no_grad():
-            self._build()
-
-    # ---------------------------------------------------------------- helpers --
-    def _new(self, shape) -> torch.Tensor:
-        t = torch.empty(tuple(int(s) for s in shape), dtype=F32, device=self.dev)
-        self.keep.append(t)
-        return t
-
-    def _hold(self, t: torch.Tensor) -> torch.Tensor:
-        t = t.detach().to(device=self.dev, dtype=F32).contiguous()
-        self.keep.append(t)
-        return t
-
-    def _op(self, fn, *args, flops: int = 0, kind: str = "other"):
-        if self._into_label_ops:
-            self.label_ops.append((fn, args))
-            self.n_label_launches += 1
-            return
-        self.ops.append((fn, args))
-        self.op_info.append((kind, flops, 1))
-        self.n_launches += 1
-        self.flops += flops
-
-    @staticmethod
-    def _ptr(t):
-        return None if t is None else t.data_ptr()
+    ACT_DTYPE = F32
 
     def _pack(self, w: torch.Tensor, transposed: bool = False) -> torch.Tensor:
         """OIHW (or ConvTranspose2d's [Cin][Cout][k][k]) -> [k*k][Cin][CoutP] fp32, CoutP = Cout rounded up to 4."""
@@ -100,8 +56,8 @@ class UNetPlanF32:
             return v.data_ptr() + 4 * off, (0 if v.shape[0] == 1 else v.shape[1])
         vp, vs = vptr(vec, vec_off)
         vp2, vs2 = vptr(vec2, vec2_off)
-        self._op(self.L.its_f32_conv2d, out.data_ptr(), x0.data_ptr(), C0, self._ptr(x1), C1, wt.data_ptr(), self._ptr(b),
-                 vp, vs, vp2, vs2, self._ptr(res), B, Hin, Win, cout, k, stride, mode, int(out_nchw),
+        self._op(self.L.its_f32_conv2d, out.data_ptr(), x0.data_ptr(), C0, _ptr(x1), C1, wt.data_ptr(), _ptr(b),
+                 vp, vs, vp2, vs2, _ptr(res), B, Hin, Win, cout, k, stride, mode, int(out_nchw),
                  flops=2 * B * Hout * Wout * cout * (C0 + C1) * k * k // (4 if mode == 2 else 1), kind="f32_conv2d")
         return out
 
@@ -111,22 +67,13 @@ class UNetPlanF32:
         B, H, W, C0 = x0.shape
         C1 = x1.shape[-1] if x1 is not None else 0
         out = self._new((B, H, W, C0 + C1))
-        self._op(self.L.its_f32_group_norm, out.data_ptr(), x0.data_ptr(), C0, self._ptr(x1), C1,
+        self._op(self.L.its_f32_group_norm, out.data_ptr(), x0.data_ptr(), C0, _ptr(x1), C1,
                  self._hold(gn.weight).data_ptr(), self._hold(gn.bias).data_ptr(), B, H * W, gn.num_groups,
                  float(gn.eps), int(silu), kind="f32_group_norm")
         return out
 
-    def linear(self, x: torch.Tensor, lin, *, silu_in=False, silu_out=False, W=None, b=None) -> torch.Tensor:
-        W = self._hold(lin.weight) if W is None else W
-        b = self._hold(lin.bias) if b is None else b
-        rows, K = x.shape
-        y = self._new((rows, W.shape[0]))
-        self._op(self.L.its_linear, y.data_ptr(), x.data_ptr(), W.data_ptr(), b.data_ptr(), rows, K, W.shape[0],
-                 int(silu_in), int(silu_out), 0, flops=2 * rows * K * W.shape[0], kind="linear")
-        return y
-
     # ----------------------------------------------------------------- blocks --
-    def _res_block(self, rb, xs: List[torch.Tensor], off: int) -> torch.Tensor:
+    def _res_block(self, rb, xs: List[torch.Tensor], off: int, next_gn=None) -> torch.Tensor:
         """Model.py:167-209 / ModelCondition.py:121-161."""
         a1 = self.group_norm(xs, rb.block1[0], True)
         h = self.conv([a1], rb.block1[2].weight, rb.block1[2].bias, vec=self.tproj, vec_off=off, vec2=self.cproj,
@@ -156,7 +103,7 @@ class UNetPlanF32:
                  flops=4 * B * H * W * H * W * Cc, kind="f32_attention")
         return self.conv([o], at.proj.weight, at.proj.bias, res=x)
 
-    def _down(self, ds, x: torch.Tensor) -> torch.Tensor:
+    def _down(self, ds, x: torch.Tensor, next_gn=None) -> torch.Tensor:
         if hasattr(ds, "main"):                                       # Model.py:96-108
             return self.conv([x], ds.main.weight, ds.main.bias, stride=2)
         t = self.conv([x], ds.c1.weight, ds.c1.bias, stride=2)       # ModelCondition.py:65-73: c1(x) + c2(x)
@@ -168,80 +115,11 @@ class UNetPlanF32:
         t = self.conv([x], us.t.weight, us.t.bias, stride=2, mode=2, transposed=True)   # ModelCondition.py:76-86
         return self.conv([t], us.c.weight, us.c.bias)
 
-    # ------------------------------------------------------------------ build --
-    def _build(self):
-        m, L = self.model, self.L
-        B, H, W = self.n_img, self.H, self.W
-        ch = m.head.out_channels
-        self.x_in = self._new((self.n_img_in, 3, H, W))
-        self.t_dev = torch.zeros(1, dtype=torch.int32, device=self.dev)
-        self.t_idx = torch.zeros(B, dtype=torch.int64, device=self.dev)
-        self.labels = torch.zeros(B, dtype=torch.int64, device=self.dev) if self.cond else None
-        rows = 1 if self.uniform_t else B
-        t_idx_ptr = None if self.uniform_t else self.t_idx.data_ptr()
-        te = m.time_embedding
-        emb = self._new((rows, ch))
-        if self.cond:
-            table = self._hold(te.timembedding[0].weight)
-            self._op(L.its_embed_rows, emb.data_ptr(), table.data_ptr(), t_idx_ptr, self.t_dev.data_ptr(), rows, ch,
-                     table.shape[0])
-            lin1, lin2 = te.timembedding[1], te.timembedding[3]
-        else:
-            freq = self._hold(te.freq_coeffs)
-            self._op(L.its_time_embed, emb.data_ptr(), t_idx_ptr, self.t_dev.data_ptr(), freq.data_ptr(), rows, ch)
-            lin1, lin2 = te.timembedding[0], te.timembedding[2]
-        temb = self.linear(self.linear(emb, lin1, silu_out=True), lin2)
-        blocks = [b for b in list(m.downblocks) + list(m.middleblocks) + list(m.upblocks) if hasattr(b, "temb_proj")]
-        offs, o = {}, 0
-        for rb in blocks:
-            offs[id(rb)] = o
-            o += rb.temb_proj[1].out_features
-        wt = self._hold(torch.cat([rb.temb_proj[1].weight.detach().float() for rb in blocks], 0))
-        bt = self._hold(torch.cat([rb.temb_proj[1].bias.detach().float() for rb in blocks], 0))
-        self.tproj = self.linear(temb, None, silu_in=True, W=wt, b=bt)          # Model.py:181-184, every block at once
-        self.cproj = None
-        if self.cond:
-            self._into_label_ops = True       # functions of the labels only (ModelCondition.py:216,131-135)
-            ce = m.cond_embedding.condEmbedding
-            ctab = self._hold(ce[0].weight)
-            cemb0 = self._new((B, ch))
-            self._op(L.its_embed_rows, cemb0.data_ptr(), ctab.data_ptr(), self.labels.data_ptr(), None, B, ch,
-                     ctab.shape[0])
-            cemb = self.linear(self.linear(cemb0, ce[1], silu_out=True), ce[3])
-            wc = self._hold(torch.cat([rb.cond_proj[1].weight.detach().float() for rb in blocks], 0))
-            bc = self._hold(torch.cat([rb.cond_proj[1].bias.detach().float() for rb in blocks], 0))
-            self.cproj = self.linear(cemb, None, silu_in=True, W=wc, b=bc)
-            self._into_label_ops = False
+    def head_conv(self, weight, bias, x_in: torch.Tensor, B: int, H: int, W: int, next_gn=None) -> torch.Tensor:
+        """Model.py:269 on the NCHW fp32 sampler state (broadcast over n_img / n_img_in)."""
         x = self._new((B, H, W, 3))
-        self._op(L.its_f32_nchw_to_nhwc, x.data_ptr(), self.x_in.data_ptr(), B, self.n_img_in, 3, H, W, kind="layout")
-        h = self.conv([x], m.head.weight, m.head.bias)                           # Model.py:269
-        hs = [h]
-        for layer in m.downblocks:
-            h = self._res_block(layer, [h], offs[id(layer)]) if hasattr(layer, "temb_proj") else self._down(layer, h)
-            hs.append(h)
-        for layer in m.middleblocks:
-            h = self._res_block(layer, [h], offs[id(layer)])
-        for layer in m.upblocks:
-            if hasattr(layer, "temb_proj"):
-                h = self._res_block(layer, [h, hs.pop()], offs[id(layer)])       # torch.cat([h, hs.pop()], 1)
-            else:
-                h = self._up(layer, h)
-        assert len(hs) == 0
-        a = self.group_norm([h], m.tail[0], True)
-        self.eps = self._new((B, 3, H, W))
-        self.conv([a], m.tail[2].weight, m.tail[2].bias, out=self.eps, out_nchw=True)   # Model.py:257-262
+        self._op(self.L.its_f32_nchw_to_nhwc, x.data_ptr(), x_in.data_ptr(), B, x_in.shape[0], 3, H, W, kind="layout")
+        return self.conv([x], weight, bias)
 
-    # -------------------------------------------------------------------- run --
-    def run_label_ops(self) -> None:
-        s = _lib.stream_ptr(self.dev)
-        for fn, args in self.label_ops:
-            rc = fn(*args, s)
-            if rc != 0:
-                _lib.check(rc, fn.__name__)
-
-    def run(self) -> None:
-        s = _lib.stream_ptr(self.dev)
-        for fn, args in self.ops:
-            rc = fn(*args, s)
-            if rc != 0:
-                _lib.check(rc, fn.__name__)
+    def _tail_conv(self, conv, a: torch.Tensor) -> None:
+        self.conv([a], conv.weight, conv.bias, out=self.eps, out_nchw=True)     # Model.py:257-262
