@@ -377,6 +377,14 @@ int its_argmax_first(int32_t* idx_out, float* val_out, const float* scores,
  * winner (search_algorithm.py:79-81); north_star's "top-k/argmax" — used for keeping several pivots.       */
 int its_topk_first(int32_t* idx_out, float* val_out, const float* scores,
                    int32_t n, int32_t k, void* stream);
+/* The same selection in n_seg independent segments, one CTA each: segment s is scores[s*seg_len, (s+1)*seg_len)
+ * and its k best go to idx_out[s*k + r], val_out[s*k + r].  Indices are flat (s*seg_len + local), so the
+ * output can be passed unchanged as its_path_expand's parent array over the whole population; -1 / -inf past
+ * a segment's eligible scores.  Generalises the reference's per-search winner (search_algorithm.py:79-81) to
+ * one winner (k = 1) or k survivors per query of a batch of searches.  its_topk_first is the n_seg = 1 case.
+ * Requires n_seg, seg_len, k >= 1 and n_seg * seg_len <= INT32_MAX; no allocation, no synchronisation.   */
+int its_topk_first_segmented(int32_t* idx_out, float* val_out, const float* scores,
+                             int32_t n_seg, int32_t seg_len, int32_t k, void* stream);
 
 /* ------------------------------------------------------------------------
  * fp32-grade path (precision = "fp32").  The reference computes everything in

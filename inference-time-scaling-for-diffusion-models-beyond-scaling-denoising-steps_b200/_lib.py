@@ -22,7 +22,7 @@ SYMBOLS = [
     "its_group_norm_apply", "its_conv_stats_parts", "its_set_pdl", "its_attention_fused", "its_head_patches",
     "its_attention_flash", "its_attention_group", "its_conv_gn_sync_words",
     "its_f32_nchw_to_nhwc", "its_f32_conv2d", "its_f32_group_norm", "its_f32_attention",
-    "its_topk_first", "its_ddpm_step_x0", "its_path_expand",
+    "its_topk_first", "its_ddpm_step_x0", "its_path_expand", "its_topk_first_segmented",
 ]
 
 
@@ -112,6 +112,7 @@ def lib() -> C.CDLL:
     L.its_candidate_scores.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp]
     L.its_argmax_first.argtypes = [vp, vp, vp, i32, vp]
     L.its_topk_first.argtypes = [vp, vp, vp, i32, i32, vp]
+    L.its_topk_first_segmented.argtypes = [vp, vp, vp, i32, i32, i32, vp]
     for s in SYMBOLS:
         if s not in ("its_version", "its_last_error_string"):
             getattr(L, s).restype = i32

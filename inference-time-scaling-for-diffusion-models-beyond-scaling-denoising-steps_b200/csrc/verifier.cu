@@ -1,5 +1,5 @@
 // Verifier statistics, per-candidate scores and first-index argmax
-// (search/verifier.py:45-66, 207-248, 262-287; search/search_algorithm.py:79-81).
+// and (segmented) top-k (search/verifier.py:45-66, 207-248, 262-287; search/search_algorithm.py:79-81).
 // All reductions are warp-shuffle + one shared-memory hop.
 #include "its_common.cuh"
 
@@ -163,18 +163,22 @@ __global__ void __launch_bounds__(1024) argmax_first_kernel(int* __restrict__ id
 
 // Top-k selection, same ordering rule applied k times: rank r is the first index of the largest score that comes
 // after rank r-1 in the order (score descending, index ascending).  NaN and -inf never rank; ranks beyond the
-// number of eligible scores get index -1.  One block, warp-shuffle + shared-memory reduction per rank.
+// number of eligible scores get index -1.  One block per segment: block s ranks scores[s*seg_len, (s+1)*seg_len)
+// and writes flat indices (s*seg_len + local) to idx_out[s*k + r].  Warp-shuffle + shared-memory reduction per rank.
 __global__ void __launch_bounds__(1024) topk_first_kernel(int* __restrict__ idx_out, float* __restrict__ val_out,
-                                                          const float* __restrict__ scores, int n, int k) {
+                                                          const float* __restrict__ scores, int seg_len, int k) {
   pdl_prologue();
   __shared__ float s_v[32];
   __shared__ int s_i[32];
   __shared__ Best s_prev;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int base = blockIdx.x * seg_len, end = base + seg_len;   // n_seg * seg_len fits int32 (checked on the host)
+  idx_out += (long long)blockIdx.x * k;
+  val_out += (long long)blockIdx.x * k;
   Best prev = {INFINITY, -1};
   for (int r = 0; r < k; ++r) {
     Best b = {-INFINITY, -1};
-    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+    for (int i = base + threadIdx.x; i < end; i += blockDim.x) {
       const float v = scores[i];
       const bool after = r == 0 || v < prev.v || (v == prev.v && i > prev.i);
       if (after && v > b.v) { b.v = v; b.i = i; }
@@ -242,10 +246,23 @@ extern "C" int its_argmax_first(int32_t* idx_out, float* val_out, const float* s
   return ITS_OK;
 }
 
+extern "C" int its_topk_first_segmented(int32_t* idx_out, float* val_out, const float* scores, int32_t n_seg,
+                                        int32_t seg_len, int32_t k, void* stream) {
+  ITS_REQUIRE(idx_out && val_out && scores, "its_topk_first_segmented: null pointer");
+  ITS_REQUIRE(n_seg > 0 && seg_len > 0 && k > 0, "its_topk_first_segmented: n_seg=%d seg_len=%d k=%d must be >= 1",
+              n_seg, seg_len, k);
+  ITS_REQUIRE((long long)n_seg * seg_len <= INT32_MAX,
+              "its_topk_first_segmented: n_seg * seg_len = %lld exceeds int32", (long long)n_seg * seg_len);
+  // one warp per 32 scores of a segment, up to 32 warps: search populations are tens to hundreds per segment
+  const int threads = seg_len >= 1024 ? 1024 : (seg_len + 31) / 32 * 32;
+  ITS_LAUNCH(its::topk_first_kernel, dim3(n_seg), dim3(threads), 0, its::as_stream(stream), idx_out, val_out, scores,
+             seg_len, k);
+  ITS_CHECK_LAUNCH();
+  return ITS_OK;
+}
+
 extern "C" int its_topk_first(int32_t* idx_out, float* val_out, const float* scores, int32_t n, int32_t k,
                               void* stream) {
   ITS_REQUIRE(idx_out && val_out && scores && n > 0 && k > 0, "its_topk_first: bad arguments");
-  ITS_LAUNCH(its::topk_first_kernel, dim3(1), dim3(1024), 0, its::as_stream(stream), idx_out, val_out, scores, n, k);
-  ITS_CHECK_LAUNCH();
-  return ITS_OK;
+  return its_topk_first_segmented(idx_out, val_out, scores, 1, n, k, stream);
 }

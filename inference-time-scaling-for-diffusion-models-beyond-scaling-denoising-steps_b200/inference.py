@@ -282,6 +282,9 @@ def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Op
     img_size.  search_over_paths takes n_beams (4), n_children (4), start_step (800), delta_f (50) and
     delta_b (100), and returns the winner's initial x_T with the images the search itself finished (the winner's
     path is re-noised along the way: denoising its x_T again would not reproduce it).
+    `n_queries` (K, default 1) > 1 runs K independent random / search_over_paths searches as one population
+    (`search_batch`): `labels` is then [K] or [K, B] (one row per query), and the results are stacked over the
+    queries (best_noise and images [K, B, 3, H, W], a list of K scores).
     With torch.distributed initialised the candidates are sharded over the ranks."""
     from .search import search_algorithm as S
     sc = dict(config.get("search") or {})
@@ -289,6 +292,9 @@ def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Op
     B, H = int(config.get("batch_size", 1)), int(config["img_size"])
     shape = (B, 3, H, H)
     ver = make_verifier(sc.get("verifier", "oracle"))
+    K = int(sc.get("n_queries", 1))
+    if K > 1:
+        return _run_batch(sampler, sc, algo, K, shape, ver, device, labels=labels, seed=seed)
     den = S.make_denoise_fn(sampler, labels, max_images=int(sc.get("max_images", 256)), seed=seed)
     dev = str(device)
     if algo == "search_over_paths":
@@ -323,6 +329,35 @@ def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Op
     return best, score, images
 
 
+def _run_batch(sampler, sc: Dict[str, Any], algo: str, K: int, shape, ver, device, *, labels=None,
+               seed: Optional[int] = None):
+    """run_search for n_queries = K > 1: one `search_batch` over K queries."""
+    from .search import search_algorithm as S
+    batched = ("random", "search_over_paths")
+    if algo not in batched:
+        raise ValueError(f"search.n_queries={K} needs search.algorithm in {list(batched)}, got {algo!r}")
+    den = S.make_denoise_fn(sampler, max_images=int(sc.get("max_images", 256)), seed=seed)
+    dev = torch.device(device)
+    if algo == "search_over_paths":
+        search = S.SearchOverPaths(n_beams=int(sc.get("n_beams", 4)), n_children=int(sc.get("n_children", 4)),
+                                   start_step=int(sc.get("start_step", 800)), delta_f=int(sc.get("delta_f", 50)),
+                                   delta_b=int(sc.get("delta_b", 100)))
+        images, scores, _ = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev))
+        best = torch.stack([S.philox_normal((1,) + shape, search.last_seed, q * search.n_beams + p, S.TAG_X_T, dev)[0]
+                            for q, p in enumerate(search.last_index)])
+        return best, scores, images
+    search = S.RandomSearch(n_candidates=int(sc.get("n_candidates", 4)))
+    best, scores = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev))
+    # each winner's images from its own trajectory (the global candidate id it was scored under)
+    images = torch.full_like(best, float("nan"))
+    rows = None if labels is None else labels.to(dev, torch.int64).reshape(K, -1).expand(K, shape[0])
+    for q, i in enumerate(search.last_index):
+        if i >= 0:
+            images[q] = den.denoise_candidates(best[q:q + 1], q * search.n_candidates + i, seed=search.last_seed,
+                                               cand_labels=None if rows is None else rows[q:q + 1])[0]
+    return best, scores, images
+
+
 def save_image_grid(images: torch.Tensor, path: str, nrow: int = 8) -> str:
     """[-1, 1] samples -> [0, 1] PNG grid (abstract_metrics_from_pretrained_ddpm.py:621-628)."""
     from torchvision.utils import save_image
@@ -349,12 +384,19 @@ def main(argv: Optional[List[str]] = None) -> int:
     sampler = create_sampler(model, cfg, device)
     sampler.print_steps = False
     labels = None
+    K = int((cfg.get("search") or {}).get("n_queries", 1))
     if getattr(model, "is_conditional", False):
+        # query q's labels are 1 + (q*B + arange(B)) % num_labels; a single search takes query 0's
         B = int(cfg.get("batch_size", 1))
-        labels = (1 + torch.arange(B, device=device) % int(cfg["num_labels"])).to(torch.int64)
+        labels = (1 + torch.arange(K * B, device=device) % int(cfg["num_labels"])).to(torch.int64)
+        labels = labels.view(K, B) if K > 1 else labels
     if cfg.get("search"):
         best, score, images = run_search(sampler, cfg, device, labels=labels, seed=cfg.get("seed"))
-        print(f"search: best score {score:.6f}")
+        if K > 1:
+            print("search: best scores " + " ".join(f"{v:.6f}" for v in score))
+            images = images.reshape(-1, *images.shape[2:])       # the grid holds all K*B winning images
+        else:
+            print(f"search: best score {score:.6f}")
     else:
         B, H = int(cfg.get("batch_size", 1)), int(cfg["img_size"])
         x_T = torch.randn(B, 3, H, H, device=device)

@@ -24,6 +24,10 @@ true mid-trajectory restart at `injection_step`).
 SearchOverPaths is not in the reference: it is the search over paths of Ma et al. (a beam of partial
 trajectories, re-noised and pruned by top-k on x0 predictions), in population mode only.
 
+Batched searches (not in the reference): `RandomSearch.search_batch` and `SearchOverPaths.search_batch` run K
+independent queries, each with its own labels, as one candidate population and select every query's winner
+(or survivors) on the device with one segmented top-k.  `search` is the K = 1 case of the same code.
+
 GradientBasedSearch (:343-438) needs autograd through the whole trajectory: it is kept
 for arbitrary differentiable callables (callable mode only, the reference's loop); the
 kernel sampler is not differentiable and is refused with a clear error.
@@ -94,23 +98,30 @@ class SamplerDenoiser:
         return self.denoise_candidates(noise.unsqueeze(0), i, labels=kwargs.get("labels"))[0]
 
     def denoise_candidates(self, cands: torch.Tensor, first_cand: int, *, labels=None,
-                           t_start: Optional[int] = None, seed: Optional[int] = None, t_stop: int = 0) -> torch.Tensor:
+                           t_start: Optional[int] = None, seed: Optional[int] = None, t_stop: int = 0,
+                           cand_labels: Optional[torch.Tensor] = None) -> torch.Tensor:
         """cands [n, B, C, H, W] -> images [n, B, C, H, W]; candidate i is global
         candidate first_cand + i (its Philox streams are keyed by that id).  `t_start` (default T-1) and `t_stop`
         bound the loop as the sampler's own arguments do (a `t_stop` > 0 returns the states step t_stop - 1
         starts from)."""
         t_start = self.sampler.T - 1 if t_start is None else t_start
         return self.denoise_segment(cands, first_cand, t_start=t_start, t_stop=t_stop, labels=labels, seed=seed,
-                                    x0=False)[0]
+                                    x0=False, cand_labels=cand_labels)[0]
 
     def denoise_segment(self, states: torch.Tensor, first_cand: int, *, t_start: int, t_stop: int,
                         cand_offset: int = 0, labels=None, seed: Optional[int] = None,
-                        x0: bool = True) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+                        x0: bool = True, cand_labels: Optional[torch.Tensor] = None
+                        ) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
         """states [n, B, C, H, W] at step t_start -> (states after step t_stop, x0 predictions of step t_stop or
         None), in chunks of `max_images`.  Candidate i's per-step Philox streams are keyed by
-        cand_offset + (first_cand + i) * B + image; every chunk replays the sampler's one step graph."""
+        cand_offset + (first_cand + i) * B + image; every chunk replays the sampler's one step graph.  The guided
+        sampler's labels are `cand_labels` [n, B] (int64, one row per candidate) when given, else `labels` (or the
+        denoiser's own) [B] for every candidate."""
         n, B = states.shape[:2]
         guided = getattr(self.sampler, "guided", False)
+        if cand_labels is not None and tuple(cand_labels.shape) != (n, B):
+            raise ValueError(f"cand_labels must be [{n}, {B}] (one label row per candidate), got "
+                             f"{tuple(cand_labels.shape)}")
         per_call = max(1, self.max_images // B)
         out = torch.empty_like(states)
         out_x0 = torch.empty_like(states) if x0 else None
@@ -122,7 +133,13 @@ class SamplerDenoiser:
                                       cand_id0=cand_offset + (first_cand + i0) * B, x0=x0)
             if self.step_noise is not None:
                 kw["noise"] = self.step_noise.repeat(1, i1 - i0, 1, 1, 1)
-            y, p = self.sampler.segment(x, self._labels_for(i1 - i0, labels) if guided else None, **kw)
+            if not guided:
+                lab = None
+            elif cand_labels is not None:
+                lab = cand_labels[i0:i1].reshape(-1)
+            else:
+                lab = self._labels_for(i1 - i0, labels)
+            y, p = self.sampler.segment(x, lab, **kw)
             out[i0:i1] = y.view(i1 - i0, B, *states.shape[2:])
             if x0:
                 out_x0[i0:i1] = p.view(i1 - i0, B, *states.shape[2:])
@@ -220,15 +237,19 @@ def argmax_first(scores: torch.Tensor) -> Tuple[int, float]:
     return int(idx.item()), float(val.item())
 
 
-def _topk_device(scores: torch.Tensor, k: int) -> Tuple[torch.Tensor, torch.Tensor]:
-    """topk_first with the (int32 indices, fp32 values) left on the device."""
+def _topk_device(scores: torch.Tensor, k: int, n_seg: int = 1) -> Tuple[torch.Tensor, torch.Tensor]:
+    """topk_first of each of `n_seg` equal segments of `scores`, with the (int32 indices, fp32 values) left on the
+    device: [n_seg * k], segment s's ranks at s*k ... s*k + k - 1, indices flat into `scores`."""
     _lib.require_cuda()
     s = scores.detach().to(torch.float32).contiguous()
-    idx = torch.empty(k, dtype=torch.int32, device=s.device)
-    val = torch.empty(k, dtype=torch.float32, device=s.device)
+    if n_seg < 1 or s.numel() % n_seg:
+        raise ValueError(f"{s.numel()} scores do not split into {n_seg} equal segments")
+    idx = torch.empty(n_seg * k, dtype=torch.int32, device=s.device)
+    val = torch.empty(n_seg * k, dtype=torch.float32, device=s.device)
     with torch.cuda.device(s.device):
-        _lib.check(_lib.lib().its_topk_first(idx.data_ptr(), val.data_ptr(), s.data_ptr(), s.numel(), int(k),
-                                             _lib.stream_ptr(s.device)), "its_topk_first")
+        _lib.check(_lib.lib().its_topk_first_segmented(idx.data_ptr(), val.data_ptr(), s.data_ptr(), int(n_seg),
+                                                       s.numel() // n_seg, int(k), _lib.stream_ptr(s.device)),
+                   "its_topk_first_segmented")
     return idx, val
 
 
@@ -262,21 +283,57 @@ def path_expand(x: torch.Tensor, parent: torch.Tensor, m: int, child0: int, n_ch
 
 
 def _score_population(cands_local: torch.Tensor, lo: int, n_total: int, denoise: SamplerDenoiser, ver,
-                      kwargs, t_start=None, seed=None) -> torch.Tensor:
+                      kwargs, t_start=None, seed=None, cand_labels=None) -> torch.Tensor:
     """Denoise + score this rank's block of candidates, return ALL n_total scores.  `seed`: the search's
-    shared seed, used for the step noise when the denoiser has none of its own (same on every rank)."""
+    shared seed, used for the step noise when the denoiser has none of its own (same on every rank).
+    `cand_labels`: label rows of this rank's candidates ([n_local, B]), else kwargs' `labels` for all."""
     B = cands_local.shape[1] if cands_local.numel() else 1
     if cands_local.shape[0] > 0:
-        imgs = denoise.denoise_candidates(cands_local, lo, labels=kwargs.get("labels"), t_start=t_start, seed=seed)
+        imgs = denoise.denoise_candidates(cands_local, lo, labels=kwargs.get("labels"), t_start=t_start, seed=seed,
+                                          cand_labels=cand_labels)
         local = ver.score_candidates(imgs.reshape(-1, *imgs.shape[2:]), B)
     else:
         local = torch.empty(0, dtype=torch.float32, device=cands_local.device)
     return _gather_scores(local, n_total)
 
 
+def _check_queries(n_queries: int, noise_shape: Sequence[int], labels: Optional[torch.Tensor]) -> int:
+    """K of a batched search; its `labels` must be [K] (one label per query) or [K, B] (one row per query)."""
+    K = int(n_queries)
+    if K < 1:
+        raise ValueError(f"n_queries={n_queries} must be >= 1")
+    B = int(noise_shape[0])
+    if labels is not None and tuple(labels.shape) not in ((K,), (K, B)):
+        raise ValueError(f"labels must be [{K}] or [{K}, {B}] (one label or one label row per query), got "
+                         f"{list(labels.shape)}")
+    return K
+
+
+def _check_shape(name: str, t: Optional[torch.Tensor], want: Sequence[int]) -> None:
+    if t is not None and tuple(t.shape) != tuple(want):
+        raise ValueError(f"{name} must be {list(want)}, got {list(t.shape)}")
+
+
+def _label_rows(labels: Optional[torch.Tensor], K: int, per_query: int, B: int, device) -> Optional[torch.Tensor]:
+    """Query labels ([K] or [K, B]) as one int64 row per population member, query-major: [K * per_query, B]."""
+    if labels is None:
+        return None
+    lab = labels.to(device=device, dtype=torch.int64).reshape(K, 1, -1).expand(K, per_query, B)
+    return lab.reshape(K * per_query, B)
+
+
+def _rows(rows: Optional[torch.Tensor], lo: int, hi: int) -> Optional[torch.Tensor]:
+    return None if rows is None else rows[lo:hi]
+
+
+def _query(K: int, q: int) -> str:
+    """Prefix naming the query in the errors of a batched search (a single search keeps its messages)."""
+    return f"query {q}, " if K > 1 else ""
+
+
 # ------------------------------------------------------------ RandomSearch --
 class RandomSearch:
-    """N random x_T candidates; keep the best verifier score (:18-87)."""
+    """N random x_T candidates; keep the best verifier score (:18-87).  `search_batch` runs K such searches at once."""
 
     def __init__(self, n_candidates: int = 4):
         self.n_candidates = n_candidates
@@ -301,30 +358,76 @@ class RandomSearch:
                 if score > best_score:
                     best_score, best_noise = score, noise.clone()
             return best_noise, best_score
+        best, vals, ids = self._population(noise_shape, denoise_fn, ver, 1, cand_noise=cand_noise, cand_labels=None,
+                                           seed=seed, device=device, kwargs=kwargs)
+        self.last_scores = self.last_scores[0]
+        if ids[0] < 0:
+            return None, float('-inf')
+        self.last_index = ids[0]
+        return best[0], vals[0]
+
+    def search_batch(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
+                     n_queries: int, *, labels: Optional[torch.Tensor] = None,
+                     candidate_noise: Optional[torch.Tensor] = None, seed: Optional[int] = None,
+                     device: str = 'cuda') -> Tuple[torch.Tensor, List[float]]:
+        """K = `n_queries` independent random searches of `n_candidates` (N) each, evaluated as one population of
+        K*N candidates, with one winner per query selected on the device.  Population mode only.
+
+        `labels` [K] or [K, B]: query q's labels (guided sampler; default: the denoiser's own for every query).
+        `candidate_noise` [K, N, *noise_shape]: injected candidates.  Query q's candidate i is global candidate
+        q*N + i (its x_T draw under TAG_X_T and its step noise are keyed by that id), so an unguided batch of K
+        searches draws and scores exactly the population of RandomSearch(K*N).search with the same seed.
+        Returns (best_noise [K, *noise_shape], best_scores); sets `last_scores` [K, N] (device), `last_index`
+        (within-query indices) and `last_seed`.  A query with no rankable score gets a NaN row, -inf and -1."""
+        K = _check_queries(n_queries, noise_shape, labels)
+        ver = _population_mode(denoise_fn, verifier_fn)
+        if ver is None:
+            raise ValueError("search_batch needs an its_b200 SamplerDenoiser and a kernel verifier's .score "
+                             "(population mode)")
+        N = self.n_candidates
+        _check_shape("candidate_noise", candidate_noise, (K, N, *noise_shape))
+        denoise_fn.reset_calls()
+        cand = None if candidate_noise is None else candidate_noise.reshape(K * N, *noise_shape)
+        best, vals, ids = self._population(noise_shape, denoise_fn, ver, K, cand_noise=cand,
+                                           cand_labels=_label_rows(labels, K, N, noise_shape[0], device),
+                                           seed=seed, device=device, kwargs={})
+        self.last_index = ids
+        return best, vals
+
+    def _population(self, noise_shape, denoise_fn: SamplerDenoiser, ver, K: int, *, cand_noise, cand_labels, seed,
+                    device, kwargs) -> Tuple[torch.Tensor, List[float], List[int]]:
+        """K queries of N candidates as one population sharded over the ranks; query q's candidate i is global
+        candidate q*N + i.  One segmented top-k (k = 1 per query) selects every winner.  Sets `last_seed` and
+        `last_scores` [K, N]; returns (winners [K, *noise_shape], scores, within-query indices), a NaN row, -inf
+        and -1 for a query with no rankable score."""
         dist, rank, world = _dist()
         dev = torch.device(device)
         seed = _shared_seed(seed, dev)
         self.last_seed = seed
+        N = self.n_candidates
+        n = K * N
         lo, hi = _shard(n, rank, world)
-        B = noise_shape[0]
         if cand_noise is not None:
             local = cand_noise[lo:hi].to(dev, torch.float32)
         else:
             local = philox_normal((hi - lo,) + tuple(noise_shape), seed, lo, TAG_X_T, dev) \
                 if hi > lo else torch.empty((0, *noise_shape), device=dev)
         with torch.no_grad():
-            scores = _score_population(local, lo, n, denoise_fn, ver, kwargs, seed=seed)
+            scores = _score_population(local, lo, n, denoise_fn, ver, kwargs, seed=seed,
+                                       cand_labels=_rows(cand_labels, lo, hi))
         self.nfes += n
-        self.last_scores = scores
-        idx, val = argmax_first(scores)
-        if idx < 0:
-            return None, float('-inf')
-        if cand_noise is not None:
-            best = cand_noise[idx].to(dev, torch.float32).clone()
-        else:  # every rank regenerates the winner from its key: no broadcast needed
-            best = philox_normal((1,) + tuple(noise_shape), seed, idx, TAG_X_T, dev)[0]
-        self.last_index = idx
-        return best, val
+        self.last_scores = scores.view(K, N)
+        idx, val = _topk_device(scores, 1, n_seg=K)
+        ids, vals = idx.tolist(), val.tolist()
+        best = torch.full((K, *noise_shape), float('nan'), dtype=torch.float32, device=dev)
+        for q, i in enumerate(ids):
+            if i < 0:
+                continue
+            if cand_noise is not None:
+                best[q] = cand_noise[i].to(dev, torch.float32)
+            else:  # every rank regenerates the winner from its key: no broadcast needed
+                best[q] = philox_normal((1,) + tuple(noise_shape), seed, i, TAG_X_T, dev)[0]
+        return best, vals, [i - q * N if i >= 0 else -1 for q, i in enumerate(ids)]
 
     def reset_nfes(self):
         self.nfes = 0
@@ -530,7 +633,7 @@ class SearchOverPaths:
     `start_step`.  Each round (`path_rounds`) re-noises every survivor `n_children` (M) times with q(x_s' | x_s)
     (`delta_f` forward steps), denoises all N*M children `delta_b` steps, scores each on the x0 prediction of its
     segment's last UNet evaluation (no extra evaluation) and keeps the N best (`topk_first`); the last round
-    ends at step 0 and returns the best finished sample (`argmax_first`).
+    ends at step 0 and returns the best finished sample (k = 1, `argmax_first`'s rule).
 
     Population mode only: an its_b200 `SamplerDenoiser` and a kernel verifier's `.score`.  Paths and children
     are sharded over the ranks by global id; per round one score all_gather and one all_gather of the fp32
@@ -540,7 +643,8 @@ class SearchOverPaths:
     `search(noise_shape, denoise_fn, verifier_fn, ...)` returns (best_images [B,C,H,W], best_score, history);
     keyword extensions: `seed`, `labels`, `candidate_noise`, `forward_noise` ([rounds][N*M, *noise_shape]
     injected re-noising draws).  `last_index` is the winner's initial path id, `last_seed` the search seed.
-    `nfes` counts UNet steps x candidates (the reference's classes count denoise_fn calls)."""
+    `nfes` counts UNet steps x candidates (the reference's classes count denoise_fn calls).  `search_batch` runs
+    K such searches, with their own labels, as one population."""
 
     def __init__(self, n_beams: int = 4, n_children: int = 4, start_step: int = 800, delta_f: int = 50,
                  delta_b: int = 100, verbose: bool = False):
@@ -558,7 +662,55 @@ class SearchOverPaths:
         cand_noise = kwargs.pop("candidate_noise", None)
         fwd_noise = kwargs.pop("forward_noise", None)
         seed = kwargs.pop("seed", None)
-        labels = kwargs.get("labels")
+        ver, rounds = self._schedule(denoise_fn, verifier_fn)
+        if fwd_noise is not None and len(fwd_noise) < len(rounds):
+            raise ValueError(f"forward_noise has {len(fwd_noise)} rounds, the schedule {len(rounds)}")
+        images, best, h = self._population(tuple(noise_shape), denoise_fn, ver, rounds, 1, labels=kwargs.get("labels"),
+                                           query_labels=None, cand_noise=cand_noise, fwd_noise=fwd_noise, seed=seed,
+                                           device=device)
+        history = {'rounds': h['rounds'], 'scores': h['scores'][0], 'survivors': h['survivors'][0],
+                   'lineage': h['lineage'][0], 'unet_image_steps': h['unet_image_steps']}
+        self.last_index = history['lineage']['path']
+        return images[0], best[0], history
+
+    def search_batch(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
+                     n_queries: int, *, labels: Optional[torch.Tensor] = None,
+                     candidate_noise: Optional[torch.Tensor] = None, forward_noise=None, seed: Optional[int] = None,
+                     device: str = 'cuda') -> Tuple[torch.Tensor, List[float], Dict[str, Any]]:
+        """K = `n_queries` independent searches over paths evaluated as one population: K*N paths in stage 0 and
+        K*N*M children per round, with the N survivors (and at the end the winner) of every query selected on the
+        device by one segmented top-k.  Population mode only.
+
+        `labels` [K] or [K, B]: query q's labels (guided sampler; default: the denoiser's own for every query).
+        `candidate_noise` [K, N, *noise_shape] and `forward_noise` [rounds][K, N*M, *noise_shape]: injected draws.
+        Query q's path i is global path q*N + i and its child c global child q*N*M + c; x_T, step noise and
+        re-noising draws are keyed by those ids, so K = 1 is `search` and a query's result does not depend on
+        the other queries, the rank count or `max_images`.
+        Returns (best_images [K, *noise_shape], best_scores, history): history 'rounds' as in `search`; 'scores',
+        'survivors' and 'lineage' are lists over the queries, with within-query ids; 'unet_image_steps' is the
+        whole batch's.  `last_index` is the list of the winners' initial path ids.  A query whose children cannot
+        be ranked raises ValueError naming the query and the round."""
+        K = _check_queries(n_queries, noise_shape, labels)
+        ver, rounds = self._schedule(denoise_fn, verifier_fn)
+        shape = tuple(noise_shape)
+        N, NM = int(self.n_beams), int(self.n_beams) * int(self.n_children)
+        _check_shape("candidate_noise", candidate_noise, (K, N) + shape)
+        fwd = None
+        if forward_noise is not None:
+            if len(forward_noise) < len(rounds):
+                raise ValueError(f"forward_noise has {len(forward_noise)} rounds, the schedule {len(rounds)}")
+            for r in range(len(rounds)):
+                _check_shape(f"forward_noise[{r}]", forward_noise[r], (K, NM) + shape)
+            fwd = [forward_noise[r].reshape((K * NM,) + shape) for r in range(len(rounds))]
+        images, best, history = self._population(
+            shape, denoise_fn, ver, rounds, K, labels=None, query_labels=labels,
+            cand_noise=None if candidate_noise is None else candidate_noise.reshape((K * N,) + shape),
+            fwd_noise=fwd, seed=seed, device=device)
+        self.last_index = [lin['path'] for lin in history['lineage']]
+        return images, best, history
+
+    def _schedule(self, denoise_fn, verifier_fn) -> Tuple[Any, List[Tuple[int, int, int]]]:
+        """(kernel verifier, round schedule) after checking the mode and the parameters against sampler.T."""
         ver = _population_mode(denoise_fn, verifier_fn)
         if ver is None:
             raise ValueError("SearchOverPaths needs an its_b200 SamplerDenoiser and a kernel verifier's .score "
@@ -566,24 +718,33 @@ class SearchOverPaths:
         N, M = int(self.n_beams), int(self.n_children)
         if N < 1 or M < 1:
             raise ValueError(f"n_beams={N} and n_children={M} must be >= 1")
+        return ver, path_rounds(denoise_fn.sampler.T, self.start_step, self.delta_f, self.delta_b)
+
+    def _population(self, shape: Tuple[int, ...], denoise_fn: SamplerDenoiser, ver, rounds, K: int, *, labels,
+                    query_labels, cand_noise, fwd_noise, seed, device):
+        """K queries as one population sharded over the ranks (query q's path i is global path q*N + i, its child c
+        global child q*N*M + c).  `labels`: shared labels of every member; `query_labels` ([K] or [K, B]): one
+        label row per query.  Returns (best images [K, *shape], best scores, history with per-query 'scores',
+        'survivors' and 'lineage' in within-query ids)."""
+        N, M = int(self.n_beams), int(self.n_children)
+        NM = N * M
         smp = denoise_fn.sampler
         T = smp.T
-        rounds = path_rounds(T, self.start_step, self.delta_f, self.delta_b)
-        if fwd_noise is not None and len(fwd_noise) < len(rounds):
-            raise ValueError(f"forward_noise has {len(fwd_noise)} rounds, the schedule {len(rounds)}")
         dist, rank, world = _dist()
         dev = torch.device(device)
         seed = _shared_seed(seed, dev)
         self.last_seed = seed
-        shape = tuple(noise_shape)
         B = shape[0]
         abar = torch.cumprod(1. - smp.betas.detach().double().cpu(), dim=0)
         denoise_fn.reset_calls()
-        history: Dict[str, Any] = {'rounds': [], 'scores': [], 'survivors': []}
+        path_labels, child_labels = _label_rows(query_labels, K, N, B, dev), _label_rows(query_labels, K, NM, B, dev)
+        history: Dict[str, Any] = {'rounds': [], 'scores': [[] for _ in range(K)],
+                                   'survivors': [[] for _ in range(K)]}
         steps = 0                                     # UNet steps x candidates
         with torch.no_grad():
-            # stage 0: N paths from x_T down to the states at step start_step
-            lo, hi = _shard(N, rank, world)
+            # stage 0: K*N paths from x_T down to the states at step start_step
+            n_p = K * N
+            lo, hi = _shard(n_p, rank, world)
             if cand_noise is not None:
                 local = cand_noise[lo:hi].to(dev, torch.float32)
             elif hi > lo:
@@ -592,11 +753,12 @@ class SearchOverPaths:
                 local = torch.empty((0,) + shape, device=dev)
             s0 = rounds[0][0]
             if s0 < T - 1 and hi > lo:
-                local = denoise_fn.denoise_candidates(local, lo, labels=labels, seed=seed, t_stop=s0 + 1)
-            steps += N * (T - 1 - s0)
-            parents = _gather_states(local.contiguous(), N)
-            parent_idx = torch.arange(N, dtype=torch.int32, device=dev)
-            n_c = N * M
+                local = denoise_fn.denoise_candidates(local, lo, labels=labels, seed=seed, t_stop=s0 + 1,
+                                                      cand_labels=_rows(path_labels, lo, hi))
+            steps += n_p * (T - 1 - s0)
+            parents = _gather_states(local.contiguous(), n_p)
+            parent_idx = torch.arange(n_p, dtype=torch.int32, device=dev)
+            n_c = K * NM
             lo, hi = _shard(n_c, rank, world)
             for r, (s, sp, e) in enumerate(rounds):
                 ratio = float(abar[sp] / abar[s])
@@ -607,7 +769,8 @@ class SearchOverPaths:
                                        z=None if z is None else z.reshape(hi - lo, -1), seed=seed,
                                        cand_id0=(r + 1) * ROUND_STRIDE, tag=TAG_FORWARD).view((hi - lo,) + shape)
                     states, x0 = denoise_fn.denoise_segment(kids, lo, t_start=sp, t_stop=e, labels=labels, seed=seed,
-                                                            cand_offset=(r + 1) * ROUND_STRIDE, x0=True)
+                                                            cand_offset=(r + 1) * ROUND_STRIDE, x0=True,
+                                                            cand_labels=_rows(child_labels, lo, hi))
                     judged = x0 if e > 0 else states   # the last round scores the finished, clipped samples
                     local_scores = ver.score_candidates(judged.reshape(-1, *shape[1:]), B)
                 else:
@@ -616,33 +779,36 @@ class SearchOverPaths:
                 steps += n_c * (sp - e + 1)
                 scores = _gather_scores(local_scores, n_c)
                 history['rounds'].append((s, sp, e))
-                history['scores'].append([float(v) for v in scores.tolist()])
+                for q, row in enumerate(scores.view(K, NM).tolist()):
+                    history['scores'][q].append(row)
                 parents = _gather_states(states.contiguous(), n_c)
-                if e > 0:
-                    parent_idx, _ = _topk_device(scores, N)
-                    ids = parent_idx.tolist()
-                    if min(ids) < 0:
-                        raise ValueError(f"round {r}: only {sum(i >= 0 for i in ids)} of {n_c} children have a "
-                                         f"score that can be ranked; {N} survivors are needed")
-                    history['survivors'].append(ids)
-                else:
-                    idx, best = argmax_first(scores)
-                    if idx < 0:
-                        raise ValueError(f"last round: none of the {n_c} finished samples has a score that can be "
-                                         "ranked")
-                    history['survivors'].append([idx])
-        # lineage of the winner: child id in every round, back to its initial path
-        child = idx
-        lineage = [child]
-        for ids in reversed(history['survivors'][:-1]):
-            child = ids[child // M]
-            lineage.append(child)
-        lineage.reverse()
-        history['lineage'] = {'path': lineage[0] // M, 'children': lineage}
+                # survivors (k = N per query) or the winner (k = 1): flat child ids, passed on as parents as they are
+                parent_idx, best = _topk_device(scores, N if e > 0 else 1, n_seg=K)
+                ids = parent_idx.tolist()
+                k = len(ids) // K
+                for q in range(K):
+                    own = [i - q * NM if i >= 0 else -1 for i in ids[q * k:(q + 1) * k]]
+                    if min(own) >= 0:
+                        history['survivors'][q].append(own)
+                    elif e > 0:
+                        raise ValueError(f"{_query(K, q)}round {r}: only {sum(i >= 0 for i in own)} of {NM} children "
+                                         f"have a score that can be ranked; {N} survivors are needed")
+                    else:
+                        raise ValueError(f"{_query(K, q)}last round: none of the {NM} finished samples has a score "
+                                         "that can be ranked")
+        # lineage of each winner: child id in every round, back to its initial path
+        history['lineage'] = []
+        for surv in history['survivors']:
+            child = surv[-1][0]
+            lineage = [child]
+            for ids in reversed(surv[:-1]):
+                child = ids[child // M]
+                lineage.append(child)
+            lineage.reverse()
+            history['lineage'].append({'path': lineage[0] // M, 'children': lineage})
         history['unet_image_steps'] = steps * B * (2 if getattr(smp, "guided", False) else 1)
         self.nfes += steps
-        self.last_index = lineage[0] // M
-        return parents[idx].clone(), best, history
+        return parents[parent_idx.long()].clone(), best.tolist(), history
 
     def reset_nfes(self):
         self.nfes = 0

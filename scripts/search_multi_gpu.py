@@ -1,4 +1,4 @@
-"""Multi-GPU check of the three searches (BASELINE.json configs[3]): run under torchrun, one rank per GPU.
+"""Multi-GPU check of the searches (BASELINE.json configs[3]), single and batched: run under torchrun, one rank per GPU.
 Every rank must end with the same selection, and that selection must be bit-identical to the one the
 same rank computes alone over the whole population (candidate ids, Philox streams and summation orders
 do not depend on the number of ranks).  The only collective per round is the score all_gather (search over
@@ -56,6 +56,13 @@ def run_all():
     sop = S.SearchOverPaths(n_beams=3, n_children=3, start_step=3 * T // 4, delta_f=T // 8, delta_b=T // 4)
     si, ss, sh = sop.search(shape, den, ver.score, device=str(dev), seed=24)   # 9 children: ragged over 2 ranks
     out["search_over_paths"] = (si.clone(), ss, torch.tensor(sh["scores"]))
+    # batched: 3 queries x 5 candidates and 3 queries x 3 x 2 children, ragged over 2/4/8 ranks
+    rb = S.RandomSearch(n_candidates=5)
+    bn, bs = rb.search_batch(shape, den, ver.score, 3, seed=25, device=str(dev))
+    out["random_batch"] = (bn.clone(), bs, rb.last_scores.clone())
+    sb = S.SearchOverPaths(n_beams=3, n_children=2, start_step=3 * T // 4, delta_f=T // 8, delta_b=T // 4)
+    si, ss, sh = sb.search_batch(shape, den, ver.score, 3, seed=26, device=str(dev))
+    out["search_over_paths_batch"] = (si.clone(), ss, torch.tensor(sh["scores"]))
     return out
 
 
