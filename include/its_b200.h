@@ -387,6 +387,32 @@ int its_topk_first_segmented(int32_t* idx_out, float* val_out, const float* scor
                              int32_t n_seg, int32_t seg_len, int32_t k, void* stream);
 
 /* ------------------------------------------------------------------------
+ * Denoising verifier: the diffusion model scores a sample by how well it
+ * predicts the noise added to it at S levels t_s (the eps-prediction loss of
+ * Ho et al. 2020, a Monte-Carlo estimate of the denoising ELBO), and, with the
+ * guided net, by the gap between its unconditional and conditional errors (the
+ * diffusion model as a zero-shot classifier, Li et al. 2023; Clark & Jaini 2023).
+ * Not in the reference; the specification is tests/denoising_verifier_oracle.py.
+ *   its_level_inputs: out[i*S + s] = coef[s].a * x[i] + coef[s].b * eps_tab[s]
+ *     (image-major, level-minor; torch `a * x + b * eps`, fp32, separately
+ *     rounded mul / mul / add).  x [n_img][n_per], eps_tab [S][n_per], coef a
+ *     device [S][2] fp32 table {sqrt(abar_t), sqrt(1 - abar_t)}; out is usually
+ *     the UNet plan's x_in.
+ *   its_denoise_scores: one fp32 score per candidate over the UNet outputs of
+ *     rows (c*per_cand + b)*S + s:  D = sum (eps[row] - eps_tab[s])^2, each
+ *     difference one fp32 subtraction, squares and sums in double in a fixed
+ *     order (one CTA per candidate); count = per_cand * S * n_per.
+ *     eps_u == NULL: -D_c / count (likelihood); else (D_u - D_c) / count with
+ *     eps_u the null-label outputs of the same rows (class).  NaN propagates.
+ * Both require n_img / n_cand, per_cand, S >= 1 and n_per a positive multiple
+ * of 4; no allocation, no synchronisation, no atomics.                       */
+int its_level_inputs(float* out, const float* x, const float* eps_tab, const float* coef,
+                     int32_t n_img, int32_t n_levels, int64_t n_per, void* stream);
+int its_denoise_scores(float* scores, const float* eps_c, const float* eps_u,
+                       const float* eps_tab, int32_t n_cand, int32_t per_cand,
+                       int32_t n_levels, int64_t n_per, void* stream);
+
+/* ------------------------------------------------------------------------
  * fp32-grade path (precision = "fp32").  The reference computes everything in
  * fp32 (Diffusion/Diffusion.py:74-99 over Model.py / ModelCondition.py) and
  * north_star states 1e-4 on the samples for that mode: plain CUDA-core kernels

@@ -1,5 +1,6 @@
 // Verifier statistics, per-candidate scores and first-index argmax
-// and (segmented) top-k (search/verifier.py:45-66, 207-248, 262-287; search/search_algorithm.py:79-81).
+// and (segmented) top-k (search/verifier.py:45-66, 207-248, 262-287; search/search_algorithm.py:79-81); the two
+// ends of the denoising verifier around its UNet pass (level inputs, per-candidate denoising error).
 // All reductions are warp-shuffle + one shared-memory hop.
 #include "its_common.cuh"
 
@@ -213,7 +214,108 @@ __global__ void __launch_bounds__(1024) topk_first_kernel(int* __restrict__ idx_
   }
 }
 
+// Inputs of the denoising verifier: out[i*S + s] = a_s * x[i] + b_s * eps_tab[s] (image-major, level-minor), one
+// float4 per thread, separately rounded mul / mul / add (torch's `a * x + b * eps` in fp32).
+__global__ void __launch_bounds__(256) level_inputs_kernel(float* __restrict__ out, const float* __restrict__ x,
+                                                           const float* __restrict__ eps_tab,
+                                                           const float* __restrict__ coef, int n_levels,
+                                                           long long quads_per, long long total) {
+  pdl_prologue();
+  for (long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x; q < total;
+       q += (long long)gridDim.x * blockDim.x) {
+    const long long row = q / quads_per;
+    const long long quad = q - row * quads_per;
+    const long long img = row / n_levels;
+    const int s = (int)(row - img * n_levels);
+    const float a = __ldg(coef + 2 * s), b = __ldg(coef + 2 * s + 1);
+    const float4 xv = __ldg(reinterpret_cast<const float4*>(x) + img * quads_per + quad);
+    const float4 ev = __ldg(reinterpret_cast<const float4*>(eps_tab) + s * quads_per + quad);
+    float4 o;
+    o.x = __fadd_rn(__fmul_rn(a, xv.x), __fmul_rn(b, ev.x));
+    o.y = __fadd_rn(__fmul_rn(a, xv.y), __fmul_rn(b, ev.y));
+    o.z = __fadd_rn(__fmul_rn(a, xv.z), __fmul_rn(b, ev.z));
+    o.w = __fadd_rn(__fmul_rn(a, xv.w), __fmul_rn(b, ev.w));
+    reinterpret_cast<float4*>(out)[q] = o;
+  }
+}
+
+__device__ __forceinline__ double warp_sum_d(double v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  return v;
+}
+
+__device__ __forceinline__ double sq_err4(const float4 p, const float4 e) {
+  const double d0 = __fsub_rn(p.x, e.x), d1 = __fsub_rn(p.y, e.y), d2 = __fsub_rn(p.z, e.z), d3 = __fsub_rn(p.w, e.w);
+  return ((d0 * d0 + d1 * d1) + d2 * d2) + d3 * d3;
+}
+
+constexpr int kScoreThreads = 256;
+
+// One CTA of kScoreThreads per candidate: D = sum over its rows (c*per_cand + b)*S + s of (eps_hat - eps_tab[s])^2,
+// differences in fp32, squares and sums in double.  Thread j takes quads j, j + 256, ... of the candidate; the
+// per-thread sums are combined by a fixed shuffle tree, so the order depends on nothing but the candidate's size.
+// eps_u == NULL: score = -D_c / count; else (D_u - D_c) / count.  A NaN anywhere propagates to the score.
+__global__ void __launch_bounds__(kScoreThreads) denoise_scores_kernel(
+    float* __restrict__ scores, const float* __restrict__ eps_c, const float* __restrict__ eps_u,
+    const float* __restrict__ eps_tab, int n_levels, long long rows_per_cand, long long quads_per) {
+  pdl_prologue();
+  __shared__ double s_c[kScoreThreads / 32], s_u[kScoreThreads / 32];
+  const long long row0 = (long long)blockIdx.x * rows_per_cand;
+  const long long n_q = rows_per_cand * quads_per;
+  const float4* pc = reinterpret_cast<const float4*>(eps_c) + row0 * quads_per;
+  const float4* pu = eps_u ? reinterpret_cast<const float4*>(eps_u) + row0 * quads_per : nullptr;
+  const float4* pe = reinterpret_cast<const float4*>(eps_tab);
+  double acc_c = 0.0, acc_u = 0.0;
+  for (long long q = threadIdx.x; q < n_q; q += kScoreThreads) {
+    const long long r = q / quads_per;
+    const long long quad = q - r * quads_per;
+    const int s = (int)((row0 + r) % n_levels);
+    const float4 e = __ldg(pe + s * quads_per + quad);
+    acc_c += sq_err4(__ldg(pc + q), e);
+    if (pu) acc_u += sq_err4(__ldg(pu + q), e);
+  }
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  acc_c = warp_sum_d(acc_c);
+  acc_u = warp_sum_d(acc_u);
+  if (lane == 0) { s_c[warp] = acc_c; s_u[warp] = acc_u; }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double dc = 0.0, du = 0.0;
+    for (int w = 0; w < kScoreThreads / 32; ++w) { dc += s_c[w]; du += s_u[w]; }
+    const double count = (double)rows_per_cand * (double)(quads_per * 4);
+    scores[blockIdx.x] = (float)((pu ? du - dc : -dc) / count);
+  }
+}
+
 }  // namespace its
+
+extern "C" int its_level_inputs(float* out, const float* x, const float* eps_tab, const float* coef, int32_t n_img,
+                                int32_t n_levels, int64_t n_per, void* stream) {
+  ITS_REQUIRE(out && x && eps_tab && coef, "its_level_inputs: null pointer");
+  ITS_REQUIRE(n_img >= 1 && n_levels >= 1 && n_per >= 1 && n_per % 4 == 0,
+              "its_level_inputs: n_img=%d n_levels=%d must be >= 1, n_per=%lld a positive multiple of 4", n_img,
+              n_levels, (long long)n_per);
+  const long long quads = n_per / 4, total = (long long)n_img * n_levels * quads;
+  long long grid = (total + 255) / 256;
+  if (grid > 148LL * 8) grid = 148LL * 8;  // 8 resident 256-thread CTAs per SM, grid-stride beyond
+  ITS_LAUNCH(its::level_inputs_kernel, dim3((unsigned)grid), dim3(256), 0, its::as_stream(stream), out, x, eps_tab,
+             coef, (int)n_levels, quads, total);
+  ITS_CHECK_LAUNCH();
+  return ITS_OK;
+}
+
+extern "C" int its_denoise_scores(float* scores, const float* eps_c, const float* eps_u, const float* eps_tab,
+                                  int32_t n_cand, int32_t per_cand, int32_t n_levels, int64_t n_per, void* stream) {
+  ITS_REQUIRE(scores && eps_c && eps_tab, "its_denoise_scores: null pointer");
+  ITS_REQUIRE(n_cand >= 1 && per_cand >= 1 && n_levels >= 1 && n_per >= 1 && n_per % 4 == 0,
+              "its_denoise_scores: n_cand=%d per_cand=%d n_levels=%d must be >= 1, n_per=%lld a positive multiple "
+              "of 4", n_cand, per_cand, n_levels, (long long)n_per);
+  ITS_LAUNCH(its::denoise_scores_kernel, dim3((unsigned)n_cand), dim3(its::kScoreThreads), 0, its::as_stream(stream),
+             scores, eps_c, eps_u, eps_tab, (int)n_levels, (long long)per_cand * n_levels, (long long)(n_per / 4));
+  ITS_CHECK_LAUNCH();
+  return ITS_OK;
+}
 
 extern "C" int its_image_stats(float* stats, float* feats, const float* images, int32_t n_img,
                                int32_t C, int32_t H, int32_t W, void* stream) {

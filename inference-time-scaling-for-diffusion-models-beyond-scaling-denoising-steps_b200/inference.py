@@ -265,9 +265,22 @@ def sample_with_metrics_tracking(sampler, x_T: torch.Tensor, fid_calculator=None
 
 
 # -------------------------------------------------------------- search -------
-def make_verifier(name: str):
+DENOISING_VERIFIERS = {"denoising": "likelihood", "diffusion_classifier": "class"}
+
+
+def make_verifier(name: str, sampler=None, *, n_levels: int = 8, seed: int = 0, max_images: int = 256):
+    """Verifier by config name.  `denoising` / `diffusion_classifier` are the sampler's own model scoring its
+    samples (DenoisingVerifier, kinds likelihood / class) and need `sampler`; the class form needs the guided net."""
     from .search import verifier as V
     table = {"oracle": V.OracleVerifier, "self_supervised": V.SelfSupervisedVerifier, "aesthetic": V.AestheticPredictor}
+    if name in DENOISING_VERIFIERS:
+        if sampler is None:
+            raise ValueError(f"verifier {name!r} scores with the diffusion model: pass the sampler")
+        if name == "diffusion_classifier" and not getattr(sampler._unet(), "is_conditional", False):
+            raise ValueError("verifier 'diffusion_classifier' needs the conditional net (num_labels in the config): "
+                             "it compares the conditional and unconditional denoising errors")
+        return V.DenoisingVerifier(sampler, DENOISING_VERIFIERS[name], n_levels=n_levels, seed=seed,
+                                   max_images=max_images)
     if name not in table:
         raise ValueError(f"verifier {name!r}: choose one of {sorted(table)} (the CLIP-backed verifiers need "
                          "third-party weights that are not bundled)")
@@ -277,7 +290,8 @@ def make_verifier(name: str):
 def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Optional[int] = None):
     """`search:` block of the config -> (best_noise, best_score, images of the best candidate).
     Keys: algorithm (random | zero_order | path | search_over_paths), verifier (oracle | self_supervised |
-    aesthetic), n_candidates / n_neighbors / n_iterations / lambda_radius / n_paths / injection_step / noise_scale
+    aesthetic | denoising | diffusion_classifier; the last two score with the sampler's own model at score_levels
+    (8) noise levels drawn from score_seed (0), in chunks of max_images UNet images), n_candidates / n_neighbors / n_iterations / lambda_radius / n_paths / injection_step / noise_scale
     (defaults: the reference constructors', search_algorithm.py:24,98-100,246-248), batch_size,
     img_size.  search_over_paths takes n_beams (4), n_children (4), start_step (800), delta_f (50) and
     delta_b (100), and returns the winner's initial x_T with the images the search itself finished (the winner's
@@ -291,7 +305,8 @@ def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Op
     algo = sc.get("algorithm", "random")
     B, H = int(config.get("batch_size", 1)), int(config["img_size"])
     shape = (B, 3, H, H)
-    ver = make_verifier(sc.get("verifier", "oracle"))
+    ver = make_verifier(sc.get("verifier", "oracle"), sampler, n_levels=int(sc.get("score_levels", 8)),
+                        seed=int(sc.get("score_seed", 0)), max_images=int(sc.get("max_images", 256)))
     K = int(sc.get("n_queries", 1))
     if K > 1:
         return _run_batch(sampler, sc, algo, K, shape, ver, device, labels=labels, seed=seed)

@@ -84,8 +84,16 @@ class SamplerDenoiser:
             self._fallback_seed = int(torch.randint(0, 2 ** 62, (1,)).item())
         return self._fallback_seed
 
-    def _labels_for(self, n_cand: int, kw_labels) -> Optional[torch.Tensor]:
-        lab = kw_labels if kw_labels is not None else self.labels
+    def image_labels(self, n_cand: int, labels=None, cand_labels: Optional[torch.Tensor] = None
+                     ) -> Optional[torch.Tensor]:
+        """Flat per-image labels [n_cand * B] the guided sampler is fed for `n_cand` candidates: `cand_labels`
+        [n_cand, B] (one row per candidate) when given, else `labels` (or the denoiser's own) [B] for every
+        candidate; None for an unguided sampler.  The verifiers that read labels score with the same vector."""
+        if not getattr(self.sampler, "guided", False):
+            return None
+        if cand_labels is not None:
+            return cand_labels.reshape(-1)
+        lab = labels if labels is not None else self.labels
         if lab is None:
             return None
         return lab.reshape(-1).repeat(n_cand)
@@ -118,7 +126,6 @@ class SamplerDenoiser:
         sampler's labels are `cand_labels` [n, B] (int64, one row per candidate) when given, else `labels` (or the
         denoiser's own) [B] for every candidate."""
         n, B = states.shape[:2]
-        guided = getattr(self.sampler, "guided", False)
         if cand_labels is not None and tuple(cand_labels.shape) != (n, B):
             raise ValueError(f"cand_labels must be [{n}, {B}] (one label row per candidate), got "
                              f"{tuple(cand_labels.shape)}")
@@ -133,12 +140,7 @@ class SamplerDenoiser:
                                       cand_id0=cand_offset + (first_cand + i0) * B, x0=x0)
             if self.step_noise is not None:
                 kw["noise"] = self.step_noise.repeat(1, i1 - i0, 1, 1, 1)
-            if not guided:
-                lab = None
-            elif cand_labels is not None:
-                lab = cand_labels[i0:i1].reshape(-1)
-            else:
-                lab = self._labels_for(i1 - i0, labels)
+            lab = self.image_labels(i1 - i0, labels, None if cand_labels is None else cand_labels[i0:i1])
             y, p = self.sampler.segment(x, lab, **kw)
             out[i0:i1] = y.view(i1 - i0, B, *states.shape[2:])
             if x0:
@@ -282,6 +284,15 @@ def path_expand(x: torch.Tensor, parent: torch.Tensor, m: int, child0: int, n_ch
     return out
 
 
+def _score_candidates(ver, images: torch.Tensor, B: int, denoise: SamplerDenoiser, labels=None,
+                      cand_labels: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """ver.score_candidates over candidates of B images; a verifier with `uses_labels` also gets the flat labels
+    the denoiser fed the sampler for them."""
+    if not getattr(ver, "uses_labels", False):
+        return ver.score_candidates(images, B)
+    return ver.score_candidates(images, B, labels=denoise.image_labels(images.shape[0] // B, labels, cand_labels))
+
+
 def _score_population(cands_local: torch.Tensor, lo: int, n_total: int, denoise: SamplerDenoiser, ver,
                       kwargs, t_start=None, seed=None, cand_labels=None) -> torch.Tensor:
     """Denoise + score this rank's block of candidates, return ALL n_total scores.  `seed`: the search's
@@ -291,7 +302,8 @@ def _score_population(cands_local: torch.Tensor, lo: int, n_total: int, denoise:
     if cands_local.shape[0] > 0:
         imgs = denoise.denoise_candidates(cands_local, lo, labels=kwargs.get("labels"), t_start=t_start, seed=seed,
                                           cand_labels=cand_labels)
-        local = ver.score_candidates(imgs.reshape(-1, *imgs.shape[2:]), B)
+        local = _score_candidates(ver, imgs.reshape(-1, *imgs.shape[2:]), B, denoise, kwargs.get("labels"),
+                                  cand_labels)
     else:
         local = torch.empty(0, dtype=torch.float32, device=cands_local.device)
     return _gather_scores(local, n_total)
@@ -772,7 +784,8 @@ class SearchOverPaths:
                                                             cand_offset=(r + 1) * ROUND_STRIDE, x0=True,
                                                             cand_labels=_rows(child_labels, lo, hi))
                     judged = x0 if e > 0 else states   # the last round scores the finished, clipped samples
-                    local_scores = ver.score_candidates(judged.reshape(-1, *shape[1:]), B)
+                    local_scores = _score_candidates(ver, judged.reshape(-1, *shape[1:]), B, denoise_fn, labels,
+                                                     _rows(child_labels, lo, hi))
                 else:
                     states = torch.empty((0,) + shape, device=dev)
                     local_scores = torch.empty(0, dtype=torch.float32, device=dev)

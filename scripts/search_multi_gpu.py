@@ -38,6 +38,7 @@ smp.print_steps = False
 shape = (2, 3, 32, 32)
 den = S.make_denoise_fn(smp, max_images=64, seed=11)
 ver = V.OracleVerifier()
+dver = V.DenoisingVerifier(smp, "likelihood", n_levels=4, seed=3, max_images=64)
 x0 = S.philox_normal((1,) + shape, 5, 0, S.TAG_X_T, dev)[0]
 
 
@@ -63,6 +64,10 @@ def run_all():
     sb = S.SearchOverPaths(n_beams=3, n_children=2, start_step=3 * T // 4, delta_f=T // 8, delta_b=T // 4)
     si, ss, sh = sb.search_batch(shape, den, ver.score, 3, seed=26, device=str(dev))
     out["search_over_paths_batch"] = (si.clone(), ss, torch.tensor(sh["scores"]))
+    # the denoising verifier: the model's own scores, with noise common to every candidate on every rank
+    rd = S.RandomSearch(n_candidates=13)
+    bn, bs = rd.search(shape, den, dver.score, device=str(dev), verbose=False, seed=27)
+    out["random_denoising_verifier"] = (bn.clone(), bs, rd.last_scores.clone())
     return out
 
 
