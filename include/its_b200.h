@@ -385,6 +385,29 @@ int its_topk_first(int32_t* idx_out, float* val_out, const float* scores,
  * Requires n_seg, seg_len, k >= 1 and n_seg * seg_len <= INT32_MAX; no allocation, no synchronisation.   */
 int its_topk_first_segmented(int32_t* idx_out, float* val_out, const float* scores,
                              int32_t n_seg, int32_t seg_len, int32_t k, void* stream);
+/* Systematic resampling of Feynman-Kac particles (Singhal et al. 2025, "A General Framework for Inference-time
+ * Scaling and Steering of Diffusion Models"; not in the reference), one CTA per segment (query).  Segment s is
+ * reward[s*seg_len, (s+1)*seg_len); for its particle i:
+ *   l_i = lam * (reward_i - carried_i)   fp32, separately rounded; carried_in == NULL means carried_i = 0
+ *   w_i = exp((double)l_i - m)           in double, m the largest finite l_i; w_i = 0 when reward_i or l_i is
+ *                                        not finite (NaN, +-inf)
+ *   C_i = w_0 + ... + w_i                in double
+ *   u   = ((c0 >> 5) * 2^26 + (c1 >> 6)) * 2^-53 in [0, 1), with (c0, c1, c2, c3) = Philox4x32-10 of the counter
+ *         {s, (uint32)round, tag, (uint32)(round >> 32)} under the key {(uint32)seed, (uint32)(seed >> 32)}
+ *         (the generator of its_philox_normal): one uniform per (seed, segment, round)
+ *   child j < seg_len takes the smallest i with C_i > (u + j) / seg_len * C_last, evaluated without a division
+ *   as seg_len * C_i > (u + j) * C_last in double (a position that rounding puts at or past C_last goes to the
+ *   last i with w_i > 0; the exact rule never puts one there).
+ * Outputs: ancestor_out[s*seg_len + j] = s*seg_len + i (flat, as its_topk_first_segmented's indices),
+ * carried_out[s*seg_len + j] = reward_i of that ancestor (the next call's carried_in), ess_out[s] =
+ * (sum w)^2 / sum w^2.  A segment with no finite weight gets ancestors -1, carried NaN and ESS 0.  Sums have a
+ * fixed order and no atomics: the outputs are a deterministic function of the inputs, so every rank draws the
+ * same ancestors from the same gathered rewards.  Requires n_seg, seg_len >= 1, n_seg * seg_len <= INT32_MAX,
+ * lam finite and >= 0; no allocation, no synchronisation.                                                      */
+int its_resample_systematic(int32_t* ancestor_out, float* carried_out, float* ess_out,
+                            const float* reward, const float* carried_in, float lam,
+                            int32_t n_seg, int32_t seg_len, uint64_t seed, int64_t round,
+                            int32_t tag, void* stream);
 
 /* ------------------------------------------------------------------------
  * Denoising verifier: the diffusion model scores a sample by how well it

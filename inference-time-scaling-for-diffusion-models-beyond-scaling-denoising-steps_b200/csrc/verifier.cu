@@ -1,6 +1,7 @@
 // Verifier statistics, per-candidate scores and first-index argmax
 // and (segmented) top-k (search/verifier.py:45-66, 207-248, 262-287; search/search_algorithm.py:79-81); the two
-// ends of the denoising verifier around its UNet pass (level inputs, per-candidate denoising error).
+// ends of the denoising verifier around its UNet pass (level inputs, per-candidate denoising error); systematic
+// resampling of Feynman-Kac particles.
 // All reductions are warp-shuffle + one shared-memory hop.
 #include "its_common.cuh"
 
@@ -214,6 +215,125 @@ __global__ void __launch_bounds__(1024) topk_first_kernel(int* __restrict__ idx_
   }
 }
 
+// Systematic resampling of a Feynman-Kac particle population, one CTA per segment (query).  Particle i of the
+// segment has the log-potential l_i = lam * (reward_i - carried_i) (fp32, separately rounded) and the weight
+// w_i = exp((double)l_i - m), m the largest finite l_i; a non-finite reward or l_i weighs 0.  Thread t owns the
+// contiguous particles [t*per, (t+1)*per): its partial sums run in particle order, thread 0 scans the partials in
+// thread order, so C_i = P_t + (w_a + ... + w_i) and every sum has one fixed order (no atomics).  Child j takes the
+// smallest i with seg_len * C_i > (u + j) * C_last; a thread finds the children of its own particles by a binary
+// search over j (the positions are monotone in j) and walks its particles once.  A position that rounding puts at
+// or past C_last (the exact rule never does) goes to the last particle of non-zero weight.
+constexpr int kResampleThreads = 256;
+
+__device__ __forceinline__ double fk_weight(const float* __restrict__ reward, const float* __restrict__ carried,
+                                            int i, float lam, double m) {
+  const float r = reward[i];
+  if (!isfinite(r)) return 0.0;
+  const float l = __fmul_rn(lam, __fsub_rn(r, carried ? carried[i] : 0.f));
+  return isfinite(l) ? exp((double)l - m) : 0.0;
+}
+
+__global__ void __launch_bounds__(kResampleThreads) resample_systematic_kernel(
+    int* __restrict__ ancestor_out, float* __restrict__ carried_out, float* __restrict__ ess_out,
+    const float* __restrict__ reward, const float* __restrict__ carried, float lam, int seg_len, uint64_t seed,
+    long long round, uint32_t tag) {
+  pdl_prologue();
+  __shared__ double s_part[kResampleThreads], s_sq[kResampleThreads];
+  __shared__ float s_max[32];
+  __shared__ int s_last[32];
+  __shared__ double s_total;
+  const int tid = threadIdx.x, nt = blockDim.x, lane = tid & 31, warp = tid >> 5, nw = nt >> 5;
+  const int base = blockIdx.x * seg_len;    // n_seg * seg_len fits int32 (checked on the host)
+  reward += base;
+  if (carried) carried += base;
+  ancestor_out += base;
+  carried_out += base;
+  const int per = (seg_len + nt - 1) / nt;
+  const int a = min(seg_len, tid * per), b = min(seg_len, a + per);
+
+  // m: the largest finite log-potential (a max is exact in any order)
+  float mx = -INFINITY;
+  for (int i = a; i < b; ++i) {
+    const float r = reward[i];
+    if (!isfinite(r)) continue;
+    const float l = __fmul_rn(lam, __fsub_rn(r, carried ? carried[i] : 0.f));
+    if (isfinite(l)) mx = fmaxf(mx, l);
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  if (lane == 0) s_max[warp] = mx;
+  __syncthreads();
+  mx = -INFINITY;
+  for (int w = 0; w < nw; ++w) mx = fmaxf(mx, s_max[w]);
+  if (mx == -INFINITY) {                    // no particle has a finite weight
+    for (int j = tid; j < seg_len; j += nt) { ancestor_out[j] = -1; carried_out[j] = __int_as_float(0x7fc00000); }
+    if (tid == 0) ess_out[blockIdx.x] = 0.f;
+    return;
+  }
+  const double m = (double)mx;
+
+  // per-thread sums in particle order, the last particle of non-zero weight
+  double S = 0.0, sq = 0.0;
+  int last = -1;
+  for (int i = a; i < b; ++i) {
+    const double w = fk_weight(reward, carried, i, lam, m);
+    S += w;
+    sq += w * w;
+    if (w > 0.0) last = i;
+  }
+  s_part[tid] = S;
+  s_sq[tid] = sq;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) last = max(last, __shfl_xor_sync(0xffffffffu, last, o));
+  if (lane == 0) s_last[warp] = last;
+  __syncthreads();
+  if (tid == 0) {                           // exclusive scan of the partials in thread order
+    double acc = 0.0, acc_sq = 0.0;
+    for (int t = 0; t < nt; ++t) {
+      const double v = s_part[t];
+      s_part[t] = acc;
+      acc += v;
+      acc_sq += s_sq[t];
+    }
+    s_total = acc;
+    ess_out[blockIdx.x] = (float)(acc * acc / acc_sq);
+  }
+  for (int w = 0; w < nw; ++w) last = max(last, s_last[w]);
+  __syncthreads();
+  const double P = s_part[tid], E = P + S, total = s_total;
+
+  // one uniform per (seed, segment, round): 53 bits of Philox4x32-10
+  uint32_t c[4] = {(uint32_t)blockIdx.x, (uint32_t)round, tag, (uint32_t)((unsigned long long)round >> 32)};
+  philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));
+  const double u = ((double)(c[0] >> 5) * 67108864.0 + (double)(c[1] >> 6)) * 1.1102230246251565e-16;
+  const double n = (double)seg_len;
+  // position of child j, scaled by seg_len: (u + j) * C_last (no division: its slow path would spill)
+  auto pos = [&](int j) { return (u + (double)j) * total; };
+  auto first_at_least = [&](double C) {     // smallest j in [0, seg_len] with pos(j) >= seg_len * C
+    const double x = n * C;
+    int lo = 0, hi = seg_len;
+    while (lo < hi) {
+      const int mid = (lo + hi) >> 1;
+      if (pos(mid) >= x) hi = mid; else lo = mid + 1;
+    }
+    return lo;
+  };
+  if (S > 0.0) {                            // children with P <= position < E fall on this thread's particles
+    int j = first_at_least(P);
+    const int j_end = first_at_least(E);
+    double acc = 0.0;
+    for (int i = a; i < b && j < j_end; ++i) {
+      acc += fk_weight(reward, carried, i, lam, m);
+      const double C = n * (P + acc);
+      for (; j < j_end && pos(j) < C; ++j) { ancestor_out[j] = base + i; carried_out[j] = reward[i]; }
+    }
+  }
+  for (int j = first_at_least(total) + tid; j < seg_len; j += nt) {
+    ancestor_out[j] = base + last;
+    carried_out[j] = reward[last];
+  }
+}
+
 // Inputs of the denoising verifier: out[i*S + s] = a_s * x[i] + b_s * eps_tab[s] (image-major, level-minor), one
 // float4 per thread, separately rounded mul / mul / add (torch's `a * x + b * eps` in fp32).
 __global__ void __launch_bounds__(256) level_inputs_kernel(float* __restrict__ out, const float* __restrict__ x,
@@ -359,6 +479,22 @@ extern "C" int its_topk_first_segmented(int32_t* idx_out, float* val_out, const 
   const int threads = seg_len >= 1024 ? 1024 : (seg_len + 31) / 32 * 32;
   ITS_LAUNCH(its::topk_first_kernel, dim3(n_seg), dim3(threads), 0, its::as_stream(stream), idx_out, val_out, scores,
              seg_len, k);
+  ITS_CHECK_LAUNCH();
+  return ITS_OK;
+}
+
+extern "C" int its_resample_systematic(int32_t* ancestor_out, float* carried_out, float* ess_out, const float* reward,
+                                       const float* carried_in, float lam, int32_t n_seg, int32_t seg_len,
+                                       uint64_t seed, int64_t round, int32_t tag, void* stream) {
+  ITS_REQUIRE(ancestor_out && carried_out && ess_out && reward, "its_resample_systematic: null pointer");
+  ITS_REQUIRE(n_seg >= 1 && seg_len >= 1, "its_resample_systematic: n_seg=%d seg_len=%d must be >= 1", n_seg,
+              seg_len);
+  ITS_REQUIRE((long long)n_seg * seg_len <= INT32_MAX, "its_resample_systematic: n_seg * seg_len = %lld exceeds int32",
+              (long long)n_seg * seg_len);
+  ITS_REQUIRE(isfinite(lam) && lam >= 0.f, "its_resample_systematic: lam=%g must be finite and >= 0", (double)lam);
+  const int threads = seg_len >= its::kResampleThreads ? its::kResampleThreads : (seg_len + 31) / 32 * 32;
+  ITS_LAUNCH(its::resample_systematic_kernel, dim3(n_seg), dim3(threads), 0, its::as_stream(stream), ancestor_out,
+             carried_out, ess_out, reward, carried_in, lam, (int)seg_len, seed, (long long)round, (uint32_t)tag);
   ITS_CHECK_LAUNCH();
   return ITS_OK;
 }

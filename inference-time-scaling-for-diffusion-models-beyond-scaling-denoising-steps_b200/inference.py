@@ -11,8 +11,8 @@ reference (SURVEY.md §8f rows 1 and 3), without Hydra.
     the sampler's step graph (`forward(..., t_start=a, t_stop=b)`), so tracking costs nothing between
     metric points.  Calculators are duck-typed (FID / IS / CLIP weights are third-party downloads the
     reference fetches at run time, SURVEY.md §8c): pass the reference's own objects, or None.
-  * run_search               — config-driven search (random / zero_order / path / search_over_paths) with the
-                               kernel verifiers
+  * run_search               — config-driven search (random / zero_order / path / search_over_paths /
+                               fk_steering) with the kernel verifiers
   * save_image_grid          — torchvision.utils.save_image grid as the reference writes it (:621-628)
 
     python -m its_b200.inference config/inference_config.yaml T=1000 img_size=32 batch_size=64
@@ -289,15 +289,17 @@ def make_verifier(name: str, sampler=None, *, n_levels: int = 8, seed: int = 0, 
 
 def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Optional[int] = None):
     """`search:` block of the config -> (best_noise, best_score, images of the best candidate).
-    Keys: algorithm (random | zero_order | path | search_over_paths), verifier (oracle | self_supervised |
+    Keys: algorithm (random | zero_order | path | search_over_paths | fk_steering), verifier (oracle | self_supervised |
     aesthetic | denoising | diffusion_classifier; the last two score with the sampler's own model at score_levels
     (8) noise levels drawn from score_seed (0), in chunks of max_images UNet images), n_candidates / n_neighbors / n_iterations / lambda_radius / n_paths / injection_step / noise_scale
     (defaults: the reference constructors', search_algorithm.py:24,98-100,246-248), batch_size,
     img_size.  search_over_paths takes n_beams (4), n_children (4), start_step (800), delta_f (50) and
     delta_b (100), and returns the winner's initial x_T with the images the search itself finished (the winner's
-    path is re-noised along the way: denoising its x_T again would not reproduce it).
-    `n_queries` (K, default 1) > 1 runs K independent random / search_over_paths searches as one population
-    (`search_batch`): `labels` is then [K] or [K, B] (one row per query), and the results are stacked over the
+    path is re-noised along the way: denoising its x_T again would not reproduce it).  fk_steering takes
+    n_particles (4), start_step (800), resample_interval (100) and fk_lambda (10.0), and returns the same pair
+    (a resampled particle's trajectory is not the one its x_T alone would give).
+    `n_queries` (K, default 1) > 1 runs K independent random / search_over_paths / fk_steering searches as one
+    population (`search_batch`): `labels` is then [K] or [K, B] (one row per query), and the results are stacked over the
     queries (best_noise and images [K, B, 3, H, W], a list of K scores).
     With torch.distributed initialised the candidates are sharded over the ranks."""
     from .search import search_algorithm as S
@@ -319,6 +321,11 @@ def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Op
         images, score, _ = search.search(shape, den, ver.score, device=dev, verbose=False, seed=seed)
         best = S.philox_normal((1,) + shape, search.last_seed, search.last_index, S.TAG_X_T, torch.device(device))[0]
         return best, score, images
+    if algo == "fk_steering":
+        search = _fk_steering(sc)
+        images, score, _ = search.search(shape, den, ver.score, device=dev, seed=seed)
+        best = S.philox_normal((1,) + shape, search.last_seed, search.last_index, S.TAG_X_T, torch.device(device))[0]
+        return best, score, images
     if algo == "random":
         search = S.RandomSearch(n_candidates=int(sc.get("n_candidates", 4)))
         best, score = search.search(shape, den, ver.score, device=dev, verbose=False, seed=seed)
@@ -334,7 +341,8 @@ def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Op
                                   noise_scale=float(sc.get("noise_scale", 0.1)))
             best, score, _ = search.search(x0, den, ver.score, device=dev, verbose=False, seed=seed)
         else:
-            raise ValueError(f"search.algorithm {algo!r}: random | zero_order | path | search_over_paths")
+            raise ValueError(f"search.algorithm {algo!r}: random | zero_order | path | search_over_paths | "
+                             "fk_steering")
     # the images of the winner: its own trajectory (the Philox stream of the candidate id it was scored under),
     # so that the returned images are the ones that produced the returned score
     images = None
@@ -348,7 +356,7 @@ def _run_batch(sampler, sc: Dict[str, Any], algo: str, K: int, shape, ver, devic
                seed: Optional[int] = None):
     """run_search for n_queries = K > 1: one `search_batch` over K queries."""
     from .search import search_algorithm as S
-    batched = ("random", "search_over_paths")
+    batched = ("random", "search_over_paths", "fk_steering")
     if algo not in batched:
         raise ValueError(f"search.n_queries={K} needs search.algorithm in {list(batched)}, got {algo!r}")
     den = S.make_denoise_fn(sampler, max_images=int(sc.get("max_images", 256)), seed=seed)
@@ -361,6 +369,12 @@ def _run_batch(sampler, sc: Dict[str, Any], algo: str, K: int, shape, ver, devic
         best = torch.stack([S.philox_normal((1,) + shape, search.last_seed, q * search.n_beams + p, S.TAG_X_T, dev)[0]
                             for q, p in enumerate(search.last_index)])
         return best, scores, images
+    if algo == "fk_steering":
+        search = _fk_steering(sc)
+        images, scores, _ = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev))
+        best = torch.stack([S.philox_normal((1,) + shape, search.last_seed, q * search.n_particles + p, S.TAG_X_T,
+                                            dev)[0] for q, p in enumerate(search.last_index)])
+        return best, scores, images
     search = S.RandomSearch(n_candidates=int(sc.get("n_candidates", 4)))
     best, scores = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev))
     # each winner's images from its own trajectory (the global candidate id it was scored under)
@@ -371,6 +385,12 @@ def _run_batch(sampler, sc: Dict[str, Any], algo: str, K: int, shape, ver, devic
             images[q] = den.denoise_candidates(best[q:q + 1], q * search.n_candidates + i, seed=search.last_seed,
                                                cand_labels=None if rows is None else rows[q:q + 1])[0]
     return best, scores, images
+
+
+def _fk_steering(sc: Dict[str, Any]):
+    from .search import search_algorithm as S
+    return S.FKSteering(n_particles=int(sc.get("n_particles", 4)), start_step=int(sc.get("start_step", 800)),
+                        resample_interval=int(sc.get("resample_interval", 100)), lam=float(sc.get("fk_lambda", 10.0)))
 
 
 def save_image_grid(images: torch.Tensor, path: str, nrow: int = 8) -> str:

@@ -24,9 +24,13 @@ true mid-trajectory restart at `injection_step`).
 SearchOverPaths is not in the reference: it is the search over paths of Ma et al. (a beam of partial
 trajectories, re-noised and pruned by top-k on x0 predictions), in population mode only.
 
-Batched searches (not in the reference): `RandomSearch.search_batch` and `SearchOverPaths.search_batch` run K
+Batched searches (not in the reference): `RandomSearch.search_batch`, `SearchOverPaths.search_batch` and
+`FKSteering.search_batch` run K
 independent queries, each with its own labels, as one candidate population and select every query's winner
 (or survivors) on the device with one segmented top-k.  `search` is the K = 1 case of the same code.
+
+FKSteering is not in the reference either: Feynman-Kac steering of Singhal et al. (a population of particles
+resampled by verifier potentials on their x0 predictions), in population mode only.
 
 GradientBasedSearch (:343-438) needs autograd through the whole trajectory: it is kept
 for arbitrary differentiable callables (callable mode only, the reference's loop); the
@@ -47,6 +51,7 @@ TAG_X_T = X_T_TAG            # candidate x_T draws
 TAG_NEIGHBOR = X_T_TAG + 16  # + iteration
 TAG_PATH = X_T_TAG + 8
 TAG_FORWARD = X_T_TAG + 4    # SearchOverPaths re-noising draws, keyed by round and child
+TAG_RESAMPLE = X_T_TAG + 2   # FKSteering: the one uniform of each systematic resampling, keyed by query and round
 # SearchOverPaths: image b of child c in round r (1-based; the initial paths are round 0) draws its step noise from
 # Philox candidate id r * ROUND_STRIDE + c * B + b
 ROUND_STRIDE = 1 << 40
@@ -253,6 +258,31 @@ def _topk_device(scores: torch.Tensor, k: int, n_seg: int = 1) -> Tuple[torch.Te
                                                        s.numel() // n_seg, int(k), _lib.stream_ptr(s.device)),
                    "its_topk_first_segmented")
     return idx, val
+
+
+def resample_systematic(reward: torch.Tensor, carried: Optional[torch.Tensor], lam: float, n_seg: int, seed: int,
+                        round: int, tag: int = TAG_RESAMPLE) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """Systematic resampling of `n_seg` equal segments of particles by the potentials exp(lam * (reward - carried))
+    (its_resample_systematic; `carried` None = 0), left on the device: (ancestors int32 [n], flat into `reward`
+    like `_topk_device`'s indices, the ancestors' rewards fp32 [n] for the next call's `carried`, ESS fp32
+    [n_seg]).  A segment without a finite weight gets ancestors -1, NaN rewards and ESS 0.  One uniform per
+    (seed, segment, round), so every rank draws the same ancestors from the same gathered rewards."""
+    _lib.require_cuda()
+    r = reward.detach().to(torch.float32).contiguous()
+    if n_seg < 1 or r.numel() % n_seg:
+        raise ValueError(f"{r.numel()} rewards do not split into {n_seg} equal segments")
+    c = None if carried is None else carried.detach().to(device=r.device, dtype=torch.float32).contiguous()
+    if c is not None and c.numel() != r.numel():
+        raise ValueError(f"carried holds {c.numel()} values, reward {r.numel()}")
+    anc = torch.empty(r.numel(), dtype=torch.int32, device=r.device)
+    out = torch.empty(r.numel(), dtype=torch.float32, device=r.device)
+    ess = torch.empty(n_seg, dtype=torch.float32, device=r.device)
+    with torch.cuda.device(r.device):
+        _lib.check(_lib.lib().its_resample_systematic(anc.data_ptr(), out.data_ptr(), ess.data_ptr(), r.data_ptr(),
+                                                      None if c is None else c.data_ptr(), float(lam), int(n_seg),
+                                                      r.numel() // n_seg, int(seed), int(round), int(tag),
+                                                      _lib.stream_ptr(r.device)), "its_resample_systematic")
+    return anc, out, ess
 
 
 def topk_first(scores: torch.Tensor, k: int) -> Tuple[List[int], List[float]]:
@@ -822,6 +852,189 @@ class SearchOverPaths:
         history['unet_image_steps'] = steps * B * (2 if getattr(smp, "guided", False) else 1)
         self.nfes += steps
         return parents[parent_idx.long()].clone(), best.tolist(), history
+
+    def reset_nfes(self):
+        self.nfes = 0
+
+
+# -------------------------------------------------------------- FKSteering --
+def fk_segments(T: int, start_step: int, interval: int) -> List[Tuple[int, int]]:
+    """Segment schedule of Feynman-Kac steering: (t_start, t_stop) per segment, steps t_start ... t_stop inclusive.
+    The first segment is (T-1, start_step); each following one starts one step below the previous stop and runs
+    `interval` steps, (stop - 1, max(stop - interval, 0)); the last one ends with step 0.  The population is
+    resampled after every segment but the last.  Raises ValueError unless 0 <= start_step <= T-1, interval >= 1."""
+    T, s, interval = int(T), int(start_step), int(interval)
+    if T < 1:
+        raise ValueError(f"T={T} must be >= 1")
+    if not 0 <= s <= T - 1:
+        raise ValueError(f"start_step={s} outside [0, T-1={T - 1}]")
+    if interval < 1:
+        raise ValueError(f"resample_interval={interval} must be >= 1")
+    segments = [(T - 1, s)]
+    while segments[-1][1] > 0:
+        stop = segments[-1][1]
+        segments.append((stop - 1, max(stop - interval, 0)))
+    return segments
+
+
+class FKSteering:
+    """Feynman-Kac steering (Singhal et al., "A General Framework for Inference-time Scaling and Steering of
+    Diffusion Models", 2025): `n_particles` (N) trajectories denoised together from x_T (Philox TAG_X_T keyed by
+    particle id, as RandomSearch draws candidates, or `candidate_noise` [N, *noise_shape]).  After each segment of
+    `fk_segments(T, start_step, resample_interval)` but the last, every particle's x0 prediction (the segment's last
+    UNet evaluation, no extra one) is scored and the population is resampled systematically with the potentials
+    exp(lam * (reward - reward at the previous resampling)) (`resample_systematic`).  Nothing is re-noised and no
+    step runs twice: the UNet budget is RandomSearch(N)'s.  The last segment ends at step 0; the best finished
+    sample wins under `argmax_first`'s rule.
+
+    Population mode only: an its_b200 `SamplerDenoiser` and a kernel verifier's `.score`.  Particle j of segment r
+    draws its step noise from Philox candidate id r * ROUND_STRIDE + j * B + image, so segment 0 continues
+    RandomSearch's streams and the copies a resampling makes of one particle go on with streams of their own.
+    Particles are sharded over the ranks; per resampling one score all_gather and one all_gather of the fp32
+    states, and every rank draws the same ancestors.
+
+    `search(noise_shape, denoise_fn, verifier_fn, ...)` returns (best_images [B,C,H,W], best_score, history);
+    keyword extensions: `seed`, `labels`, `candidate_noise`.  history: 'segments'; per resampling 'scores' (N),
+    'ancestors' (N particle ids) and 'ess'; 'lineage', the winner's particle id in every segment (lineage[0] is its
+    x_T id); 'unet_image_steps'.  `last_index` is the winner's x_T id, `last_seed` the search seed; `nfes` counts
+    UNet steps x particles (N * T per search).  `search_batch` runs K such searches, with their own labels, as one
+    population."""
+
+    def __init__(self, n_particles: int = 4, start_step: int = 800, resample_interval: int = 100, lam: float = 10.0):
+        self.n_particles = n_particles
+        self.start_step = start_step
+        self.resample_interval = resample_interval
+        self.lam = lam
+        self.nfes = 0
+
+    def search(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
+               device: str = 'cuda', verbose: Optional[bool] = None,
+               **kwargs) -> Tuple[torch.Tensor, float, Dict[str, Any]]:
+        cand_noise = kwargs.pop("candidate_noise", None)
+        seed = kwargs.pop("seed", None)
+        shape = tuple(noise_shape)
+        ver, segments = self._schedule(denoise_fn, verifier_fn)
+        _check_shape("candidate_noise", cand_noise, (int(self.n_particles),) + shape)
+        images, best, h = self._population(shape, denoise_fn, ver, segments, 1, labels=kwargs.get("labels"),
+                                           query_labels=None, cand_noise=cand_noise, seed=seed, device=device)
+        history = {'segments': h['segments'], 'scores': h['scores'][0], 'ancestors': h['ancestors'][0],
+                   'ess': h['ess'][0], 'lineage': h['lineage'][0], 'unet_image_steps': h['unet_image_steps']}
+        self.last_index = history['lineage'][0]
+        return images[0], best[0], history
+
+    def search_batch(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
+                     n_queries: int, *, labels: Optional[torch.Tensor] = None,
+                     candidate_noise: Optional[torch.Tensor] = None, seed: Optional[int] = None,
+                     device: str = 'cuda') -> Tuple[torch.Tensor, List[float], Dict[str, Any]]:
+        """K = `n_queries` independent FK-steering searches evaluated as one population of K*N particles, resampled
+        per query by one segmented kernel launch, with every query's winner selected on the device by one segmented
+        top-k.  Population mode only.
+
+        `labels` [K] or [K, B]: query q's labels (guided sampler; default: the denoiser's own for every query).
+        `candidate_noise` [K, N, *noise_shape]: injected x_T.  Query q's particle j is global particle q*N + j
+        (its x_T draw and step noise are keyed by that id, its resampling uniform by q, ancestors never cross
+        queries), so K = 1 is `search`, query 0 is the single search with query 0's inputs, and a query's result
+        does not depend on the other queries' inputs, the rank count or `max_images`.
+        Returns (best_images [K, *noise_shape], best_scores, history): 'segments' as in `search`; 'scores',
+        'ancestors', 'ess' and 'lineage' are lists over the queries, with within-query ids; 'unet_image_steps' is
+        the whole batch's.  `last_index` is the list of the winners' x_T ids.  A query none of whose particles can
+        be weighted raises ValueError naming the query and the resampling round."""
+        K = _check_queries(n_queries, noise_shape, labels)
+        shape = tuple(noise_shape)
+        ver, segments = self._schedule(denoise_fn, verifier_fn)
+        N = int(self.n_particles)
+        _check_shape("candidate_noise", candidate_noise, (K, N) + shape)
+        images, best, history = self._population(
+            shape, denoise_fn, ver, segments, K, labels=None, query_labels=labels,
+            cand_noise=None if candidate_noise is None else candidate_noise.reshape((K * N,) + shape),
+            seed=seed, device=device)
+        self.last_index = [lin[0] for lin in history['lineage']]
+        return images, best, history
+
+    def _schedule(self, denoise_fn, verifier_fn) -> Tuple[Any, List[Tuple[int, int]]]:
+        """(kernel verifier, segment schedule) after checking the mode and the parameters against sampler.T."""
+        ver = _population_mode(denoise_fn, verifier_fn)
+        if ver is None:
+            raise ValueError("FKSteering needs an its_b200 SamplerDenoiser and a kernel verifier's .score "
+                             "(population mode)")
+        if int(self.n_particles) < 1:
+            raise ValueError(f"n_particles={self.n_particles} must be >= 1")
+        if not (math.isfinite(float(self.lam)) and float(self.lam) >= 0.0):
+            raise ValueError(f"lam={self.lam} must be finite and >= 0")
+        return ver, fk_segments(denoise_fn.sampler.T, self.start_step, self.resample_interval)
+
+    def _population(self, shape: Tuple[int, ...], denoise_fn: SamplerDenoiser, ver, segments, K: int, *, labels,
+                    query_labels, cand_noise, seed, device):
+        """K queries of N particles as one population sharded over the ranks (query q's particle j is global
+        particle q*N + j).  `labels`: shared labels of every particle; `query_labels` ([K] or [K, B]): one label row
+        per query.  Returns (best images [K, *shape], best scores, history with per-query 'scores', 'ancestors',
+        'ess' and 'lineage' in within-query ids)."""
+        N = int(self.n_particles)
+        n = K * N
+        smp = denoise_fn.sampler
+        dist, rank, world = _dist()
+        dev = torch.device(device)
+        seed = _shared_seed(seed, dev)
+        self.last_seed = seed
+        B = shape[0]
+        denoise_fn.reset_calls()
+        rows = _label_rows(query_labels, K, N, B, dev)
+        lo, hi = _shard(n, rank, world)
+        history: Dict[str, Any] = {'segments': list(segments), 'scores': [[] for _ in range(K)],
+                                   'ancestors': [[] for _ in range(K)], 'ess': [[] for _ in range(K)]}
+        steps = 0                                     # UNet steps x particles
+        carried = None
+        with torch.no_grad():
+            if cand_noise is not None:
+                local = cand_noise[lo:hi].to(dev, torch.float32)
+            elif hi > lo:
+                local = philox_normal((hi - lo,) + shape, seed, lo, TAG_X_T, dev)
+            else:
+                local = torch.empty((0,) + shape, device=dev)
+            for r, (t_start, t_stop) in enumerate(segments):
+                last = t_stop == 0
+                if hi > lo:
+                    local, x0 = denoise_fn.denoise_segment(local, lo, t_start=t_start, t_stop=t_stop, labels=labels,
+                                                           seed=seed, cand_offset=r * ROUND_STRIDE, x0=True,
+                                                           cand_labels=_rows(rows, lo, hi))
+                    judged = local if last else x0    # the last segment scores the finished, clipped samples
+                    local_scores = _score_candidates(ver, judged.reshape(-1, *shape[1:]), B, denoise_fn, labels,
+                                                     _rows(rows, lo, hi))
+                else:
+                    local_scores = torch.empty(0, dtype=torch.float32, device=dev)
+                steps += n * (t_start - t_stop + 1)
+                scores = _gather_scores(local_scores, n)
+                states = _gather_states(local.contiguous(), n)
+                if last:
+                    break
+                anc, carried, ess = resample_systematic(scores, carried, self.lam, K, seed, r)
+                ids, vals, ess_q = anc.tolist(), scores.view(K, N).tolist(), ess.tolist()
+                for q in range(K):
+                    own = [i - q * N if i >= 0 else -1 for i in ids[q * N:(q + 1) * N]]
+                    if own[0] < 0:
+                        raise ValueError(f"{_query(K, q)}resampling round {r}: none of the {N} particles has a "
+                                         "finite score to weight")
+                    history['scores'][q].append(vals[q])
+                    history['ancestors'][q].append(own)
+                    history['ess'][q].append(ess_q[q])
+                local = states.index_select(0, anc[lo:hi].long())
+            idx, best = _topk_device(scores, 1, n_seg=K)
+            winners = idx.tolist()
+        history['lineage'] = []
+        for q, i in enumerate(winners):
+            if i < 0:
+                raise ValueError(f"{_query(K, q)}last segment: none of the {N} finished samples has a score that can "
+                                 "be ranked")
+            j = i - q * N
+            lineage = [j]
+            for own in reversed(history['ancestors'][q]):
+                j = own[j]
+                lineage.append(j)
+            lineage.reverse()
+            history['lineage'].append(lineage)
+        history['unet_image_steps'] = steps * B * (2 if getattr(smp, "guided", False) else 1)
+        self.nfes += steps
+        return states.index_select(0, idx.long()), best.tolist(), history
 
     def reset_nfes(self):
         self.nfes = 0
