@@ -408,6 +408,20 @@ int its_resample_systematic(int32_t* ancestor_out, float* carried_out, float* es
                             const float* reward, const float* carried_in, float lam,
                             int32_t n_seg, int32_t seg_len, uint64_t seed, int64_t round,
                             int32_t tag, void* stream);
+/* Rank ensemble of n_members (V) verifiers (the verifier ensemble of Ma et al.; not in the reference), one CTA
+ * per segment (query).  scores is candidate-major [n_seg*seg_len][V] fp32, weights a device fp32 [V] array (finite
+ * and > 0, checked by the caller).  In segment s, candidate i is eligible when none of its V scores is NaN or
+ * -inf (+inf is an ordinary value); E is the segment's eligible set.  For eligible i and member v:
+ *   r_v(i) = |{j in E : S[j][v] < S[i][v]}| + |{j in E, j != i : S[j][v] == S[i][v]}| / 2
+ *            (average ranks counted from 0: scipy's rankdata(method="average") - 1 over E)
+ *   out[i] = (sum_v w_v r_v(i)) / ((sum_v w_v) (|E| - 1))  in double, member order, each product and sum
+ *            separately rounded, then rounded to fp32; 1.0 when |E| = 1
+ * and out[i] = NaN for an ineligible i, so it never ranks in its_topk_first_segmented.  out lies in [0, 1], higher
+ * is better, and depends only on the segment's own scores.  Cost O(V seg_len^2) comparisons per segment; shared
+ * memory is a fixed 8 KB tile.  Requires n_members in [1, 8], n_seg, seg_len >= 1 and n_seg * seg_len <=
+ * INT32_MAX; no allocation, no synchronisation, no atomics.                                                  */
+int its_rank_ensemble(float* out, const float* scores, const float* weights, int32_t n_members,
+                      int32_t n_seg, int32_t seg_len, void* stream);
 
 /* ------------------------------------------------------------------------
  * Denoising verifier: the diffusion model scores a sample by how well it

@@ -23,7 +23,7 @@ SYMBOLS = [
     "its_attention_flash", "its_attention_group", "its_conv_gn_sync_words",
     "its_f32_nchw_to_nhwc", "its_f32_conv2d", "its_f32_group_norm", "its_f32_attention",
     "its_topk_first", "its_ddpm_step_x0", "its_path_expand", "its_topk_first_segmented",
-    "its_level_inputs", "its_denoise_scores", "its_resample_systematic",
+    "its_level_inputs", "its_denoise_scores", "its_resample_systematic", "its_rank_ensemble",
 ]
 
 
@@ -117,6 +117,7 @@ def lib() -> C.CDLL:
     L.its_level_inputs.argtypes = [vp, vp, vp, vp, i32, i32, i64, vp]
     L.its_denoise_scores.argtypes = [vp, vp, vp, vp, i32, i32, i32, i64, vp]
     L.its_resample_systematic.argtypes = [vp, vp, vp, vp, vp, f32, i32, i32, u64, i64, i32, vp]
+    L.its_rank_ensemble.argtypes = [vp, vp, vp, i32, i32, i32, vp]
     for s in SYMBOLS:
         if s not in ("its_version", "its_last_error_string"):
             getattr(L, s).restype = i32

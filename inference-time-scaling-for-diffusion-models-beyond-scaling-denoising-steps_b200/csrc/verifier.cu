@@ -1,7 +1,7 @@
 // Verifier statistics, per-candidate scores and first-index argmax
 // and (segmented) top-k (search/verifier.py:45-66, 207-248, 262-287; search/search_algorithm.py:79-81); the two
 // ends of the denoising verifier around its UNet pass (level inputs, per-candidate denoising error); systematic
-// resampling of Feynman-Kac particles.
+// resampling of Feynman-Kac particles; the rank ensemble of several verifiers' scores.
 // All reductions are warp-shuffle + one shared-memory hop.
 #include "its_common.cuh"
 
@@ -334,6 +334,91 @@ __global__ void __launch_bounds__(kResampleThreads) resample_systematic_kernel(
   }
 }
 
+// Rank ensemble of V member verifiers, one CTA per segment (query).  Candidate i of the segment is eligible when
+// none of its V scores is NaN or -inf; for an eligible i and member v, r_v(i) = #{eligible j: S_jv < S_iv} +
+// (#{eligible j: S_jv == S_iv} - 1) / 2 (average ranks from 0, exact half-integers), and
+// out_i = (sum_v w_v r_v(i)) / ((sum_v w_v) (|E| - 1)) in double, member order, separately rounded (no FMA), then
+// fp32; 1 when |E| = 1, NaN for an ineligible i.  Thread t owns candidates t, t + nt, ...; the comparison partners
+// stream through a tile of nt candidates in shared memory, so shared memory does not grow with seg_len.  Counts are
+// per-thread integers: no atomics, and the output does not depend on the launch shape.
+constexpr int kRankThreads = 256;
+constexpr int kRankMaxMembers = 8;
+
+__device__ __forceinline__ bool rank_eligible(float x) { return !(isnan(x) || x == -INFINITY); }
+
+__global__ void __launch_bounds__(kRankThreads) rank_ensemble_kernel(float* __restrict__ out,
+                                                                     const float* __restrict__ scores,
+                                                                     const float* __restrict__ weights, int V,
+                                                                     int seg_len) {
+  pdl_prologue();
+  __shared__ float s_tile[kRankThreads * kRankMaxMembers];
+  __shared__ unsigned char s_ok[kRankThreads];
+  const int tid = threadIdx.x, nt = blockDim.x;
+  const long long base = (long long)blockIdx.x * seg_len;   // n_seg * seg_len fits int32 (checked on the host)
+  scores += base * V;
+  out += base;
+  for (int i0 = 0; i0 < seg_len; i0 += nt) {
+    const int i = i0 + tid;
+    float mine[kRankMaxMembers];
+    int less[kRankMaxMembers], eq[kRankMaxMembers];
+    bool ok = i < seg_len;
+#pragma unroll
+    for (int v = 0; v < kRankMaxMembers; ++v) {
+      mine[v] = (v < V && i < seg_len) ? scores[(long long)i * V + v] : 0.f;
+      if (v < V) ok = ok && rank_eligible(mine[v]);
+      less[v] = 0;
+      eq[v] = 0;
+    }
+    int n_ok = 0;
+    for (int j0 = 0; j0 < seg_len; j0 += nt) {
+      const int cnt = min(nt, seg_len - j0);
+      __syncthreads();                      // the previous tile has been read
+      const float* src = scores + (long long)j0 * V;
+      for (int e = tid; e < cnt * V; e += nt) s_tile[e] = src[e];
+      __syncthreads();
+      if (tid < cnt) {
+        bool okj = true;
+        for (int v = 0; v < V; ++v) okj = okj && rank_eligible(s_tile[tid * V + v]);
+        s_ok[tid] = okj;
+      }
+      __syncthreads();
+      if (!ok) continue;
+      for (int jj = 0; jj < cnt; ++jj) {
+        if (!s_ok[jj]) continue;
+        ++n_ok;
+#pragma unroll
+        for (int v = 0; v < kRankMaxMembers; ++v) {
+          if (v < V) {
+            const float x = s_tile[jj * V + v];
+            less[v] += x < mine[v];
+            eq[v] += x == mine[v];
+          }
+        }
+      }
+    }
+    if (i >= seg_len) continue;
+    if (!ok) {
+      out[i] = __int_as_float(0x7fc00000);
+      continue;
+    }
+    if (n_ok == 1) {
+      out[i] = 1.0f;
+      continue;
+    }
+    double num = 0.0, wsum = 0.0;
+    for (int v = 0; v < V; ++v) {
+      double r = 0.0;
+#pragma unroll
+      for (int u = 0; u < kRankMaxMembers; ++u)       // register arrays: select member v without local memory
+        if (u == v) r = (double)less[u] + 0.5 * (double)(eq[u] - 1);
+      const double w = (double)__ldg(weights + v);
+      num = __dadd_rn(num, __dmul_rn(w, r));
+      wsum = __dadd_rn(wsum, w);
+    }
+    out[i] = (float)__ddiv_rn(num, __dmul_rn(wsum, (double)(n_ok - 1)));
+  }
+}
+
 // Inputs of the denoising verifier: out[i*S + s] = a_s * x[i] + b_s * eps_tab[s] (image-major, level-minor), one
 // float4 per thread, separately rounded mul / mul / add (torch's `a * x + b * eps` in fp32).
 __global__ void __launch_bounds__(256) level_inputs_kernel(float* __restrict__ out, const float* __restrict__ x,
@@ -495,6 +580,21 @@ extern "C" int its_resample_systematic(int32_t* ancestor_out, float* carried_out
   const int threads = seg_len >= its::kResampleThreads ? its::kResampleThreads : (seg_len + 31) / 32 * 32;
   ITS_LAUNCH(its::resample_systematic_kernel, dim3(n_seg), dim3(threads), 0, its::as_stream(stream), ancestor_out,
              carried_out, ess_out, reward, carried_in, lam, (int)seg_len, seed, (long long)round, (uint32_t)tag);
+  ITS_CHECK_LAUNCH();
+  return ITS_OK;
+}
+
+extern "C" int its_rank_ensemble(float* out, const float* scores, const float* weights, int32_t n_members,
+                                 int32_t n_seg, int32_t seg_len, void* stream) {
+  ITS_REQUIRE(out && scores && weights, "its_rank_ensemble: null pointer");
+  ITS_REQUIRE(n_members >= 1 && n_members <= its::kRankMaxMembers, "its_rank_ensemble: n_members=%d outside [1, %d]",
+              n_members, its::kRankMaxMembers);
+  ITS_REQUIRE(n_seg >= 1 && seg_len >= 1, "its_rank_ensemble: n_seg=%d seg_len=%d must be >= 1", n_seg, seg_len);
+  ITS_REQUIRE((long long)n_seg * seg_len <= INT32_MAX, "its_rank_ensemble: n_seg * seg_len = %lld exceeds int32",
+              (long long)n_seg * seg_len);
+  const int threads = seg_len >= its::kRankThreads ? its::kRankThreads : (seg_len + 31) / 32 * 32;
+  ITS_LAUNCH(its::rank_ensemble_kernel, dim3(n_seg), dim3(threads), 0, its::as_stream(stream), out, scores, weights,
+             (int)n_members, (int)seg_len);
   ITS_CHECK_LAUNCH();
   return ITS_OK;
 }

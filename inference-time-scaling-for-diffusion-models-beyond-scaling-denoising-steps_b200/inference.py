@@ -268,10 +268,23 @@ def sample_with_metrics_tracking(sampler, x_T: torch.Tensor, fid_calculator=None
 DENOISING_VERIFIERS = {"denoising": "likelihood", "diffusion_classifier": "class"}
 
 
-def make_verifier(name: str, sampler=None, *, n_levels: int = 8, seed: int = 0, max_images: int = 256):
+def make_verifier(name: str, sampler=None, *, n_levels: int = 8, seed: int = 0, max_images: int = 256,
+                  ensemble=None, ensemble_weights=None):
     """Verifier by config name.  `denoising` / `diffusion_classifier` are the sampler's own model scoring its
-    samples (DenoisingVerifier, kinds likelihood / class) and need `sampler`; the class form needs the guided net."""
+    samples (DenoisingVerifier, kinds likelihood / class) and need `sampler`; the class form needs the guided net.
+    The name `ensemble` builds an EnsembleVerifier of the verifiers named in the keyword list `ensemble` (each built
+    as it would be alone), weighted by `ensemble_weights` (default: all 1)."""
     from .search import verifier as V
+    if name == "ensemble":
+        if not isinstance(ensemble, (list, tuple)) or not ensemble:
+            raise ValueError("verifier 'ensemble' needs search.ensemble: a non-empty list of verifier names")
+        if "ensemble" in ensemble:
+            raise ValueError("search.ensemble cannot name 'ensemble': ensembles do not nest")
+        if ensemble_weights is not None and not isinstance(ensemble_weights, (list, tuple)):
+            raise ValueError(f"search.ensemble_weights must be a list of floats, got {ensemble_weights!r}")
+        members = [make_verifier(str(m), sampler, n_levels=n_levels, seed=seed, max_images=max_images)
+                   for m in ensemble]
+        return V.EnsembleVerifier(members, ensemble_weights)
     table = {"oracle": V.OracleVerifier, "self_supervised": V.SelfSupervisedVerifier, "aesthetic": V.AestheticPredictor}
     if name in DENOISING_VERIFIERS:
         if sampler is None:
@@ -290,8 +303,11 @@ def make_verifier(name: str, sampler=None, *, n_levels: int = 8, seed: int = 0, 
 def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Optional[int] = None):
     """`search:` block of the config -> (best_noise, best_score, images of the best candidate).
     Keys: algorithm (random | zero_order | path | search_over_paths | fk_steering), verifier (oracle | self_supervised |
-    aesthetic | denoising | diffusion_classifier; the last two score with the sampler's own model at score_levels
-    (8) noise levels drawn from score_seed (0), in chunks of max_images UNet images), n_candidates / n_neighbors / n_iterations / lambda_radius / n_paths / injection_step / noise_scale
+    aesthetic | denoising | diffusion_classifier | ensemble; denoising and diffusion_classifier score with the
+    sampler's own model at score_levels (8) noise levels drawn from score_seed (0), in chunks of max_images UNet
+    images; ensemble ranks the candidates of each query under every verifier named in the list `ensemble` and
+    averages the ranks with the weights `ensemble_weights` (default all 1.0), for random, path and
+    search_over_paths only), n_candidates / n_neighbors / n_iterations / lambda_radius / n_paths / injection_step / noise_scale
     (defaults: the reference constructors', search_algorithm.py:24,98-100,246-248), batch_size,
     img_size.  search_over_paths takes n_beams (4), n_children (4), start_step (800), delta_f (50) and
     delta_b (100), and returns the winner's initial x_T with the images the search itself finished (the winner's
@@ -308,7 +324,8 @@ def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Op
     B, H = int(config.get("batch_size", 1)), int(config["img_size"])
     shape = (B, 3, H, H)
     ver = make_verifier(sc.get("verifier", "oracle"), sampler, n_levels=int(sc.get("score_levels", 8)),
-                        seed=int(sc.get("score_seed", 0)), max_images=int(sc.get("max_images", 256)))
+                        seed=int(sc.get("score_seed", 0)), max_images=int(sc.get("max_images", 256)),
+                        ensemble=sc.get("ensemble"), ensemble_weights=sc.get("ensemble_weights"))
     K = int(sc.get("n_queries", 1))
     if K > 1:
         return _run_batch(sampler, sc, algo, K, shape, ver, device, labels=labels, seed=seed)

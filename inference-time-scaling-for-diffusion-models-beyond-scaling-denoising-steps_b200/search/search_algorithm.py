@@ -32,6 +32,11 @@ independent queries, each with its own labels, as one candidate population and s
 FKSteering is not in the reference either: Feynman-Kac steering of Singhal et al. (a population of particles
 resampled by verifier potentials on their x0 predictions), in population mode only.
 
+A rank ensemble (`verifier.EnsembleVerifier`) scores relative to a population: RandomSearch, PathSearch and
+SearchOverPaths gather its [n, V] member scores and combine them per query right after the gather, on every rank,
+with the segments the selection uses.  ZeroOrderSearch and FKSteering compare scores across populations and refuse
+it.
+
 GradientBasedSearch (:343-438) needs autograd through the whole trajectory: it is kept
 for arbitrary differentiable callables (callable mode only, the reference's loop); the
 kernel sampler is not differentiable and is refused with a clear error.
@@ -323,11 +328,35 @@ def _score_candidates(ver, images: torch.Tensor, B: int, denoise: SamplerDenoise
     return ver.score_candidates(images, B, labels=denoise.image_labels(images.shape[0] // B, labels, cand_labels))
 
 
+def _no_scores(ver, device) -> torch.Tensor:
+    """The score block of a rank that owns no candidates: [0] fp32, or [0, V] for a rank ensemble of V members (its
+    gathered scores are the [n, V] member matrix)."""
+    shape = (0, len(ver.members)) if getattr(ver, "ranks_population", False) else (0,)
+    return torch.empty(shape, dtype=torch.float32, device=device)
+
+
+def _combine(ver, scores: torch.Tensor, n_seg: int) -> torch.Tensor:
+    """One score per candidate from the gathered scores: a rank ensemble ranks its member matrix within each of
+    `n_seg` equal segments (one query's population each); any other verifier's scores are returned as they are
+    (no copy, no launch)."""
+    if not getattr(ver, "ranks_population", False):
+        return scores
+    return ver.combine(scores, n_seg)
+
+
+def _refuse_ranks(verifier_fn, search: str, why: str) -> None:
+    """Searches that compare scores of different populations cannot use a population-relative verifier."""
+    if getattr(getattr(verifier_fn, "__self__", None), "ranks_population", False):
+        raise ValueError(f"{search} cannot use a rank ensemble: {why}, and ranks from different populations "
+                         "cannot be compared")
+
+
 def _score_population(cands_local: torch.Tensor, lo: int, n_total: int, denoise: SamplerDenoiser, ver,
-                      kwargs, t_start=None, seed=None, cand_labels=None) -> torch.Tensor:
+                      kwargs, t_start=None, seed=None, cand_labels=None, n_seg: int = 1) -> torch.Tensor:
     """Denoise + score this rank's block of candidates, return ALL n_total scores.  `seed`: the search's
     shared seed, used for the step noise when the denoiser has none of its own (same on every rank).
-    `cand_labels`: label rows of this rank's candidates ([n_local, B]), else kwargs' `labels` for all."""
+    `cand_labels`: label rows of this rank's candidates ([n_local, B]), else kwargs' `labels` for all.
+    A rank ensemble's member scores are combined over `n_seg` equal segments of the population."""
     B = cands_local.shape[1] if cands_local.numel() else 1
     if cands_local.shape[0] > 0:
         imgs = denoise.denoise_candidates(cands_local, lo, labels=kwargs.get("labels"), t_start=t_start, seed=seed,
@@ -335,8 +364,8 @@ def _score_population(cands_local: torch.Tensor, lo: int, n_total: int, denoise:
         local = _score_candidates(ver, imgs.reshape(-1, *imgs.shape[2:]), B, denoise, kwargs.get("labels"),
                                   cand_labels)
     else:
-        local = torch.empty(0, dtype=torch.float32, device=cands_local.device)
-    return _gather_scores(local, n_total)
+        local = _no_scores(ver, cands_local.device)
+    return _combine(ver, _gather_scores(local, n_total), n_seg)
 
 
 def _check_queries(n_queries: int, noise_shape: Sequence[int], labels: Optional[torch.Tensor]) -> int:
@@ -456,7 +485,7 @@ class RandomSearch:
                 if hi > lo else torch.empty((0, *noise_shape), device=dev)
         with torch.no_grad():
             scores = _score_population(local, lo, n, denoise_fn, ver, kwargs, seed=seed,
-                                       cand_labels=_rows(cand_labels, lo, hi))
+                                       cand_labels=_rows(cand_labels, lo, hi), n_seg=K)
         self.nfes += n
         self.last_scores = scores.view(K, N)
         idx, val = _topk_device(scores, 1, n_seg=K)
@@ -494,6 +523,8 @@ class ZeroOrderSearch:
     def search(self, initial_noise: torch.Tensor, denoise_fn: Callable, verifier_fn: Callable,
                device: str = 'cuda', verbose: Optional[bool] = None,
                **kwargs) -> Tuple[torch.Tensor, float, Dict[str, Any]]:
+        _refuse_ranks(verifier_fn, "ZeroOrderSearch", "it compares each round's best with the best of earlier "
+                      "rounds")
         perts = kwargs.pop("perturbations", None)    # [iters][K, *shape] injected N(0,1) draws
         seed = kwargs.pop("seed", None)
         ver = _population_mode(denoise_fn, verifier_fn)
@@ -818,9 +849,9 @@ class SearchOverPaths:
                                                      _rows(child_labels, lo, hi))
                 else:
                     states = torch.empty((0,) + shape, device=dev)
-                    local_scores = torch.empty(0, dtype=torch.float32, device=dev)
+                    local_scores = _no_scores(ver, dev)
                 steps += n_c * (sp - e + 1)
-                scores = _gather_scores(local_scores, n_c)
+                scores = _combine(ver, _gather_scores(local_scores, n_c), K)
                 history['rounds'].append((s, sp, e))
                 for q, row in enumerate(scores.view(K, NM).tolist()):
                     history['scores'][q].append(row)
@@ -953,6 +984,8 @@ class FKSteering:
 
     def _schedule(self, denoise_fn, verifier_fn) -> Tuple[Any, List[Tuple[int, int]]]:
         """(kernel verifier, segment schedule) after checking the mode and the parameters against sampler.T."""
+        _refuse_ranks(verifier_fn, "FKSteering", "it weights particles by the change of their reward between "
+                      "resamplings")
         ver = _population_mode(denoise_fn, verifier_fn)
         if ver is None:
             raise ValueError("FKSteering needs an its_b200 SamplerDenoiser and a kernel verifier's .score "

@@ -4,6 +4,8 @@
 reduction kernels of libits_b200 (its_image_stats / its_candidate_scores); the
 extra `.score_candidates(images, per_cand)` returns one score per candidate as a
 device tensor so a whole population is scored without a host round-trip.
+EnsembleVerifier combines several of them by each candidate's rank within its
+query's population (its_rank_ensemble).
 
 SupervisedVerifier, CLIPScore and IntegratedVerifier (:69-188, :290-388) wrap
 openai-CLIP, which is not installed and whose weights cannot be fetched: parity
@@ -257,6 +259,86 @@ class DenoisingVerifier(_KernelVerifier):
     def score(self, images: torch.Tensor, labels: Optional[torch.Tensor] = None) -> float:
         """The whole batch as one candidate (the reference's verifier protocol)."""
         return float(self.score_candidates(images, images.shape[0], labels).item())
+
+
+MAX_ENSEMBLE = 8     # its_rank_ensemble's member limit
+
+
+def rank_ensemble(scores: torch.Tensor, weights: torch.Tensor, n_seg: int = 1) -> torch.Tensor:
+    """[n] fp32 device tensor: the rank ensemble (its_rank_ensemble) of the member scores [n, V] over `n_seg`
+    equal segments, with device fp32 `weights` [V].  Eligible candidates score in [0, 1], higher is better; a
+    candidate with a NaN or -inf member score gets NaN."""
+    _lib.require_cuda()
+    s = scores.detach().to(torch.float32).contiguous()
+    if s.dim() != 2 or not 1 <= s.shape[1] <= MAX_ENSEMBLE:
+        raise ValueError(f"member scores must be [n, V] with 1 <= V <= {MAX_ENSEMBLE}, got {tuple(s.shape)}")
+    n, V = s.shape
+    if n_seg < 1 or n % n_seg:
+        raise ValueError(f"{n} candidates do not split into {n_seg} equal segments")
+    w = weights.to(device=s.device, dtype=torch.float32).contiguous()
+    if w.numel() != V:
+        raise ValueError(f"{w.numel()} weights for {V} members")
+    out = torch.empty(n, dtype=torch.float32, device=s.device)
+    with torch.cuda.device(s.device):
+        _lib.check(_lib.lib().its_rank_ensemble(out.data_ptr(), s.data_ptr(), w.data_ptr(), V, int(n_seg), n // n_seg,
+                                                _lib.stream_ptr(s.device)), "its_rank_ensemble")
+    return out
+
+
+class EnsembleVerifier(_KernelVerifier):
+    """Several kernel verifiers combined by rank (the verifier ensemble of Ma et al., a guard against one verifier
+    being exploited by a large search; not in the reference).  Each member scores the same candidates; within each
+    query's population a candidate's score is the weighted mean of its average ranks under the members, scaled to
+    [0, 1] (`rank_ensemble`).  Ranks do not depend on the members' scales, so a likelihood of ~-0.1, a class gap of
+    ~1e-4 and a pixel statistic weigh as the weights say.
+
+    A rank exists only within a population, so the searches use an ensemble in population mode: they gather the
+    member scores [n, V] (`score_candidates`) and turn them into one score per candidate with `combine` before
+    selecting.  `score` (one batch as one candidate) raises.  Zero-order search and FK steering compare scores of
+    different populations and refuse an ensemble (`ranks_population`)."""
+    ranks_population = True
+
+    def __init__(self, members, weights=None):
+        members = list(members)
+        if not 1 <= len(members) <= MAX_ENSEMBLE:
+            raise ValueError(f"an ensemble takes 1 to {MAX_ENSEMBLE} members, got {len(members)}")
+        for m in members:
+            if isinstance(m, EnsembleVerifier):
+                raise ValueError("an ensemble cannot be a member of another ensemble")
+            if not isinstance(m, _KernelVerifier):
+                raise ValueError(f"ensemble member {type(m).__name__} is not a kernel verifier")
+            if isinstance(m, OracleVerifier) and m.dataset_stats is not None:
+                raise ValueError("an OracleVerifier with dataset_stats scores a batch, not candidates: it cannot be "
+                                 "an ensemble member")
+        w = [1.0] * len(members) if weights is None else [float(x) for x in weights]
+        if len(w) != len(members):
+            raise ValueError(f"{len(w)} ensemble weights for {len(members)} members")
+        if not all(np.isfinite(x) and x > 0.0 for x in w):
+            raise ValueError(f"ensemble weights must be finite and > 0, got {w}")
+        self.members = members
+        self.weights = w
+        self.uses_labels = any(getattr(m, "uses_labels", False) for m in members)
+        self._w: Dict[str, torch.Tensor] = {}
+
+    def score_candidates(self, images: torch.Tensor, per_cand: int,
+                         labels: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """[n_cand, V] fp32 device scores: column v is member v's scores of the same candidates; `labels` go to the
+        members that use them."""
+        cols = [m.score_candidates(images, per_cand, labels=labels) if getattr(m, "uses_labels", False)
+                else m.score_candidates(images, per_cand) for m in self.members]
+        return torch.stack(cols, dim=1)
+
+    def combine(self, scores: torch.Tensor, n_seg: int) -> torch.Tensor:
+        """[n] ensemble scores of the gathered member scores [n, V], ranked within each of `n_seg` equal segments."""
+        key = str(scores.device)
+        w = self._w.get(key)
+        if w is None:
+            w = self._w[key] = torch.tensor(self.weights, dtype=torch.float32, device=scores.device)
+        return rank_ensemble(scores, w, n_seg)
+
+    def score(self, images: torch.Tensor, labels: Optional[torch.Tensor] = None) -> float:
+        raise ValueError("a rank ensemble scores a population: one image batch has no rank.  Pass the ensemble's "
+                         ".score to a search with a SamplerDenoiser, or use score_candidates + combine")
 
 
 def _need_clip():
