@@ -107,6 +107,24 @@ int its_ddpm_step_x0(float* x, float* x0_out, const float* eps_c,
                      const int64_t* cand_dev, int32_t* nan_flag,
                      int32_t clip_last, void* stream);
 
+/* its_ddpm_step_x0 with one guidance weight per image, for searches over the
+ * weight: image i of the launch mixes (DiffusionCondition.py:85)
+ *   eps = w_img[2i+1] * eps_c - w_img[2i] * eps_u
+ * with separately rounded mul / mul / sub.  w_img is a device array of n_img
+ * fp32 pairs {w, 1 + w} (8-byte aligned), each formed on the host from the
+ * double w as its_ddpm_step_x0 forms its scalars: (float)w, (float)(1.0 + w).
+ * With every pair equal, the output is its_ddpm_step_x0's bit for bit (same
+ * kernel body: posterior mean, noise, x0 prediction, NaN flag, final clip).
+ * eps_u and w_img are required: the entry point only serves the guided path.
+ * ---------------------------------------------------------------------- */
+int its_ddpm_step_x0_w(float* x, float* x0_out, const float* eps_c,
+                       const float* eps_u, const float* noise,
+                       int64_t noise_t_stride, int64_t n_img, int64_t n_per_img,
+                       const float* coef, const float* x0_coef,
+                       const int32_t* t_dev, const float* w_img, uint64_t seed,
+                       const int64_t* cand_dev, int32_t* nan_flag,
+                       int32_t clip_last, void* stream);
+
 /* Children of one search-over-paths round, q(x_s' | x_s) applied to survivors:
  *   out[i] = a * x[parent[(child0 + i) / m]] + b * z[i],   i < n_child
  * torch: a * x[parents] + b * z  (fp32, separately rounded mul / mul / add).

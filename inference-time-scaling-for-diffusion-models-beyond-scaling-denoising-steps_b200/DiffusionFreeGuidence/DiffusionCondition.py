@@ -30,9 +30,11 @@ class GaussianDiffusionSampler(SamplerBase):
         eps = (1. + self.w) * eps - self.w * non_eps
         return self.predict_xt_prev_mean_from_eps(x_t, t, eps=eps), var
 
-    def forward(self, x_T, labels, *, noise=None, seed=None, cand_id0=0, t_start=None, clip=True, t_stop=0):
+    def forward(self, x_T, labels, *, noise=None, seed=None, cand_id0=0, t_start=None, clip=True, t_stop=0,
+                guidance=None):
         """Algorithm 2 with guidance (DiffusionCondition.py:89-105), replaying the
         sampler's captured step graph as the unconditional sampler does.
-        Keyword-only extensions as in the unconditional sampler."""
+        Keyword-only extensions as in the unconditional sampler; `guidance` [B] gives
+        image i its own weight guidance[i] in place of `self.w` (see `segment`)."""
         return self._run(x_T, labels, t_start=t_start, t_stop=t_stop, seed=seed, cand_id0=cand_id0, noise=noise,
-                         clip=clip, want_x0=False, check_nan=True)[0]
+                         clip=clip, want_x0=False, check_nan=True, guidance=guidance)[0]

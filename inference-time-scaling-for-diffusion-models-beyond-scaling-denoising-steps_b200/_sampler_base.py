@@ -20,6 +20,17 @@ from ._unet_base import PlannedUNet
 X_T_TAG = 0x40000000  # Philox step tags >= this never collide with a time step
 
 
+def guidance_pairs(guidance, n_img: int, device) -> torch.Tensor:
+    """[n_img, 2] fp32 {w, 1 + w} per image from `guidance` (1-D tensor or sequence of n_img finite weights), formed
+    in float64 and rounded to fp32 as its_ddpm_step_x0 forms its scalar pair from the Python float w."""
+    g = torch.as_tensor(guidance, dtype=torch.float64).to(device)
+    if g.dim() != 1 or g.shape[0] != n_img:
+        raise ValueError(f"guidance must be 1-D with one weight per image ({n_img}), got shape {list(g.shape)}")
+    if not bool(torch.isfinite(g).all()):
+        raise ValueError("guidance weights must be finite")
+    return torch.stack([g.float(), (1.0 + g).float()], dim=1)
+
+
 def extract(v, t, x_shape):
     """Coefficients at the given timesteps as [B,1,1,...] fp32 (Diffusion.py:9-16)."""
     out = torch.gather(v, index=t, dim=0).float().to(t.device)
@@ -27,16 +38,19 @@ def extract(v, t, x_shape):
 
 
 class _Trajectory:
-    """Device state of one (plan, noise shape, x0, clip) and its captured step graph."""
+    """Device state of one (plan, noise shape, x0, clip[, per-image weights]) and its captured step graph."""
 
-    def __init__(self, plan, x: torch.Tensor, noise_buf: Optional[torch.Tensor], want_x0: bool):
+    def __init__(self, plan, x: torch.Tensor, noise_buf: Optional[torch.Tensor], want_x0: bool,
+                 per_image_w: bool = False):
         self.plan = plan      # the captured graph bakes pointers into this plan: holding it keeps them alive
         self.noise_buf = noise_buf       # [T, *x.shape] injected noise, shared with the plan's other graphs
         self.x0_buf = torch.empty_like(x, dtype=torch.float32) if want_x0 else None
         self.nan_flag = torch.zeros(1, dtype=torch.int32, device=x.device)
         self.cand_dev = torch.zeros(1, dtype=torch.int64, device=x.device)
+        # [B, 2] fp32 {w, 1 + w} per image, written before every replay like cand_dev (its_ddpm_step_x0_w)
+        self.w_img = torch.zeros(x.shape[0], 2, dtype=torch.float32, device=x.device) if per_image_w else None
         self.graph: Optional[torch.cuda.CUDAGraph] = None
-        self.graph_key = None            # (seed or None, w) baked into the graph
+        self.graph_key = None            # (seed or None, w) baked into the graph; w is None with per-image weights
 
 
 class SamplerBase(nn.Module):
@@ -103,19 +117,24 @@ class SamplerBase(nn.Module):
 
     def _run(self, x: torch.Tensor, labels: Optional[torch.Tensor], *, t_start: Optional[int], t_stop: int,
              seed: Optional[int], cand_id0: int, noise: Optional[torch.Tensor], clip: bool, want_x0: bool,
-             check_nan: bool) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+             check_nan: bool, guidance=None) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
         """Steps time_step = t_start (default T-1) ... t_stop of the ancestral loop from state `x` (the x_t that step
         t_start takes) on the device.  Returns (state after step t_stop, clipped when `clip` if t_stop == 0;
         x0 prediction of step t_stop if `want_x0`, else None).  Per-step noise is keyed by (seed, candidate,
         time_step), so a trajectory cut into segments equals the uncut one.  The candidate base `cand_id0` is
         written to device memory, so one captured step graph per (plan, noise shape, x0, clip) is replayed by every
-        call with the same seed and guidance weight."""
+        call with the same seed and guidance weight.  `guidance` (guided sampler): one weight per image instead of
+        `self.w`, on a trajectory of its own whose graph does not bake the weights in (its_ddpm_step_x0_w), so one
+        capture serves every weight vector."""
         first = self.T - 1 if t_start is None else int(t_start)
         if not (0 <= first < self.T):
             raise ValueError(f"t_start={t_start} outside [0, {self.T})")
         t_stop = int(t_stop)
         if not (0 <= t_stop <= first):
             raise ValueError(f"t_stop={t_stop} outside [0, t_start={first}]")
+        if guidance is not None and not self.guided:
+            raise ValueError("guidance weights need the guided sampler (DiffusionFreeGuidence); this one has no "
+                             "unconditional branch to mix")
         _lib.require_cuda()
         L = _lib.lib()
         if x.device.type != "cuda":
@@ -133,10 +152,12 @@ class SamplerBase(nn.Module):
         if seed is None:
             seed = int(torch.randint(0, 2 ** 62, (1,)).item())   # follows torch.manual_seed
         B, Cc, H, W = x.shape
+        per_image_w = guidance is not None
+        w_pairs = guidance_pairs(guidance, B, x.device) if per_image_w else None
         with torch.cuda.device(x.device):   # every launch below goes to this device's current stream
             plan = net.plan(2 * B if self.guided else B, H, W, n_img_in=B, uniform_t=True,
                             impl=getattr(net, "impl", None))
-            key = (plan, n_shape, want_x0, clip)
+            key = (plan, n_shape, want_x0, clip) + (("w_img",) if per_image_w else ())
             tr = self._graphs.get(key)
             if tr is None:
                 live = list(net._plans.values())   # drop the graphs of plans the net has since rebuilt
@@ -144,11 +165,13 @@ class SamplerBase(nn.Module):
                 noise_buf = next((v.noise_buf for k, v in self._graphs.items() if k[:2] == (plan, n_shape)), None)
                 if noise is not None and noise_buf is None:
                     noise_buf = torch.empty(n_shape, dtype=torch.float32, device=x.device)
-                tr = self._graphs[key] = _Trajectory(plan, x, noise_buf, want_x0)
+                tr = self._graphs[key] = _Trajectory(plan, x, noise_buf, want_x0, per_image_w)
             with torch.no_grad():
                 plan.x_in.copy_(x)
                 plan.t_dev.fill_(first)
                 tr.cand_dev.fill_(cand_id0)
+                if per_image_w:
+                    tr.w_img.copy_(w_pairs)
                 tr.nan_flag.zero_()
                 if self.guided:
                     lab = labels.reshape(-1).to(device=x.device, dtype=torch.int64)
@@ -161,15 +184,22 @@ class SamplerBase(nn.Module):
             x0_ptr = tr.x0_buf.data_ptr() if want_x0 else None
             eps_u = plan.eps[B:].data_ptr() if self.guided else None
             noise_ptr, stride = (tr.noise_buf.data_ptr(), B * Cc * H * W) if noise is not None else (None, 0)
-            w = float(getattr(self, "w", 0.0))
+            w = None if per_image_w else float(getattr(self, "w", 0.0))
 
             def step():
                 plan.run()
                 s = _lib.stream_ptr()
-                _lib.check(L.its_ddpm_step_x0(plan.x_in.data_ptr(), x0_ptr, plan.eps.data_ptr(), eps_u, noise_ptr,
-                                              stride, B, Cc * H * W, coef.data_ptr(), x0tab, plan.t_dev.data_ptr(),
-                                              w, seed, tr.cand_dev.data_ptr(), tr.nan_flag.data_ptr(), int(clip), s),
-                           "its_ddpm_step_x0")
+                if per_image_w:
+                    _lib.check(L.its_ddpm_step_x0_w(plan.x_in.data_ptr(), x0_ptr, plan.eps.data_ptr(), eps_u,
+                                                    noise_ptr, stride, B, Cc * H * W, coef.data_ptr(), x0tab,
+                                                    plan.t_dev.data_ptr(), tr.w_img.data_ptr(), seed,
+                                                    tr.cand_dev.data_ptr(), tr.nan_flag.data_ptr(), int(clip), s),
+                               "its_ddpm_step_x0_w")
+                else:
+                    _lib.check(L.its_ddpm_step_x0(plan.x_in.data_ptr(), x0_ptr, plan.eps.data_ptr(), eps_u, noise_ptr,
+                                                  stride, B, Cc * H * W, coef.data_ptr(), x0tab, plan.t_dev.data_ptr(),
+                                                  w, seed, tr.cand_dev.data_ptr(), tr.nan_flag.data_ptr(), int(clip),
+                                                  s), "its_ddpm_step_x0")
                 _lib.check(L.its_step_advance(plan.t_dev.data_ptr(), -1, s), "its_step_advance")
 
             t_cur = first
@@ -203,13 +233,15 @@ class SamplerBase(nn.Module):
 
     def segment(self, x: torch.Tensor, labels: Optional[torch.Tensor] = None, *, t_start: int, t_stop: int,
                 seed: int, cand_id0: int = 0, noise: Optional[torch.Tensor] = None, x0: bool = False,
-                check_nan: bool = True) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
+                check_nan: bool = True, guidance=None) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
         """Steps time_step = t_start ... t_stop of the ancestral loop from state `x` (the x_t that step t_start
         takes), as `forward(x, t_start=..., t_stop=...)` computes them, bit for bit; the state after step 0 is
         clipped.  Returns (state after step t_stop, x0 prediction of step t_stop or None).  With `x0` the last
         step also yields clip(sqrt(1/abar)*x_t - sqrt(1/abar - 1)*eps, -1, 1) from that step's (guidance-mixed)
-        eps: no extra UNet evaluation.  `forward` and `segment` share the sampler's step graphs (`_run`)."""
+        eps: no extra UNet evaluation.  `forward` and `segment` share the sampler's step graphs (`_run`).
+        `guidance` (guided sampler only, else ValueError): a 1-D tensor or sequence of B finite weights, image i
+        mixed at guidance[i] instead of `self.w`; None keeps the scalar path."""
         if not (0 <= int(t_stop) <= int(t_start) < self.T):
             raise ValueError(f"segment needs 0 <= t_stop <= t_start < T={self.T}; got t_start={t_start} t_stop={t_stop}")
         return self._run(x, labels, t_start=int(t_start), t_stop=int(t_stop), seed=int(seed), cand_id0=int(cand_id0),
-                         noise=noise, clip=True, want_x0=bool(x0), check_nan=check_nan)
+                         noise=noise, clip=True, want_x0=bool(x0), check_nan=check_nan, guidance=guidance)

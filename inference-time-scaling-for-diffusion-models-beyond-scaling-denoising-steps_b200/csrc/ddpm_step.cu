@@ -56,13 +56,16 @@ __device__ __forceinline__ float clip1_keep_nan(float v) { return v != v ? v : f
 // kX0 = false: its_ddpm_step (the trailing three arguments are unused).  kX0 = true: its_ddpm_step_x0 — the
 // candidate base is read from *cand_dev and, when x0_out != NULL, the x0 prediction of the same mixed eps,
 // clip(r1[t]*x - r2[t]*eps, -1, 1) with {r1, r2} = x0_coef[t], is written to x0_out.
-template <bool kX0>
+// kWImg = true: its_ddpm_step_x0_w — image img of the launch mixes with the pair {w, 1 + w} = w_img[img] instead of
+// the scalar arguments w, opw.  w_img is the last parameter, so the other instantiations keep their parameter
+// offsets and machine code.
+template <bool kX0, bool kWImg = false>
 __global__ void __launch_bounds__(256) ddpm_step_kernel(
     float* __restrict__ x, const float* __restrict__ eps_c, const float* __restrict__ eps_u,
     const float* __restrict__ noise, long long noise_t_stride, long long n_img, long long quads_per_img,
     const float* __restrict__ coef, const int* __restrict__ t_dev, float w, float opw, uint64_t seed,
     long long cand_id0, int* __restrict__ nan_flag, int clip_last, float* __restrict__ x0_out,
-    const float* __restrict__ x0_coef, const long long* __restrict__ cand_dev) {
+    const float* __restrict__ x0_coef, const long long* __restrict__ cand_dev, const float* __restrict__ w_img) {
   pdl_prologue();
   const int t = *t_dev;
   const float4 cf = *reinterpret_cast<const float4*>(coef + 4 * (long long)t);
@@ -88,13 +91,19 @@ __global__ void __launch_bounds__(256) ddpm_step_kernel(
     float4 e = __ldg(reinterpret_cast<const float4*>(eps_c) + q);
     if (eps_u != nullptr) {
       float4 u = __ldg(reinterpret_cast<const float4*>(eps_u) + q);
+      float mw = w, mopw = opw;
+      if constexpr (kWImg) {   // 8 B per image: the pairs of a launch stay in L1
+        const float2 p = __ldg(reinterpret_cast<const float2*>(w_img) + img);
+        mw = p.x;
+        mopw = p.y;
+      }
       // (1 + w) * eps - w * nonEps: separately rounded mul, mul, sub like the
       // reference's three eager ops (no FMA contraction), so injected-noise runs
       // can match it bit for bit.
-      e.x = __fsub_rn(__fmul_rn(opw, e.x), __fmul_rn(w, u.x));
-      e.y = __fsub_rn(__fmul_rn(opw, e.y), __fmul_rn(w, u.y));
-      e.z = __fsub_rn(__fmul_rn(opw, e.z), __fmul_rn(w, u.z));
-      e.w = __fsub_rn(__fmul_rn(opw, e.w), __fmul_rn(w, u.w));
+      e.x = __fsub_rn(__fmul_rn(mopw, e.x), __fmul_rn(mw, u.x));
+      e.y = __fsub_rn(__fmul_rn(mopw, e.y), __fmul_rn(mw, u.y));
+      e.z = __fsub_rn(__fmul_rn(mopw, e.z), __fmul_rn(mw, u.z));
+      e.w = __fsub_rn(__fmul_rn(mopw, e.w), __fmul_rn(mw, u.w));
     }
     if constexpr (kX0) {
       if (x0_out != nullptr) {
@@ -233,7 +242,7 @@ extern "C" int its_ddpm_step(float* x, const float* eps_c, const float* eps_u, c
   ITS_LAUNCH(its::ddpm_step_kernel<false>, dim3(its::grid_for(n_img * quads, 256)), dim3(256), 0, its::as_stream(stream), 
       x, eps_c, eps_u, noise, noise_t_stride, n_img, quads, coef, t_dev, (float)w, (float)(1.0 + w), seed,
       cand_id0,
-      nan_flag, clip_last, (float*)nullptr, (const float*)nullptr, (const long long*)nullptr);
+      nan_flag, clip_last, (float*)nullptr, (const float*)nullptr, (const long long*)nullptr, (const float*)nullptr);
   ITS_CHECK_LAUNCH();
   return ITS_OK;
 }
@@ -250,7 +259,27 @@ extern "C" int its_ddpm_step_x0(float* x, float* x0_out, const float* eps_c, con
   const long long quads = n_per_img / 4;
   ITS_LAUNCH(its::ddpm_step_kernel<true>, dim3(its::grid_for(n_img * quads, 256)), dim3(256), 0,
       its::as_stream(stream), x, eps_c, eps_u, noise, noise_t_stride, n_img, quads, coef, t_dev, (float)w,
-      (float)(1.0 + w), seed, (long long)0, nan_flag, clip_last, x0_out, x0_coef, (const long long*)cand_dev);
+      (float)(1.0 + w), seed, (long long)0, nan_flag, clip_last, x0_out, x0_coef, (const long long*)cand_dev,
+      (const float*)nullptr);
+  ITS_CHECK_LAUNCH();
+  return ITS_OK;
+}
+
+extern "C" int its_ddpm_step_x0_w(float* x, float* x0_out, const float* eps_c, const float* eps_u, const float* noise,
+                                  int64_t noise_t_stride, int64_t n_img, int64_t n_per_img, const float* coef,
+                                  const float* x0_coef, const int32_t* t_dev, const float* w_img, uint64_t seed,
+                                  const int64_t* cand_dev, int32_t* nan_flag, int32_t clip_last, void* stream) {
+  ITS_REQUIRE(x && eps_c && eps_u && coef && t_dev && w_img && cand_dev && nan_flag,
+              "its_ddpm_step_x0_w: null pointer (eps_u and w_img are required)");
+  ITS_REQUIRE(x0_out == nullptr || x0_coef != nullptr, "its_ddpm_step_x0_w: null pointer (x0_coef with x0_out)");
+  ITS_REQUIRE(((uintptr_t)w_img & 7) == 0, "its_ddpm_step_x0_w: w_img must be 8-byte aligned ({w, 1 + w} pairs)");
+  ITS_REQUIRE(n_img > 0 && n_per_img > 0 && n_per_img % 4 == 0,
+              "its_ddpm_step_x0_w: n_per_img=%lld must be a positive multiple of 4", (long long)n_per_img);
+  ITS_REQUIRE(noise_t_stride % 4 == 0, "its_ddpm_step_x0_w: noise_t_stride must be a multiple of 4");
+  const long long quads = n_per_img / 4;
+  ITS_LAUNCH((its::ddpm_step_kernel<true, true>), dim3(its::grid_for(n_img * quads, 256)), dim3(256), 0,
+      its::as_stream(stream), x, eps_c, eps_u, noise, noise_t_stride, n_img, quads, coef, t_dev, 0.0f, 0.0f, seed,
+      (long long)0, nan_flag, clip_last, x0_out, x0_coef, (const long long*)cand_dev, w_img);
   ITS_CHECK_LAUNCH();
   return ITS_OK;
 }

@@ -300,7 +300,8 @@ def make_verifier(name: str, sampler=None, *, n_levels: int = 8, seed: int = 0, 
     return table[name]()
 
 
-def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Optional[int] = None):
+def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Optional[int] = None,
+               info: Optional[Dict[str, Any]] = None):
     """`search:` block of the config -> (best_noise, best_score, images of the best candidate).
     Keys: algorithm (random | zero_order | path | search_over_paths | fk_steering), verifier (oracle | self_supervised |
     aesthetic | denoising | diffusion_classifier | ensemble; denoising and diffusion_classifier score with the
@@ -317,35 +318,52 @@ def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Op
     `n_queries` (K, default 1) > 1 runs K independent random / search_over_paths / fk_steering searches as one
     population (`search_batch`): `labels` is then [K] or [K, B] (one row per query), and the results are stacked over the
     queries (best_noise and images [K, B, 3, H, W], a list of K scores).
+    `guidance_weights` [w_0, ..., w_{G-1}] (guided net; random, search_over_paths and fk_steering) searches over the
+    guidance weight too: candidate / path / particle i of every query runs at w_{i mod G} instead of the config's
+    `w`; the search's `last_guidance` holds the chosen weight(s), and random search's images are the winner's
+    trajectory at its weight.  A dict passed as `info` receives 'guidance': those chosen weight(s) (None without
+    `guidance_weights`).
     With torch.distributed initialised the candidates are sharded over the ranks."""
     from .search import search_algorithm as S
     sc = dict(config.get("search") or {})
     algo = sc.get("algorithm", "random")
     B, H = int(config.get("batch_size", 1)), int(config["img_size"])
     shape = (B, 3, H, H)
+    gw = _guidance_weights(sc, algo, sampler)
     ver = make_verifier(sc.get("verifier", "oracle"), sampler, n_levels=int(sc.get("score_levels", 8)),
                         seed=int(sc.get("score_seed", 0)), max_images=int(sc.get("max_images", 256)),
                         ensemble=sc.get("ensemble"), ensemble_weights=sc.get("ensemble_weights"))
     K = int(sc.get("n_queries", 1))
+    if info is not None:
+        info["guidance"] = None
     if K > 1:
-        return _run_batch(sampler, sc, algo, K, shape, ver, device, labels=labels, seed=seed)
+        *result, search = _run_batch(sampler, sc, algo, K, shape, ver, device, labels=labels, seed=seed, gw=gw)
+        if info is not None and gw is not None:
+            info["guidance"] = search.last_guidance
+        return tuple(result)
     den = S.make_denoise_fn(sampler, labels, max_images=int(sc.get("max_images", 256)), seed=seed)
     dev = str(device)
     if algo == "search_over_paths":
         search = S.SearchOverPaths(n_beams=int(sc.get("n_beams", 4)), n_children=int(sc.get("n_children", 4)),
                                    start_step=int(sc.get("start_step", 800)), delta_f=int(sc.get("delta_f", 50)),
                                    delta_b=int(sc.get("delta_b", 100)))
-        images, score, _ = search.search(shape, den, ver.score, device=dev, verbose=False, seed=seed)
+        images, score, _ = search.search(shape, den, ver.score, device=dev, verbose=False, seed=seed,
+                                         **_grid(gw, search.n_beams))
         best = S.philox_normal((1,) + shape, search.last_seed, search.last_index, S.TAG_X_T, torch.device(device))[0]
+        if info is not None and gw is not None:
+            info["guidance"] = search.last_guidance
         return best, score, images
     if algo == "fk_steering":
         search = _fk_steering(sc)
-        images, score, _ = search.search(shape, den, ver.score, device=dev, seed=seed)
+        images, score, _ = search.search(shape, den, ver.score, device=dev, seed=seed, **_grid(gw, search.n_particles))
         best = S.philox_normal((1,) + shape, search.last_seed, search.last_index, S.TAG_X_T, torch.device(device))[0]
+        if info is not None and gw is not None:
+            info["guidance"] = search.last_guidance
         return best, score, images
     if algo == "random":
         search = S.RandomSearch(n_candidates=int(sc.get("n_candidates", 4)))
-        best, score = search.search(shape, den, ver.score, device=dev, verbose=False, seed=seed)
+        best, score = search.search(shape, den, ver.score, device=dev, verbose=False, seed=seed,
+                                    **_grid(gw, search.n_candidates))
     else:
         x0 = S.philox_normal((1,) + shape, 0 if seed is None else seed, 0, S.TAG_X_T, torch.device(device))[0]
         if algo == "zero_order":
@@ -364,14 +382,43 @@ def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Op
     # so that the returned images are the ones that produced the returned score
     images = None
     if best is not None:
+        g = getattr(search, "last_guidance", None) if gw is not None else None
         images = den.denoise_candidates(best.unsqueeze(0), max(0, int(getattr(search, "last_index", 0))),
-                                        seed=getattr(search, "last_seed", seed))[0]
+                                        seed=getattr(search, "last_seed", seed),
+                                        cand_guidance=None if g is None else torch.tensor([g], dtype=torch.float64))[0]
+    if info is not None and gw is not None:
+        info["guidance"] = search.last_guidance
     return best, score, images
 
 
+def _guidance_weights(sc: Dict[str, Any], algo: str, sampler) -> Optional[List[float]]:
+    """`search.guidance_weights` as a list of finite floats, or None when absent; refused where it cannot apply."""
+    gw = sc.get("guidance_weights")
+    if gw is None:
+        return None
+    if not isinstance(gw, (list, tuple)) or not gw or not all(isinstance(v, (int, float)) and not isinstance(v, bool)
+                                                               for v in gw):
+        raise ValueError(f"search.guidance_weights must be a non-empty list of numbers, got {gw!r}")
+    if not all(math.isfinite(float(v)) for v in gw):
+        raise ValueError(f"search.guidance_weights must be finite, got {gw!r}")
+    supported = ("random", "search_over_paths", "fk_steering")
+    if algo not in supported:
+        raise ValueError(f"search.guidance_weights needs search.algorithm in {list(supported)}, got {algo!r}")
+    if not getattr(sampler, "guided", False):
+        raise ValueError("search.guidance_weights needs the guided net (num_labels and w in the config)")
+    return [float(v) for v in gw]
+
+
+def _grid(gw: Optional[List[float]], n: int) -> Dict[str, Any]:
+    """The `guidance` keyword of a search of n members: member i at gw[i % G]; nothing without weights."""
+    if gw is None:
+        return {}
+    return {"guidance": torch.tensor([gw[i % len(gw)] for i in range(int(n))], dtype=torch.float64)}
+
+
 def _run_batch(sampler, sc: Dict[str, Any], algo: str, K: int, shape, ver, device, *, labels=None,
-               seed: Optional[int] = None):
-    """run_search for n_queries = K > 1: one `search_batch` over K queries."""
+               seed: Optional[int] = None, gw: Optional[List[float]] = None):
+    """run_search for n_queries = K > 1: one `search_batch` over K queries; returns (best, scores, images, search)."""
     from .search import search_algorithm as S
     batched = ("random", "search_over_paths", "fk_steering")
     if algo not in batched:
@@ -382,26 +429,31 @@ def _run_batch(sampler, sc: Dict[str, Any], algo: str, K: int, shape, ver, devic
         search = S.SearchOverPaths(n_beams=int(sc.get("n_beams", 4)), n_children=int(sc.get("n_children", 4)),
                                    start_step=int(sc.get("start_step", 800)), delta_f=int(sc.get("delta_f", 50)),
                                    delta_b=int(sc.get("delta_b", 100)))
-        images, scores, _ = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev))
+        images, scores, _ = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev),
+                                                **_grid(gw, search.n_beams))
         best = torch.stack([S.philox_normal((1,) + shape, search.last_seed, q * search.n_beams + p, S.TAG_X_T, dev)[0]
                             for q, p in enumerate(search.last_index)])
-        return best, scores, images
+        return best, scores, images, search
     if algo == "fk_steering":
         search = _fk_steering(sc)
-        images, scores, _ = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev))
+        images, scores, _ = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev),
+                                                **_grid(gw, search.n_particles))
         best = torch.stack([S.philox_normal((1,) + shape, search.last_seed, q * search.n_particles + p, S.TAG_X_T,
                                             dev)[0] for q, p in enumerate(search.last_index)])
-        return best, scores, images
+        return best, scores, images, search
     search = S.RandomSearch(n_candidates=int(sc.get("n_candidates", 4)))
-    best, scores = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev))
-    # each winner's images from its own trajectory (the global candidate id it was scored under)
+    best, scores = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev),
+                                       **_grid(gw, search.n_candidates))
+    # each winner's images from its own trajectory (the global candidate id and weight it was scored under)
     images = torch.full_like(best, float("nan"))
     rows = None if labels is None else labels.to(dev, torch.int64).reshape(K, -1).expand(K, shape[0])
     for q, i in enumerate(search.last_index):
         if i >= 0:
+            g = None if gw is None else torch.tensor([search.last_guidance[q]], dtype=torch.float64)
             images[q] = den.denoise_candidates(best[q:q + 1], q * search.n_candidates + i, seed=search.last_seed,
-                                               cand_labels=None if rows is None else rows[q:q + 1])[0]
-    return best, scores, images
+                                               cand_labels=None if rows is None else rows[q:q + 1],
+                                               cand_guidance=g)[0]
+    return best, scores, images, search
 
 
 def _fk_steering(sc: Dict[str, Any]):
@@ -443,12 +495,18 @@ def main(argv: Optional[List[str]] = None) -> int:
         labels = (1 + torch.arange(K * B, device=device) % int(cfg["num_labels"])).to(torch.int64)
         labels = labels.view(K, B) if K > 1 else labels
     if cfg.get("search"):
-        best, score, images = run_search(sampler, cfg, device, labels=labels, seed=cfg.get("seed"))
+        info: Dict[str, Any] = {}
+        best, score, images = run_search(sampler, cfg, device, labels=labels, seed=cfg.get("seed"), info=info)
+        chosen = info["guidance"]
         if K > 1:
             print("search: best scores " + " ".join(f"{v:.6f}" for v in score))
+            if chosen is not None:
+                print("search: chosen guidance weights " + " ".join("-" if v is None else f"{v:g}" for v in chosen))
             images = images.reshape(-1, *images.shape[2:])       # the grid holds all K*B winning images
         else:
             print(f"search: best score {score:.6f}")
+            if chosen is not None:
+                print(f"search: chosen guidance weight {chosen:g}")
     else:
         B, H = int(cfg.get("batch_size", 1)), int(cfg["img_size"])
         x_T = torch.randn(B, 3, H, H, device=device)

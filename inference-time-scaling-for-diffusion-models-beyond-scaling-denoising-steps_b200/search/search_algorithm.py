@@ -32,6 +32,12 @@ independent queries, each with its own labels, as one candidate population and s
 FKSteering is not in the reference either: Feynman-Kac steering of Singhal et al. (a population of particles
 resampled by verifier potentials on their x0 predictions), in population mode only.
 
+Search over the guidance weight (guided sampler, population mode): RandomSearch, SearchOverPaths and FKSteering take
+`guidance` ([N], or [K, N] in `search_batch`), one classifier-free-guidance weight per candidate, path or particle,
+which the sampler's step mixes per image (its_ddpm_step_x0_w).  A child of search over paths inherits its parent's
+weight and an FK particle its ancestor's, so selection and resampling choose the weight together with the noise.
+Every search then sets `last_guidance`, the winner's weight (a list over the queries in `search_batch`).
+
 A rank ensemble (`verifier.EnsembleVerifier`) scores relative to a population: RandomSearch, PathSearch and
 SearchOverPaths gather its [n, V] member scores and combine them per query right after the gather, on every rank,
 with the segments the selection uses.  ZeroOrderSearch and FKSteering compare scores across populations and refuse
@@ -108,6 +114,16 @@ class SamplerDenoiser:
             return None
         return lab.reshape(-1).repeat(n_cand)
 
+    def _check_cand_guidance(self, cand_guidance, n: int):
+        if cand_guidance is None:
+            return None
+        if not getattr(self.sampler, "guided", False):
+            raise ValueError("cand_guidance needs the guided sampler: an unguided one has no weight to vary")
+        if tuple(cand_guidance.shape) != (n,):
+            raise ValueError(f"cand_guidance must be [{n}] (one weight per candidate), got "
+                             f"{list(cand_guidance.shape)}")
+        return cand_guidance
+
     def __call__(self, noise: torch.Tensor, show_progress: bool = False, **kwargs) -> torch.Tensor:
         # the reference draws fresh step noise for every candidate (Diffusion.py:96): candidate i of a serial
         # search uses Philox stream i, exactly the stream population mode gives global candidate i
@@ -117,28 +133,32 @@ class SamplerDenoiser:
 
     def denoise_candidates(self, cands: torch.Tensor, first_cand: int, *, labels=None,
                            t_start: Optional[int] = None, seed: Optional[int] = None, t_stop: int = 0,
-                           cand_labels: Optional[torch.Tensor] = None) -> torch.Tensor:
+                           cand_labels: Optional[torch.Tensor] = None,
+                           cand_guidance: Optional[torch.Tensor] = None) -> torch.Tensor:
         """cands [n, B, C, H, W] -> images [n, B, C, H, W]; candidate i is global
         candidate first_cand + i (its Philox streams are keyed by that id).  `t_start` (default T-1) and `t_stop`
         bound the loop as the sampler's own arguments do (a `t_stop` > 0 returns the states step t_stop - 1
         starts from)."""
         t_start = self.sampler.T - 1 if t_start is None else t_start
         return self.denoise_segment(cands, first_cand, t_start=t_start, t_stop=t_stop, labels=labels, seed=seed,
-                                    x0=False, cand_labels=cand_labels)[0]
+                                    x0=False, cand_labels=cand_labels, cand_guidance=cand_guidance)[0]
 
     def denoise_segment(self, states: torch.Tensor, first_cand: int, *, t_start: int, t_stop: int,
                         cand_offset: int = 0, labels=None, seed: Optional[int] = None,
-                        x0: bool = True, cand_labels: Optional[torch.Tensor] = None
+                        x0: bool = True, cand_labels: Optional[torch.Tensor] = None,
+                        cand_guidance: Optional[torch.Tensor] = None
                         ) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
         """states [n, B, C, H, W] at step t_start -> (states after step t_stop, x0 predictions of step t_stop or
         None), in chunks of `max_images`.  Candidate i's per-step Philox streams are keyed by
         cand_offset + (first_cand + i) * B + image; every chunk replays the sampler's one step graph.  The guided
         sampler's labels are `cand_labels` [n, B] (int64, one row per candidate) when given, else `labels` (or the
-        denoiser's own) [B] for every candidate."""
+        denoiser's own) [B] for every candidate.  `cand_guidance` [n] (guided sampler): candidate i's guidance weight
+        for all its B images, instead of the sampler's `w`."""
         n, B = states.shape[:2]
         if cand_labels is not None and tuple(cand_labels.shape) != (n, B):
             raise ValueError(f"cand_labels must be [{n}, {B}] (one label row per candidate), got "
                              f"{tuple(cand_labels.shape)}")
+        cand_guidance = self._check_cand_guidance(cand_guidance, n)
         per_call = max(1, self.max_images // B)
         out = torch.empty_like(states)
         out_x0 = torch.empty_like(states) if x0 else None
@@ -150,6 +170,8 @@ class SamplerDenoiser:
                                       cand_id0=cand_offset + (first_cand + i0) * B, x0=x0)
             if self.step_noise is not None:
                 kw["noise"] = self.step_noise.repeat(1, i1 - i0, 1, 1, 1)
+            if cand_guidance is not None:
+                kw["guidance"] = cand_guidance[i0:i1].repeat_interleave(B)
             lab = self.image_labels(i1 - i0, labels, None if cand_labels is None else cand_labels[i0:i1])
             y, p = self.sampler.segment(x, lab, **kw)
             out[i0:i1] = y.view(i1 - i0, B, *states.shape[2:])
@@ -352,15 +374,17 @@ def _refuse_ranks(verifier_fn, search: str, why: str) -> None:
 
 
 def _score_population(cands_local: torch.Tensor, lo: int, n_total: int, denoise: SamplerDenoiser, ver,
-                      kwargs, t_start=None, seed=None, cand_labels=None, n_seg: int = 1) -> torch.Tensor:
+                      kwargs, t_start=None, seed=None, cand_labels=None, n_seg: int = 1,
+                      cand_guidance=None) -> torch.Tensor:
     """Denoise + score this rank's block of candidates, return ALL n_total scores.  `seed`: the search's
     shared seed, used for the step noise when the denoiser has none of its own (same on every rank).
     `cand_labels`: label rows of this rank's candidates ([n_local, B]), else kwargs' `labels` for all.
+    `cand_guidance`: guidance weights of this rank's candidates ([n_local]), else the sampler's `w`.
     A rank ensemble's member scores are combined over `n_seg` equal segments of the population."""
     B = cands_local.shape[1] if cands_local.numel() else 1
     if cands_local.shape[0] > 0:
         imgs = denoise.denoise_candidates(cands_local, lo, labels=kwargs.get("labels"), t_start=t_start, seed=seed,
-                                          cand_labels=cand_labels)
+                                          cand_labels=cand_labels, cand_guidance=cand_guidance)
         local = _score_candidates(ver, imgs.reshape(-1, *imgs.shape[2:]), B, denoise, kwargs.get("labels"),
                                   cand_labels)
     else:
@@ -393,6 +417,41 @@ def _label_rows(labels: Optional[torch.Tensor], K: int, per_query: int, B: int, 
     return lab.reshape(K * per_query, B)
 
 
+def _guidance(guidance, K: int, N: int, denoise_fn, search: str, device, batch: bool) -> Optional[torch.Tensor]:
+    """Per-member guidance weights, query-major float64 [K * N] on `device`, from `guidance` [N] (every query) or,
+    in `search_batch`, [K, N]; None stays None.  Checked on the host before any device work: population mode, the
+    guided sampler, the shape and finite values."""
+    if guidance is None:
+        return None
+    if not isinstance(denoise_fn, SamplerDenoiser):
+        raise ValueError(f"{search}: guidance weights need an its_b200 SamplerDenoiser and a kernel verifier's "
+                         ".score (population mode)")
+    if not getattr(denoise_fn.sampler, "guided", False):
+        raise ValueError(f"{search}: guidance weights need the guided sampler (DiffusionFreeGuidence)")
+    g = torch.as_tensor(guidance, dtype=torch.float64).detach().cpu()
+    shapes = [(N,), (K, N)] if batch else [(N,)]
+    if tuple(g.shape) not in shapes:
+        raise ValueError(f"{search}: guidance must be " + " or ".join(str(list(x)) for x in shapes) +
+                         f" (one weight per member), got {list(g.shape)}")
+    if not bool(torch.isfinite(g).all()):
+        raise ValueError(f"{search}: guidance weights must be finite")
+    return g.reshape(-1, N).expand(K, N).reshape(K * N).to(device)
+
+
+def _refuse_guidance(kwargs, search: str) -> None:
+    if kwargs.pop("guidance", None) is not None:
+        raise ValueError(f"{search} does not search over the guidance weight; use RandomSearch, SearchOverPaths or "
+                         "FKSteering")
+
+
+def _winner_guidance(g: Optional[torch.Tensor], ids: List[int]) -> Optional[List[Optional[float]]]:
+    """Weights of the winners (flat population ids, -1 for none) as host floats; None without guidance."""
+    if g is None:
+        return None
+    host = g.tolist()
+    return [host[i] if i >= 0 else None for i in ids]
+
+
 def _rows(rows: Optional[torch.Tensor], lo: int, hi: int) -> Optional[torch.Tensor]:
     return None if rows is None else rows[lo:hi]
 
@@ -414,8 +473,14 @@ class RandomSearch:
                device: str = 'cuda', verbose: bool = True, **kwargs) -> Tuple[torch.Tensor, float]:
         cand_noise = kwargs.pop("candidate_noise", None)   # [n, *noise_shape]: injected candidates
         seed = kwargs.pop("seed", None)
+        guidance = kwargs.pop("guidance", None)            # [n] per-candidate guidance weights
         ver = _population_mode(denoise_fn, verifier_fn)
         n = self.n_candidates
+        if guidance is not None and ver is None:
+            raise ValueError("RandomSearch: guidance weights need an its_b200 SamplerDenoiser and a kernel verifier's "
+                             ".score (population mode)")
+        guidance = _guidance(guidance, 1, n, denoise_fn, "RandomSearch", device, batch=False)
+        self.last_guidance = None
         if isinstance(denoise_fn, SamplerDenoiser):
             denoise_fn.reset_calls()
         if ver is None:
@@ -430,8 +495,10 @@ class RandomSearch:
                     best_score, best_noise = score, noise.clone()
             return best_noise, best_score
         best, vals, ids = self._population(noise_shape, denoise_fn, ver, 1, cand_noise=cand_noise, cand_labels=None,
-                                           seed=seed, device=device, kwargs=kwargs)
+                                           seed=seed, device=device, kwargs=kwargs, guidance=guidance)
         self.last_scores = self.last_scores[0]
+        if guidance is not None:
+            self.last_guidance = self.last_guidance[0]
         if ids[0] < 0:
             return None, float('-inf')
         self.last_index = ids[0]
@@ -440,7 +507,7 @@ class RandomSearch:
     def search_batch(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
                      n_queries: int, *, labels: Optional[torch.Tensor] = None,
                      candidate_noise: Optional[torch.Tensor] = None, seed: Optional[int] = None,
-                     device: str = 'cuda') -> Tuple[torch.Tensor, List[float]]:
+                     device: str = 'cuda', guidance=None) -> Tuple[torch.Tensor, List[float]]:
         """K = `n_queries` independent random searches of `n_candidates` (N) each, evaluated as one population of
         K*N candidates, with one winner per query selected on the device.  Population mode only.
 
@@ -448,8 +515,10 @@ class RandomSearch:
         `candidate_noise` [K, N, *noise_shape]: injected candidates.  Query q's candidate i is global candidate
         q*N + i (its x_T draw under TAG_X_T and its step noise are keyed by that id), so an unguided batch of K
         searches draws and scores exactly the population of RandomSearch(K*N).search with the same seed.
+        `guidance` [N] or [K, N] (guided sampler): candidate i of query q runs at weight guidance[q, i] (or [i]).
         Returns (best_noise [K, *noise_shape], best_scores); sets `last_scores` [K, N] (device), `last_index`
-        (within-query indices) and `last_seed`.  A query with no rankable score gets a NaN row, -inf and -1."""
+        (within-query indices), `last_guidance` (the winners' weights, None without `guidance`) and `last_seed`.
+        A query with no rankable score gets a NaN row, -inf and -1 (and weight None)."""
         K = _check_queries(n_queries, noise_shape, labels)
         ver = _population_mode(denoise_fn, verifier_fn)
         if ver is None:
@@ -457,19 +526,20 @@ class RandomSearch:
                              "(population mode)")
         N = self.n_candidates
         _check_shape("candidate_noise", candidate_noise, (K, N, *noise_shape))
+        guidance = _guidance(guidance, K, N, denoise_fn, "RandomSearch", device, batch=True)
         denoise_fn.reset_calls()
         cand = None if candidate_noise is None else candidate_noise.reshape(K * N, *noise_shape)
         best, vals, ids = self._population(noise_shape, denoise_fn, ver, K, cand_noise=cand,
                                            cand_labels=_label_rows(labels, K, N, noise_shape[0], device),
-                                           seed=seed, device=device, kwargs={})
+                                           seed=seed, device=device, kwargs={}, guidance=guidance)
         self.last_index = ids
         return best, vals
 
     def _population(self, noise_shape, denoise_fn: SamplerDenoiser, ver, K: int, *, cand_noise, cand_labels, seed,
-                    device, kwargs) -> Tuple[torch.Tensor, List[float], List[int]]:
+                    device, kwargs, guidance=None) -> Tuple[torch.Tensor, List[float], List[int]]:
         """K queries of N candidates as one population sharded over the ranks; query q's candidate i is global
-        candidate q*N + i.  One segmented top-k (k = 1 per query) selects every winner.  Sets `last_seed` and
-        `last_scores` [K, N]; returns (winners [K, *noise_shape], scores, within-query indices), a NaN row, -inf
+        candidate q*N + i, at weight guidance[q*N + i] when given.  One segmented top-k (k = 1 per query) selects
+        every winner.  Sets `last_seed`, `last_guidance` and `last_scores` [K, N]; returns (winners [K, *noise_shape], scores, within-query indices), a NaN row, -inf
         and -1 for a query with no rankable score."""
         dist, rank, world = _dist()
         dev = torch.device(device)
@@ -485,11 +555,13 @@ class RandomSearch:
                 if hi > lo else torch.empty((0, *noise_shape), device=dev)
         with torch.no_grad():
             scores = _score_population(local, lo, n, denoise_fn, ver, kwargs, seed=seed,
-                                       cand_labels=_rows(cand_labels, lo, hi), n_seg=K)
+                                       cand_labels=_rows(cand_labels, lo, hi), n_seg=K,
+                                       cand_guidance=_rows(guidance, lo, hi))
         self.nfes += n
         self.last_scores = scores.view(K, N)
         idx, val = _topk_device(scores, 1, n_seg=K)
         ids, vals = idx.tolist(), val.tolist()
+        self.last_guidance = _winner_guidance(guidance, ids)
         best = torch.full((K, *noise_shape), float('nan'), dtype=torch.float32, device=dev)
         for q, i in enumerate(ids):
             if i < 0:
@@ -525,6 +597,7 @@ class ZeroOrderSearch:
                **kwargs) -> Tuple[torch.Tensor, float, Dict[str, Any]]:
         _refuse_ranks(verifier_fn, "ZeroOrderSearch", "it compares each round's best with the best of earlier "
                       "rounds")
+        _refuse_guidance(kwargs, "ZeroOrderSearch")
         perts = kwargs.pop("perturbations", None)    # [iters][K, *shape] injected N(0,1) draws
         seed = kwargs.pop("seed", None)
         ver = _population_mode(denoise_fn, verifier_fn)
@@ -610,6 +683,7 @@ class PathSearch:
     def search(self, initial_noise: torch.Tensor, denoise_fn: Callable, verifier_fn: Callable,
                timesteps: int = 1000, device: str = 'cuda', verbose: Optional[bool] = None,
                **kwargs) -> Tuple[torch.Tensor, float, Dict[str, Any]]:
+        _refuse_guidance(kwargs, "PathSearch")
         variations = kwargs.pop("variations", None)   # [n_paths, *shape] injected N(0,1) draws
         seed = kwargs.pop("seed", None)
         restart = bool(kwargs.pop("restart", False))
@@ -715,7 +789,10 @@ class SearchOverPaths:
 
     `search(noise_shape, denoise_fn, verifier_fn, ...)` returns (best_images [B,C,H,W], best_score, history);
     keyword extensions: `seed`, `labels`, `candidate_noise`, `forward_noise` ([rounds][N*M, *noise_shape]
-    injected re-noising draws).  `last_index` is the winner's initial path id, `last_seed` the search seed.
+    injected re-noising draws), `guidance` ([N] guidance weights of the initial paths, guided sampler: a child
+    runs at its parent's weight; history 'lineage_guidance' holds the winner's weight in every round and
+    `last_guidance` the winner's weight).  `last_index` is the winner's initial path id, `last_seed` the search
+    seed.
     `nfes` counts UNet steps x candidates (the reference's classes count denoise_fn calls).  `search_batch` runs
     K such searches, with their own labels, as one population."""
 
@@ -735,21 +812,26 @@ class SearchOverPaths:
         cand_noise = kwargs.pop("candidate_noise", None)
         fwd_noise = kwargs.pop("forward_noise", None)
         seed = kwargs.pop("seed", None)
+        guidance = kwargs.pop("guidance", None)
         ver, rounds = self._schedule(denoise_fn, verifier_fn)
+        guidance = _guidance(guidance, 1, int(self.n_beams), denoise_fn, "SearchOverPaths", device, batch=False)
         if fwd_noise is not None and len(fwd_noise) < len(rounds):
             raise ValueError(f"forward_noise has {len(fwd_noise)} rounds, the schedule {len(rounds)}")
         images, best, h = self._population(tuple(noise_shape), denoise_fn, ver, rounds, 1, labels=kwargs.get("labels"),
                                            query_labels=None, cand_noise=cand_noise, fwd_noise=fwd_noise, seed=seed,
-                                           device=device)
+                                           device=device, guidance=guidance)
         history = {'rounds': h['rounds'], 'scores': h['scores'][0], 'survivors': h['survivors'][0],
                    'lineage': h['lineage'][0], 'unet_image_steps': h['unet_image_steps']}
+        if guidance is not None:
+            history['lineage_guidance'] = h['lineage_guidance'][0]
+            self.last_guidance = self.last_guidance[0]
         self.last_index = history['lineage']['path']
         return images[0], best[0], history
 
     def search_batch(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
                      n_queries: int, *, labels: Optional[torch.Tensor] = None,
                      candidate_noise: Optional[torch.Tensor] = None, forward_noise=None, seed: Optional[int] = None,
-                     device: str = 'cuda') -> Tuple[torch.Tensor, List[float], Dict[str, Any]]:
+                     device: str = 'cuda', guidance=None) -> Tuple[torch.Tensor, List[float], Dict[str, Any]]:
         """K = `n_queries` independent searches over paths evaluated as one population: K*N paths in stage 0 and
         K*N*M children per round, with the N survivors (and at the end the winner) of every query selected on the
         device by one segmented top-k.  Population mode only.
@@ -759,15 +841,19 @@ class SearchOverPaths:
         Query q's path i is global path q*N + i and its child c global child q*N*M + c; x_T, step noise and
         re-noising draws are keyed by those ids, so K = 1 is `search` and a query's result does not depend on
         the other queries, the rank count or `max_images`.
+        `guidance` [N] or [K, N] (guided sampler): path i of query q starts at weight guidance[q, i] (or [i]); its
+        children, and theirs, keep it.
         Returns (best_images [K, *noise_shape], best_scores, history): history 'rounds' as in `search`; 'scores',
-        'survivors' and 'lineage' are lists over the queries, with within-query ids; 'unet_image_steps' is the
-        whole batch's.  `last_index` is the list of the winners' initial path ids.  A query whose children cannot
-        be ranked raises ValueError naming the query and the round."""
+        'survivors' and 'lineage' (and with `guidance` 'lineage_guidance') are lists over the queries, with
+        within-query ids; 'unet_image_steps' is the whole batch's.  `last_index` is the list of the winners' initial
+        path ids, `last_guidance` of their weights.  A query whose children cannot be ranked raises ValueError naming
+        the query and the round."""
         K = _check_queries(n_queries, noise_shape, labels)
         ver, rounds = self._schedule(denoise_fn, verifier_fn)
         shape = tuple(noise_shape)
         N, NM = int(self.n_beams), int(self.n_beams) * int(self.n_children)
         _check_shape("candidate_noise", candidate_noise, (K, N) + shape)
+        guidance = _guidance(guidance, K, N, denoise_fn, "SearchOverPaths", device, batch=True)
         fwd = None
         if forward_noise is not None:
             if len(forward_noise) < len(rounds):
@@ -778,7 +864,7 @@ class SearchOverPaths:
         images, best, history = self._population(
             shape, denoise_fn, ver, rounds, K, labels=None, query_labels=labels,
             cand_noise=None if candidate_noise is None else candidate_noise.reshape((K * N,) + shape),
-            fwd_noise=fwd, seed=seed, device=device)
+            fwd_noise=fwd, seed=seed, device=device, guidance=guidance)
         self.last_index = [lin['path'] for lin in history['lineage']]
         return images, best, history
 
@@ -794,10 +880,12 @@ class SearchOverPaths:
         return ver, path_rounds(denoise_fn.sampler.T, self.start_step, self.delta_f, self.delta_b)
 
     def _population(self, shape: Tuple[int, ...], denoise_fn: SamplerDenoiser, ver, rounds, K: int, *, labels,
-                    query_labels, cand_noise, fwd_noise, seed, device):
+                    query_labels, cand_noise, fwd_noise, seed, device, guidance=None):
         """K queries as one population sharded over the ranks (query q's path i is global path q*N + i, its child c
         global child q*N*M + c).  `labels`: shared labels of every member; `query_labels` ([K] or [K, B]): one
-        label row per query.  Returns (best images [K, *shape], best scores, history with per-query 'scores',
+        label row per query; `guidance` ([K*N] or None): the initial paths' weights, which every child inherits
+        from its parent (re-indexed by the same device survivor ids the expansion reads).  Sets `last_guidance`.
+        Returns (best images [K, *shape], best scores, history with per-query 'scores',
         'survivors' and 'lineage' in within-query ids)."""
         N, M = int(self.n_beams), int(self.n_children)
         NM = N * M
@@ -813,6 +901,8 @@ class SearchOverPaths:
         path_labels, child_labels = _label_rows(query_labels, K, N, B, dev), _label_rows(query_labels, K, NM, B, dev)
         history: Dict[str, Any] = {'rounds': [], 'scores': [[] for _ in range(K)],
                                    'survivors': [[] for _ in range(K)]}
+        self.last_guidance = None
+        g_rows, g_rounds = guidance, []               # weight of each row of `parents`; children's weights per round
         steps = 0                                     # UNet steps x candidates
         with torch.no_grad():
             # stage 0: K*N paths from x_T down to the states at step start_step
@@ -827,7 +917,8 @@ class SearchOverPaths:
             s0 = rounds[0][0]
             if s0 < T - 1 and hi > lo:
                 local = denoise_fn.denoise_candidates(local, lo, labels=labels, seed=seed, t_stop=s0 + 1,
-                                                      cand_labels=_rows(path_labels, lo, hi))
+                                                      cand_labels=_rows(path_labels, lo, hi),
+                                                      cand_guidance=_rows(g_rows, lo, hi))
             steps += n_p * (T - 1 - s0)
             parents = _gather_states(local.contiguous(), n_p)
             parent_idx = torch.arange(n_p, dtype=torch.int32, device=dev)
@@ -836,6 +927,9 @@ class SearchOverPaths:
             for r, (s, sp, e) in enumerate(rounds):
                 ratio = float(abar[sp] / abar[s])
                 a, b = math.sqrt(ratio), math.sqrt(1. - ratio)
+                if g_rows is not None:                # child c runs at the weight of its parent parent_idx[c // M]
+                    g_rows = g_rows.index_select(0, parent_idx.long()).repeat_interleave(M)
+                    g_rounds.append(g_rows.tolist())
                 if hi > lo:
                     z = None if fwd_noise is None else fwd_noise[r][lo:hi]
                     kids = path_expand(parents.reshape(parents.shape[0], -1), parent_idx, M, lo, hi - lo, a, b,
@@ -843,7 +937,8 @@ class SearchOverPaths:
                                        cand_id0=(r + 1) * ROUND_STRIDE, tag=TAG_FORWARD).view((hi - lo,) + shape)
                     states, x0 = denoise_fn.denoise_segment(kids, lo, t_start=sp, t_stop=e, labels=labels, seed=seed,
                                                             cand_offset=(r + 1) * ROUND_STRIDE, x0=True,
-                                                            cand_labels=_rows(child_labels, lo, hi))
+                                                            cand_labels=_rows(child_labels, lo, hi),
+                                                            cand_guidance=_rows(g_rows, lo, hi))
                     judged = x0 if e > 0 else states   # the last round scores the finished, clipped samples
                     local_scores = _score_candidates(ver, judged.reshape(-1, *shape[1:]), B, denoise_fn, labels,
                                                      _rows(child_labels, lo, hi))
@@ -880,6 +975,10 @@ class SearchOverPaths:
                 lineage.append(child)
             lineage.reverse()
             history['lineage'].append({'path': lineage[0] // M, 'children': lineage})
+        if guidance is not None:
+            history['lineage_guidance'] = [[g_rounds[r][q * NM + c] for r, c in enumerate(lin['children'])]
+                                           for q, lin in enumerate(history['lineage'])]
+            self.last_guidance = [lg[-1] for lg in history['lineage_guidance']]
         history['unet_image_steps'] = steps * B * (2 if getattr(smp, "guided", False) else 1)
         self.nfes += steps
         return parents[parent_idx.long()].clone(), best.tolist(), history
@@ -925,9 +1024,11 @@ class FKSteering:
     states, and every rank draws the same ancestors.
 
     `search(noise_shape, denoise_fn, verifier_fn, ...)` returns (best_images [B,C,H,W], best_score, history);
-    keyword extensions: `seed`, `labels`, `candidate_noise`.  history: 'segments'; per resampling 'scores' (N),
-    'ancestors' (N particle ids) and 'ess'; 'lineage', the winner's particle id in every segment (lineage[0] is its
-    x_T id); 'unet_image_steps'.  `last_index` is the winner's x_T id, `last_seed` the search seed; `nfes` counts
+    keyword extensions: `seed`, `labels`, `candidate_noise`, `guidance` ([N] guidance weights of the particles,
+    guided sampler: a particle keeps its ancestor's weight at every resampling).  history: 'segments'; per
+    resampling 'scores' (N), 'ancestors' (N particle ids) and 'ess'; 'lineage', the winner's particle id in every
+    segment (lineage[0] is its x_T id); with `guidance` 'lineage_guidance', its weight in every segment (and
+    `last_guidance` the winner's weight); 'unet_image_steps'.  `last_index` is the winner's x_T id, `last_seed` the search seed; `nfes` counts
     UNet steps x particles (N * T per search).  `search_batch` runs K such searches, with their own labels, as one
     population."""
 
@@ -943,20 +1044,26 @@ class FKSteering:
                **kwargs) -> Tuple[torch.Tensor, float, Dict[str, Any]]:
         cand_noise = kwargs.pop("candidate_noise", None)
         seed = kwargs.pop("seed", None)
+        guidance = kwargs.pop("guidance", None)
         shape = tuple(noise_shape)
         ver, segments = self._schedule(denoise_fn, verifier_fn)
         _check_shape("candidate_noise", cand_noise, (int(self.n_particles),) + shape)
+        guidance = _guidance(guidance, 1, int(self.n_particles), denoise_fn, "FKSteering", device, batch=False)
         images, best, h = self._population(shape, denoise_fn, ver, segments, 1, labels=kwargs.get("labels"),
-                                           query_labels=None, cand_noise=cand_noise, seed=seed, device=device)
+                                           query_labels=None, cand_noise=cand_noise, seed=seed, device=device,
+                                           guidance=guidance)
         history = {'segments': h['segments'], 'scores': h['scores'][0], 'ancestors': h['ancestors'][0],
                    'ess': h['ess'][0], 'lineage': h['lineage'][0], 'unet_image_steps': h['unet_image_steps']}
+        if guidance is not None:
+            history['lineage_guidance'] = h['lineage_guidance'][0]
+            self.last_guidance = self.last_guidance[0]
         self.last_index = history['lineage'][0]
         return images[0], best[0], history
 
     def search_batch(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
                      n_queries: int, *, labels: Optional[torch.Tensor] = None,
                      candidate_noise: Optional[torch.Tensor] = None, seed: Optional[int] = None,
-                     device: str = 'cuda') -> Tuple[torch.Tensor, List[float], Dict[str, Any]]:
+                     device: str = 'cuda', guidance=None) -> Tuple[torch.Tensor, List[float], Dict[str, Any]]:
         """K = `n_queries` independent FK-steering searches evaluated as one population of K*N particles, resampled
         per query by one segmented kernel launch, with every query's winner selected on the device by one segmented
         top-k.  Population mode only.
@@ -966,19 +1073,23 @@ class FKSteering:
         (its x_T draw and step noise are keyed by that id, its resampling uniform by q, ancestors never cross
         queries), so K = 1 is `search`, query 0 is the single search with query 0's inputs, and a query's result
         does not depend on the other queries' inputs, the rank count or `max_images`.
+        `guidance` [N] or [K, N] (guided sampler): particle j of query q starts at weight guidance[q, j] (or [j]) and
+        every resampling hands a particle its ancestor's weight.
         Returns (best_images [K, *noise_shape], best_scores, history): 'segments' as in `search`; 'scores',
-        'ancestors', 'ess' and 'lineage' are lists over the queries, with within-query ids; 'unet_image_steps' is
-        the whole batch's.  `last_index` is the list of the winners' x_T ids.  A query none of whose particles can
+        'ancestors', 'ess' and 'lineage' (and with `guidance` 'lineage_guidance') are lists over the queries, with
+        within-query ids; 'unet_image_steps' is the whole batch's.  `last_index` is the list of the winners' x_T ids,
+        `last_guidance` of their weights.  A query none of whose particles can
         be weighted raises ValueError naming the query and the resampling round."""
         K = _check_queries(n_queries, noise_shape, labels)
         shape = tuple(noise_shape)
         ver, segments = self._schedule(denoise_fn, verifier_fn)
         N = int(self.n_particles)
         _check_shape("candidate_noise", candidate_noise, (K, N) + shape)
+        guidance = _guidance(guidance, K, N, denoise_fn, "FKSteering", device, batch=True)
         images, best, history = self._population(
             shape, denoise_fn, ver, segments, K, labels=None, query_labels=labels,
             cand_noise=None if candidate_noise is None else candidate_noise.reshape((K * N,) + shape),
-            seed=seed, device=device)
+            seed=seed, device=device, guidance=guidance)
         self.last_index = [lin[0] for lin in history['lineage']]
         return images, best, history
 
@@ -997,10 +1108,11 @@ class FKSteering:
         return ver, fk_segments(denoise_fn.sampler.T, self.start_step, self.resample_interval)
 
     def _population(self, shape: Tuple[int, ...], denoise_fn: SamplerDenoiser, ver, segments, K: int, *, labels,
-                    query_labels, cand_noise, seed, device):
+                    query_labels, cand_noise, seed, device, guidance=None):
         """K queries of N particles as one population sharded over the ranks (query q's particle j is global
         particle q*N + j).  `labels`: shared labels of every particle; `query_labels` ([K] or [K, B]): one label row
-        per query.  Returns (best images [K, *shape], best scores, history with per-query 'scores', 'ancestors',
+        per query; `guidance` ([K*N] or None): the particles' weights, which follow their ancestors (`index_select`
+        with the same device ancestor ids as the states).  Sets `last_guidance`.  Returns (best images [K, *shape], best scores, history with per-query 'scores', 'ancestors',
         'ess' and 'lineage' in within-query ids)."""
         N = int(self.n_particles)
         n = K * N
@@ -1017,6 +1129,8 @@ class FKSteering:
                                    'ancestors': [[] for _ in range(K)], 'ess': [[] for _ in range(K)]}
         steps = 0                                     # UNet steps x particles
         carried = None
+        g, g_segments = guidance, []                  # particle weights now, and in every segment
+        self.last_guidance = None
         with torch.no_grad():
             if cand_noise is not None:
                 local = cand_noise[lo:hi].to(dev, torch.float32)
@@ -1026,10 +1140,13 @@ class FKSteering:
                 local = torch.empty((0,) + shape, device=dev)
             for r, (t_start, t_stop) in enumerate(segments):
                 last = t_stop == 0
+                if g is not None:
+                    g_segments.append(g.tolist())
                 if hi > lo:
                     local, x0 = denoise_fn.denoise_segment(local, lo, t_start=t_start, t_stop=t_stop, labels=labels,
                                                            seed=seed, cand_offset=r * ROUND_STRIDE, x0=True,
-                                                           cand_labels=_rows(rows, lo, hi))
+                                                           cand_labels=_rows(rows, lo, hi),
+                                                           cand_guidance=_rows(g, lo, hi))
                     judged = local if last else x0    # the last segment scores the finished, clipped samples
                     local_scores = _score_candidates(ver, judged.reshape(-1, *shape[1:]), B, denoise_fn, labels,
                                                      _rows(rows, lo, hi))
@@ -1051,6 +1168,8 @@ class FKSteering:
                     history['ancestors'][q].append(own)
                     history['ess'][q].append(ess_q[q])
                 local = states.index_select(0, anc[lo:hi].long())
+                if g is not None:
+                    g = g.index_select(0, anc.long())
             idx, best = _topk_device(scores, 1, n_seg=K)
             winners = idx.tolist()
         history['lineage'] = []
@@ -1065,6 +1184,10 @@ class FKSteering:
                 lineage.append(j)
             lineage.reverse()
             history['lineage'].append(lineage)
+        if guidance is not None:
+            history['lineage_guidance'] = [[g_segments[r][q * N + j] for r, j in enumerate(lin)]
+                                           for q, lin in enumerate(history['lineage'])]
+            self.last_guidance = [lg[-1] for lg in history['lineage_guidance']]
         history['unet_image_steps'] = steps * B * (2 if getattr(smp, "guided", False) else 1)
         self.nfes += steps
         return states.index_select(0, idx.long()), best.tolist(), history

@@ -23,6 +23,7 @@ if world > 1:
     dist.init_process_group("nccl", device_id=dev)
 
 from its_b200.Diffusion import GaussianDiffusionSampler, UNet
+from its_b200.DiffusionFreeGuidence import GaussianDiffusionSampler as GuidedSampler, UNet as CondUNet
 from its_b200.search import search_algorithm as S
 from its_b200.search import verifier as V
 
@@ -35,6 +36,15 @@ with torch.no_grad():            # the reference's zero-gain initialisers would 
             p.copy_(torch.randn_like(p) * (1.5 / (p[0].numel() ** 0.5)))
 smp = GaussianDiffusionSampler(net, 1e-4, 0.02, T).to(dev)
 smp.print_steps = False
+# the guided net, for searches over the guidance weight
+cnet = CondUNet(T=T, num_labels=10, ch=64, ch_mult=[1, 2], num_res_blocks=1, dropout=0.0).to(dev).eval()
+with torch.no_grad():
+    for p in cnet.parameters():
+        if p.dim() >= 2:
+            p.copy_(torch.randn_like(p) * (1.5 / (p[0].numel() ** 0.5)))
+gsmp = GuidedSampler(cnet, 1e-4, 0.02, T, w=1.8).to(dev)
+gsmp.print_steps = False
+glabels = torch.tensor([[1, 2], [3, 4], [5, 6]], dtype=torch.int64, device=dev)
 shape = (2, 3, 32, 32)
 den = S.make_denoise_fn(smp, max_images=64, seed=11)
 ver = V.OracleVerifier()
@@ -68,6 +78,24 @@ def run_all():
     rd = S.RandomSearch(n_candidates=13)
     bn, bs = rd.search(shape, den, dver.score, device=str(dev), verbose=False, seed=27)
     out["random_denoising_verifier"] = (bn.clone(), bs, rd.last_scores.clone())
+    # guided, mixed guidance weights per candidate / path / particle (ragged over 2/4/8 ranks); the chosen weights
+    # are compared with the scores
+    gden = S.make_denoise_fn(gsmp, max_images=64, seed=12)
+    grid = torch.tensor([[0.0, 1.8, 4.0, -0.5, 1.0], [4.0, 0.0, 1.8, 1.0, -0.5], [1.8, 1.8, 0.0, 4.0, 2.5]])
+    rg = S.RandomSearch(n_candidates=5)
+    bn, bs = rg.search_batch(shape, gden, ver.score, 3, labels=glabels, seed=28, device=str(dev), guidance=grid)
+    out["random_batch_guidance"] = (bn.clone(), bs, torch.cat([rg.last_scores.flatten().cpu(),
+                                                               torch.tensor(rg.last_guidance)]))
+    sg = S.SearchOverPaths(n_beams=3, n_children=3, start_step=3 * T // 4, delta_f=T // 8, delta_b=T // 4)
+    si, ss, sh = sg.search(shape, gden, ver.score, device=str(dev), seed=29, labels=glabels[0],
+                           guidance=grid[0, :3])
+    out["search_over_paths_guidance"] = (si.clone(), ss, torch.cat([torch.tensor(sh["scores"]).flatten(),
+                                                                    torch.tensor(sh["lineage_guidance"])]))
+    fg = S.FKSteering(n_particles=5, start_step=3 * T // 4, resample_interval=T // 4, lam=10.0)
+    fi, fs, fh = fg.search_batch(shape, gden, ver.score, 3, labels=glabels, seed=30, device=str(dev), guidance=grid)
+    out["fk_steering_batch_guidance"] = (fi.clone(), fs[0], torch.cat([torch.tensor(fh["scores"]).flatten(),
+                                                                       torch.tensor(fh["lineage_guidance"]).flatten(),
+                                                                       torch.tensor(fs)]))
     return out
 
 
