@@ -266,6 +266,9 @@ def sample_with_metrics_tracking(sampler, x_T: torch.Tensor, fid_calculator=None
 
 # -------------------------------------------------------------- search -------
 DENOISING_VERIFIERS = {"denoising": "likelihood", "diffusion_classifier": "class"}
+# the searches that answer K queries at once (search_batch) and search over the guidance weight, with the constructor
+# argument that counts the members of one query
+POPULATION_SEARCHES = {"random": "n_candidates", "search_over_paths": "n_beams", "fk_steering": "n_particles"}
 
 
 def make_verifier(name: str, sampler=None, *, n_levels: int = 8, seed: int = 0, max_images: int = 256,
@@ -334,61 +337,74 @@ def run_search(sampler, config: Dict[str, Any], device, *, labels=None, seed: Op
                         seed=int(sc.get("score_seed", 0)), max_images=int(sc.get("max_images", 256)),
                         ensemble=sc.get("ensemble"), ensemble_weights=sc.get("ensemble_weights"))
     K = int(sc.get("n_queries", 1))
-    if info is not None:
-        info["guidance"] = None
-    if K > 1:
-        *result, search = _run_batch(sampler, sc, algo, K, shape, ver, device, labels=labels, seed=seed, gw=gw)
-        if info is not None and gw is not None:
-            info["guidance"] = search.last_guidance
-        return tuple(result)
-    den = S.make_denoise_fn(sampler, labels, max_images=int(sc.get("max_images", 256)), seed=seed)
-    dev = str(device)
-    if algo == "search_over_paths":
-        search = S.SearchOverPaths(n_beams=int(sc.get("n_beams", 4)), n_children=int(sc.get("n_children", 4)),
-                                   start_step=int(sc.get("start_step", 800)), delta_f=int(sc.get("delta_f", 50)),
-                                   delta_b=int(sc.get("delta_b", 100)))
-        images, score, _ = search.search(shape, den, ver.score, device=dev, verbose=False, seed=seed,
-                                         **_grid(gw, search.n_beams))
-        best = S.philox_normal((1,) + shape, search.last_seed, search.last_index, S.TAG_X_T, torch.device(device))[0]
-        if info is not None and gw is not None:
-            info["guidance"] = search.last_guidance
-        return best, score, images
-    if algo == "fk_steering":
-        search = _fk_steering(sc)
-        images, score, _ = search.search(shape, den, ver.score, device=dev, seed=seed, **_grid(gw, search.n_particles))
-        best = S.philox_normal((1,) + shape, search.last_seed, search.last_index, S.TAG_X_T, torch.device(device))[0]
-        if info is not None and gw is not None:
-            info["guidance"] = search.last_guidance
-        return best, score, images
-    if algo == "random":
-        search = S.RandomSearch(n_candidates=int(sc.get("n_candidates", 4)))
-        best, score = search.search(shape, den, ver.score, device=dev, verbose=False, seed=seed,
-                                    **_grid(gw, search.n_candidates))
-    else:
-        x0 = S.philox_normal((1,) + shape, 0 if seed is None else seed, 0, S.TAG_X_T, torch.device(device))[0]
-        if algo == "zero_order":
-            search = S.ZeroOrderSearch(n_neighbors=int(sc.get("n_neighbors", 4)),
-                                       lambda_radius=float(sc.get("lambda_radius", 0.95)),
-                                       n_iterations=int(sc.get("n_iterations", 10)))
-            best, score, _ = search.search(x0, den, ver.score, device=dev, verbose=False, seed=seed)
-        elif algo == "path":
-            search = S.PathSearch(n_paths=int(sc.get("n_paths", 4)), injection_step=int(sc.get("injection_step", 400)),
-                                  noise_scale=float(sc.get("noise_scale", 0.1)))
-            best, score, _ = search.search(x0, den, ver.score, device=dev, verbose=False, seed=seed)
+    if K > 1 and algo not in POPULATION_SEARCHES:
+        raise ValueError(f"search.n_queries={K} needs search.algorithm in {list(POPULATION_SEARCHES)}, got {algo!r}")
+    search = _make_search(algo, sc)
+    dev = torch.device(device)
+    # a single search's labels [B] are the denoiser's own; K queries hand theirs ([K] or [K, B]) to search_batch
+    own_labels, query_labels = (labels, None) if K == 1 else (None, labels)
+    den = S.make_denoise_fn(sampler, own_labels, max_images=int(sc.get("max_images", 256)), seed=seed)
+    if algo in POPULATION_SEARCHES:
+        n = getattr(search, POPULATION_SEARCHES[algo])
+        out = search.search_batch(shape, den, ver.score, K, labels=query_labels, seed=seed, device=str(dev),
+                                  **_grid(gw, n))
+        if algo == "random":
+            best, scores = out
+            # each winner's images: its own trajectory (the global candidate id and weight it was scored under), so
+            # that the returned images are the ones that produced the returned score; NaN rows for queries without
+            # a winner (a single search keeps its one result as it is)
+            images = torch.full_like(best, float("nan")) if K > 1 else [None]
+            rows = None if query_labels is None else query_labels.to(dev, torch.int64).reshape(K, -1).expand(K, B)
+            for q, i in enumerate(search.last_index):
+                if i >= 0:
+                    g = None if gw is None else torch.tensor([search.last_guidance[q]], dtype=torch.float64)
+                    images[q] = den.denoise_candidates(best[q:q + 1], q * n + i, seed=search.last_seed,
+                                                       cand_labels=None if rows is None else rows[q:q + 1],
+                                                       cand_guidance=g)[0]
         else:
-            raise ValueError(f"search.algorithm {algo!r}: random | zero_order | path | search_over_paths | "
-                             "fk_steering")
-    # the images of the winner: its own trajectory (the Philox stream of the candidate id it was scored under),
-    # so that the returned images are the ones that produced the returned score
-    images = None
-    if best is not None:
-        g = getattr(search, "last_guidance", None) if gw is not None else None
-        images = den.denoise_candidates(best.unsqueeze(0), max(0, int(getattr(search, "last_index", 0))),
-                                        seed=getattr(search, "last_seed", seed),
-                                        cand_guidance=None if g is None else torch.tensor([g], dtype=torch.float64))[0]
-    if info is not None and gw is not None:
-        info["guidance"] = search.last_guidance
-    return best, score, images
+            images, scores, _ = out
+            # the winners' x_T, regenerated from their keys (their images are the ones the search finished)
+            x_T = [S.philox_normal((1,) + shape, search.last_seed, q * n + p, S.TAG_X_T, dev)[0]
+                   for q, p in enumerate(search.last_index)]
+            best = torch.stack(x_T) if K > 1 else x_T[0].unsqueeze(0)
+        chosen = None if gw is None else search.last_guidance
+        if K == 1:       # no query axis; a random search without a rankable candidate returns no noise and no images
+            best = best[0] if search.last_index[0] >= 0 else None
+            scores, images, chosen = scores[0], images[0], None if chosen is None else chosen[0]
+    else:                # zero_order / path: one query, searched from one x_T
+        x0 = S.philox_normal((1,) + shape, 0 if seed is None else seed, 0, S.TAG_X_T, dev)[0]
+        best, scores, _ = search.search(x0, den, ver.score, device=str(dev), verbose=False, seed=seed)
+        # the images of the winner: its own trajectory (the Philox stream of the candidate id it was scored under),
+        # so that the returned images are the ones that produced the returned score
+        images = den.denoise_candidates(best.unsqueeze(0), max(0, int(search.last_index)),
+                                        seed=getattr(search, "last_seed", seed))[0]
+        chosen = None
+    if info is not None:
+        info["guidance"] = chosen
+    return best, scores, images
+
+
+def _make_search(algo: str, sc: Dict[str, Any]):
+    """The search `search.algorithm` names, built from the keys of the `search:` block (see `run_search`)."""
+    from .search import search_algorithm as S
+    if algo == "random":
+        return S.RandomSearch(n_candidates=int(sc.get("n_candidates", 4)))
+    if algo == "zero_order":
+        return S.ZeroOrderSearch(n_neighbors=int(sc.get("n_neighbors", 4)),
+                                 lambda_radius=float(sc.get("lambda_radius", 0.95)),
+                                 n_iterations=int(sc.get("n_iterations", 10)))
+    if algo == "path":
+        return S.PathSearch(n_paths=int(sc.get("n_paths", 4)), injection_step=int(sc.get("injection_step", 400)),
+                            noise_scale=float(sc.get("noise_scale", 0.1)))
+    if algo == "search_over_paths":
+        return S.SearchOverPaths(n_beams=int(sc.get("n_beams", 4)), n_children=int(sc.get("n_children", 4)),
+                                 start_step=int(sc.get("start_step", 800)), delta_f=int(sc.get("delta_f", 50)),
+                                 delta_b=int(sc.get("delta_b", 100)))
+    if algo == "fk_steering":
+        return S.FKSteering(n_particles=int(sc.get("n_particles", 4)), start_step=int(sc.get("start_step", 800)),
+                            resample_interval=int(sc.get("resample_interval", 100)),
+                            lam=float(sc.get("fk_lambda", 10.0)))
+    raise ValueError(f"search.algorithm {algo!r}: random | zero_order | path | search_over_paths | fk_steering")
 
 
 def _guidance_weights(sc: Dict[str, Any], algo: str, sampler) -> Optional[List[float]]:
@@ -401,9 +417,9 @@ def _guidance_weights(sc: Dict[str, Any], algo: str, sampler) -> Optional[List[f
         raise ValueError(f"search.guidance_weights must be a non-empty list of numbers, got {gw!r}")
     if not all(math.isfinite(float(v)) for v in gw):
         raise ValueError(f"search.guidance_weights must be finite, got {gw!r}")
-    supported = ("random", "search_over_paths", "fk_steering")
-    if algo not in supported:
-        raise ValueError(f"search.guidance_weights needs search.algorithm in {list(supported)}, got {algo!r}")
+    if algo not in POPULATION_SEARCHES:
+        raise ValueError(f"search.guidance_weights needs search.algorithm in {list(POPULATION_SEARCHES)}, "
+                         f"got {algo!r}")
     if not getattr(sampler, "guided", False):
         raise ValueError("search.guidance_weights needs the guided net (num_labels and w in the config)")
     return [float(v) for v in gw]
@@ -414,52 +430,6 @@ def _grid(gw: Optional[List[float]], n: int) -> Dict[str, Any]:
     if gw is None:
         return {}
     return {"guidance": torch.tensor([gw[i % len(gw)] for i in range(int(n))], dtype=torch.float64)}
-
-
-def _run_batch(sampler, sc: Dict[str, Any], algo: str, K: int, shape, ver, device, *, labels=None,
-               seed: Optional[int] = None, gw: Optional[List[float]] = None):
-    """run_search for n_queries = K > 1: one `search_batch` over K queries; returns (best, scores, images, search)."""
-    from .search import search_algorithm as S
-    batched = ("random", "search_over_paths", "fk_steering")
-    if algo not in batched:
-        raise ValueError(f"search.n_queries={K} needs search.algorithm in {list(batched)}, got {algo!r}")
-    den = S.make_denoise_fn(sampler, max_images=int(sc.get("max_images", 256)), seed=seed)
-    dev = torch.device(device)
-    if algo == "search_over_paths":
-        search = S.SearchOverPaths(n_beams=int(sc.get("n_beams", 4)), n_children=int(sc.get("n_children", 4)),
-                                   start_step=int(sc.get("start_step", 800)), delta_f=int(sc.get("delta_f", 50)),
-                                   delta_b=int(sc.get("delta_b", 100)))
-        images, scores, _ = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev),
-                                                **_grid(gw, search.n_beams))
-        best = torch.stack([S.philox_normal((1,) + shape, search.last_seed, q * search.n_beams + p, S.TAG_X_T, dev)[0]
-                            for q, p in enumerate(search.last_index)])
-        return best, scores, images, search
-    if algo == "fk_steering":
-        search = _fk_steering(sc)
-        images, scores, _ = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev),
-                                                **_grid(gw, search.n_particles))
-        best = torch.stack([S.philox_normal((1,) + shape, search.last_seed, q * search.n_particles + p, S.TAG_X_T,
-                                            dev)[0] for q, p in enumerate(search.last_index)])
-        return best, scores, images, search
-    search = S.RandomSearch(n_candidates=int(sc.get("n_candidates", 4)))
-    best, scores = search.search_batch(shape, den, ver.score, K, labels=labels, seed=seed, device=str(dev),
-                                       **_grid(gw, search.n_candidates))
-    # each winner's images from its own trajectory (the global candidate id and weight it was scored under)
-    images = torch.full_like(best, float("nan"))
-    rows = None if labels is None else labels.to(dev, torch.int64).reshape(K, -1).expand(K, shape[0])
-    for q, i in enumerate(search.last_index):
-        if i >= 0:
-            g = None if gw is None else torch.tensor([search.last_guidance[q]], dtype=torch.float64)
-            images[q] = den.denoise_candidates(best[q:q + 1], q * search.n_candidates + i, seed=search.last_seed,
-                                               cand_labels=None if rows is None else rows[q:q + 1],
-                                               cand_guidance=g)[0]
-    return best, scores, images, search
-
-
-def _fk_steering(sc: Dict[str, Any]):
-    from .search import search_algorithm as S
-    return S.FKSteering(n_particles=int(sc.get("n_particles", 4)), start_step=int(sc.get("start_step", 800)),
-                        resample_interval=int(sc.get("resample_interval", 100)), lam=float(sc.get("fk_lambda", 10.0)))
 
 
 def save_image_grid(images: torch.Tensor, path: str, nrow: int = 8) -> str:

@@ -27,7 +27,10 @@ trajectories, re-noised and pruned by top-k on x0 predictions), in population mo
 Batched searches (not in the reference): `RandomSearch.search_batch`, `SearchOverPaths.search_batch` and
 `FKSteering.search_batch` run K
 independent queries, each with its own labels, as one candidate population and select every query's winner
-(or survivors) on the device with one segmented top-k.  `search` is the K = 1 case of the same code.
+(or survivors) on the device with one segmented top-k.  In population mode these classes have one path: `search`
+runs it with one query (its inputs gain a query axis of length 1) and `_unwrap` hands back query 0's results.  Every
+population search draws its initial x_T with `_x_T` and evaluates its members with `_evaluate` (denoise a segment,
+score, gather).
 
 FKSteering is not in the reference either: Feynman-Kac steering of Singhal et al. (a population of particles
 resampled by verifier potentials on their x0 predictions), in population mode only.
@@ -196,6 +199,15 @@ def _population_mode(denoise_fn, verifier_fn) -> Optional[Any]:
     return None
 
 
+def _require_population(denoise_fn, verifier_fn, search: str) -> Any:
+    """`_population_mode`'s kernel verifier, for the searches (and options) that have no callable mode."""
+    ver = _population_mode(denoise_fn, verifier_fn)
+    if ver is None:
+        raise ValueError(f"{search} needs an its_b200 SamplerDenoiser and a kernel verifier's .score "
+                         "(population mode)")
+    return ver
+
+
 # ---------------------------------------------------------------- utilities --
 def _dist():
     import torch.distributed as dist
@@ -341,15 +353,6 @@ def path_expand(x: torch.Tensor, parent: torch.Tensor, m: int, child0: int, n_ch
     return out
 
 
-def _score_candidates(ver, images: torch.Tensor, B: int, denoise: SamplerDenoiser, labels=None,
-                      cand_labels: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """ver.score_candidates over candidates of B images; a verifier with `uses_labels` also gets the flat labels
-    the denoiser fed the sampler for them."""
-    if not getattr(ver, "uses_labels", False):
-        return ver.score_candidates(images, B)
-    return ver.score_candidates(images, B, labels=denoise.image_labels(images.shape[0] // B, labels, cand_labels))
-
-
 def _no_scores(ver, device) -> torch.Tensor:
     """The score block of a rank that owns no candidates: [0] fp32, or [0, V] for a rank ensemble of V members (its
     gathered scores are the [n, V] member matrix)."""
@@ -373,23 +376,33 @@ def _refuse_ranks(verifier_fn, search: str, why: str) -> None:
                          "cannot be compared")
 
 
-def _score_population(cands_local: torch.Tensor, lo: int, n_total: int, denoise: SamplerDenoiser, ver,
-                      kwargs, t_start=None, seed=None, cand_labels=None, n_seg: int = 1,
-                      cand_guidance=None) -> torch.Tensor:
-    """Denoise + score this rank's block of candidates, return ALL n_total scores.  `seed`: the search's
-    shared seed, used for the step noise when the denoiser has none of its own (same on every rank).
-    `cand_labels`: label rows of this rank's candidates ([n_local, B]), else kwargs' `labels` for all.
-    `cand_guidance`: guidance weights of this rank's candidates ([n_local]), else the sampler's `w`.
-    A rank ensemble's member scores are combined over `n_seg` equal segments of the population."""
-    B = cands_local.shape[1] if cands_local.numel() else 1
-    if cands_local.shape[0] > 0:
-        imgs = denoise.denoise_candidates(cands_local, lo, labels=kwargs.get("labels"), t_start=t_start, seed=seed,
-                                          cand_labels=cand_labels, cand_guidance=cand_guidance)
-        local = _score_candidates(ver, imgs.reshape(-1, *imgs.shape[2:]), B, denoise, kwargs.get("labels"),
-                                  cand_labels)
+def _evaluate(states: torch.Tensor, lo: int, n_total: int, denoise: SamplerDenoiser, ver, *, t_start: int,
+              t_stop: int = 0, cand_offset: int = 0, x0: bool = False, seed: int, labels=None,
+              cand_labels: Optional[torch.Tensor] = None, cand_guidance: Optional[torch.Tensor] = None,
+              n_seg: int = 1) -> Tuple[torch.Tensor, torch.Tensor]:
+    """The evaluate step of every population search: denoise this rank's block of members (`states`
+    [n_local, B, ...] at step t_start, global ids lo, lo + 1, ...; step noise keyed as in `denoise_segment`) through
+    step t_stop, score it and gather the scores.  A segment ending at step 0 scores the finished, clipped samples,
+    any other the x0 predictions of step t_stop, which `x0` must then ask for (SearchOverPaths and FKSteering ask
+    in their last segment too, so that it replays the step graph of their other segments).  `seed`: the search's
+    shared seed, used for the step noise when the denoiser has none of its own (same on every rank).  `labels`:
+    shared labels of every member; `cand_labels`: label rows of this rank's members ([n_local, B]);
+    `cand_guidance`: their guidance weights ([n_local]), else the sampler's `w`.  A verifier with `uses_labels`
+    gets the flat labels the sampler was fed.  Returns (this rank's states after step t_stop, ALL n_total scores);
+    a rank ensemble's member scores are combined over `n_seg` equal segments of the population."""
+    if states.shape[0] > 0:
+        B = states.shape[1]
+        out, pred = denoise.denoise_segment(states, lo, t_start=t_start, t_stop=t_stop, cand_offset=cand_offset,
+                                            labels=labels, seed=seed, x0=x0, cand_labels=cand_labels,
+                                            cand_guidance=cand_guidance)
+        judged = (out if t_stop == 0 else pred).reshape(-1, *states.shape[2:])
+        if getattr(ver, "uses_labels", False):
+            local = ver.score_candidates(judged, B, labels=denoise.image_labels(states.shape[0], labels, cand_labels))
+        else:
+            local = ver.score_candidates(judged, B)
     else:
-        local = _no_scores(ver, cands_local.device)
-    return _combine(ver, _gather_scores(local, n_total), n_seg)
+        out, local = states, _no_scores(ver, states.device)
+    return out, _combine(ver, _gather_scores(local, n_total), n_seg)
 
 
 def _check_queries(n_queries: int, noise_shape: Sequence[int], labels: Optional[torch.Tensor]) -> int:
@@ -419,13 +432,10 @@ def _label_rows(labels: Optional[torch.Tensor], K: int, per_query: int, B: int, 
 
 def _guidance(guidance, K: int, N: int, denoise_fn, search: str, device, batch: bool) -> Optional[torch.Tensor]:
     """Per-member guidance weights, query-major float64 [K * N] on `device`, from `guidance` [N] (every query) or,
-    in `search_batch`, [K, N]; None stays None.  Checked on the host before any device work: population mode, the
-    guided sampler, the shape and finite values."""
+    in `search_batch`, [K, N]; None stays None.  Checked on the host before any device work (and after
+    `_require_population`): the guided sampler, the shape and finite values."""
     if guidance is None:
         return None
-    if not isinstance(denoise_fn, SamplerDenoiser):
-        raise ValueError(f"{search}: guidance weights need an its_b200 SamplerDenoiser and a kernel verifier's "
-                         ".score (population mode)")
     if not getattr(denoise_fn.sampler, "guided", False):
         raise ValueError(f"{search}: guidance weights need the guided sampler (DiffusionFreeGuidence)")
     g = torch.as_tensor(guidance, dtype=torch.float64).detach().cpu()
@@ -461,6 +471,65 @@ def _query(K: int, q: int) -> str:
     return f"query {q}, " if K > 1 else ""
 
 
+def _one(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
+    """A single search's input with the query axis of a one-query `search_batch` in front."""
+    return None if t is None else t.unsqueeze(0)
+
+
+def _unwrap(search, history: Optional[Dict[str, Any]] = None) -> Optional[Dict[str, Any]]:
+    """The results of a single search from those of a one-query population: query 0's `last_index`,
+    `last_guidance` and `last_scores`, and query 0's entry of every history list over the queries."""
+    for name in ("last_index", "last_guidance", "last_scores"):
+        value = getattr(search, name, None)
+        if value is not None:
+            setattr(search, name, value[0])
+    if history is None:
+        return None
+    whole = ("rounds", "segments", "unet_image_steps")      # entries of the whole population
+    return {k: v if k in whole else v[0] for k, v in history.items()}
+
+
+def _x_T(cand_noise: Optional[torch.Tensor], seed: int, lo: int, hi: int, shape: Sequence[int], dev) -> torch.Tensor:
+    """Initial x_T of members lo ... hi-1 ([hi - lo, *shape] fp32 on `dev`): rows of the injected `cand_noise`
+    ([n, *shape]), else Philox draws under TAG_X_T keyed by member id, so any member can be regenerated."""
+    if cand_noise is not None:
+        return cand_noise[lo:hi].to(dev, torch.float32)
+    if hi > lo:
+        return philox_normal((hi - lo,) + tuple(shape), seed, lo, TAG_X_T, dev)
+    return torch.empty((0,) + tuple(shape), device=dev)
+
+
+def _per_query(ids: List[int], K: int, size: int) -> List[List[int]]:
+    """Flat population ids ([K * k], query q's k at q*k ..., -1 for none) as K lists of ids within their query,
+    whose members are q*size ... q*size + size - 1."""
+    k = len(ids) // K
+    return [[i - q * size if i >= 0 else -1 for i in ids[q * k:(q + 1) * k]] for q in range(K)]
+
+
+def _lineage(last: int, parents: List[List[int]], m: int = 1) -> List[int]:
+    """A member's id in every round, the first to the last, from `last`, its id in the last round: member c of
+    round r + 1 descends from member parents[r][c // m] of round r."""
+    line = [last]
+    for ids in reversed(parents):
+        line.append(ids[line[-1] // m])
+    return line[::-1]
+
+
+def _finish(search, history: Dict[str, Any], lineages: List[List[int]], g_rounds: Optional[List[List[float]]],
+           size: int, steps: int, B: int, sampler) -> None:
+    """The per-query ends of SearchOverPaths and FKSteering.  With guidance (`g_rounds`: the weights of the
+    population's members in every round, host lists; None without), history 'lineage_guidance', each winner's
+    weight along its lineage (ids within queries of `size` members), and `last_guidance`; then
+    'unet_image_steps' and `nfes` from `steps` (UNet steps x members of B images)."""
+    search.last_guidance = None
+    if g_rounds is not None:
+        history['lineage_guidance'] = [[g_rounds[r][q * size + c] for r, c in enumerate(line)]
+                                       for q, line in enumerate(lineages)]
+        search.last_guidance = [lg[-1] for lg in history['lineage_guidance']]
+    history['unet_image_steps'] = steps * B * (2 if getattr(sampler, "guided", False) else 1)
+    search.nfes += steps
+
+
 # ------------------------------------------------------------ RandomSearch --
 class RandomSearch:
     """N random x_T candidates; keep the best verifier score (:18-87).  `search_batch` runs K such searches at once."""
@@ -474,35 +543,25 @@ class RandomSearch:
         cand_noise = kwargs.pop("candidate_noise", None)   # [n, *noise_shape]: injected candidates
         seed = kwargs.pop("seed", None)
         guidance = kwargs.pop("guidance", None)            # [n] per-candidate guidance weights
-        ver = _population_mode(denoise_fn, verifier_fn)
-        n = self.n_candidates
-        if guidance is not None and ver is None:
-            raise ValueError("RandomSearch: guidance weights need an its_b200 SamplerDenoiser and a kernel verifier's "
-                             ".score (population mode)")
-        guidance = _guidance(guidance, 1, n, denoise_fn, "RandomSearch", device, batch=False)
+        if guidance is not None or _population_mode(denoise_fn, verifier_fn) is not None:
+            best, vals = self._search(noise_shape, denoise_fn, verifier_fn, 1, labels=kwargs.get("labels"),
+                                      candidate_noise=_one(cand_noise), seed=seed, device=device, guidance=guidance,
+                                      batch=False)
+            _unwrap(self)
+            return (best[0], vals[0]) if self.last_index >= 0 else (None, float('-inf'))
         self.last_guidance = None
         if isinstance(denoise_fn, SamplerDenoiser):
             denoise_fn.reset_calls()
-        if ver is None:
-            best_noise, best_score = None, float('-inf')
-            for i in range(n):
-                noise = cand_noise[i].to(device) if cand_noise is not None else torch.randn(noise_shape, device=device)
-                with torch.no_grad():
-                    denoised = denoise_fn(noise, show_progress=(i == 0), **kwargs)
-                    self.nfes += 1
-                score = verifier_fn(denoised, **kwargs)
-                if score > best_score:
-                    best_score, best_noise = score, noise.clone()
-            return best_noise, best_score
-        best, vals, ids = self._population(noise_shape, denoise_fn, ver, 1, cand_noise=cand_noise, cand_labels=None,
-                                           seed=seed, device=device, kwargs=kwargs, guidance=guidance)
-        self.last_scores = self.last_scores[0]
-        if guidance is not None:
-            self.last_guidance = self.last_guidance[0]
-        if ids[0] < 0:
-            return None, float('-inf')
-        self.last_index = ids[0]
-        return best[0], vals[0]
+        best_noise, best_score = None, float('-inf')
+        for i in range(self.n_candidates):
+            noise = cand_noise[i].to(device) if cand_noise is not None else torch.randn(noise_shape, device=device)
+            with torch.no_grad():
+                denoised = denoise_fn(noise, show_progress=(i == 0), **kwargs)
+                self.nfes += 1
+            score = verifier_fn(denoised, **kwargs)
+            if score > best_score:
+                best_score, best_noise = score, noise.clone()
+        return best_noise, best_score
 
     def search_batch(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
                      n_queries: int, *, labels: Optional[torch.Tensor] = None,
@@ -519,58 +578,45 @@ class RandomSearch:
         Returns (best_noise [K, *noise_shape], best_scores); sets `last_scores` [K, N] (device), `last_index`
         (within-query indices), `last_guidance` (the winners' weights, None without `guidance`) and `last_seed`.
         A query with no rankable score gets a NaN row, -inf and -1 (and weight None)."""
-        K = _check_queries(n_queries, noise_shape, labels)
-        ver = _population_mode(denoise_fn, verifier_fn)
-        if ver is None:
-            raise ValueError("search_batch needs an its_b200 SamplerDenoiser and a kernel verifier's .score "
-                             "(population mode)")
-        N = self.n_candidates
-        _check_shape("candidate_noise", candidate_noise, (K, N, *noise_shape))
-        guidance = _guidance(guidance, K, N, denoise_fn, "RandomSearch", device, batch=True)
-        denoise_fn.reset_calls()
-        cand = None if candidate_noise is None else candidate_noise.reshape(K * N, *noise_shape)
-        best, vals, ids = self._population(noise_shape, denoise_fn, ver, K, cand_noise=cand,
-                                           cand_labels=_label_rows(labels, K, N, noise_shape[0], device),
-                                           seed=seed, device=device, kwargs={}, guidance=guidance)
-        self.last_index = ids
-        return best, vals
+        return self._search(noise_shape, denoise_fn, verifier_fn, n_queries, query_labels=labels,
+                            candidate_noise=candidate_noise, seed=seed, device=device, guidance=guidance)
 
-    def _population(self, noise_shape, denoise_fn: SamplerDenoiser, ver, K: int, *, cand_noise, cand_labels, seed,
-                    device, kwargs, guidance=None) -> Tuple[torch.Tensor, List[float], List[int]]:
-        """K queries of N candidates as one population sharded over the ranks; query q's candidate i is global
-        candidate q*N + i, at weight guidance[q*N + i] when given.  One segmented top-k (k = 1 per query) selects
-        every winner.  Sets `last_seed`, `last_guidance` and `last_scores` [K, N]; returns (winners [K, *noise_shape], scores, within-query indices), a NaN row, -inf
-        and -1 for a query with no rankable score."""
+    def _search(self, noise_shape, denoise_fn, verifier_fn, K: int, *, labels=None, query_labels=None,
+                candidate_noise=None, seed=None, device='cuda', guidance=None,
+                batch: bool = True) -> Tuple[torch.Tensor, List[float]]:
+        """`search_batch`, and `search` in population mode: K queries of N candidates as one population sharded over
+        the ranks, every winner selected by one segmented top-k (k = 1 per query).  `labels`: shared labels of every
+        candidate (a single search's); `query_labels`: one label row per query (`search_batch`'s `labels`); `batch`:
+        `guidance` may be [K, N].  Every argument is checked before any device work."""
+        K = _check_queries(K, noise_shape, query_labels)
+        ver = _require_population(denoise_fn, verifier_fn, "RandomSearch")
+        N, shape = self.n_candidates, tuple(noise_shape)
+        _check_shape("candidate_noise", candidate_noise, (K, N) + shape)
+        guidance = _guidance(guidance, K, N, denoise_fn, "RandomSearch", device, batch)
+        denoise_fn.reset_calls()
         dist, rank, world = _dist()
         dev = torch.device(device)
         seed = _shared_seed(seed, dev)
         self.last_seed = seed
-        N = self.n_candidates
         n = K * N
+        cand = None if candidate_noise is None else candidate_noise.reshape((n,) + shape)
+        rows = _label_rows(query_labels, K, N, shape[0], dev)
         lo, hi = _shard(n, rank, world)
-        if cand_noise is not None:
-            local = cand_noise[lo:hi].to(dev, torch.float32)
-        else:
-            local = philox_normal((hi - lo,) + tuple(noise_shape), seed, lo, TAG_X_T, dev) \
-                if hi > lo else torch.empty((0, *noise_shape), device=dev)
         with torch.no_grad():
-            scores = _score_population(local, lo, n, denoise_fn, ver, kwargs, seed=seed,
-                                       cand_labels=_rows(cand_labels, lo, hi), n_seg=K,
-                                       cand_guidance=_rows(guidance, lo, hi))
+            _, scores = _evaluate(_x_T(cand, seed, lo, hi, shape, dev), lo, n, denoise_fn, ver,
+                                  t_start=denoise_fn.sampler.T - 1, seed=seed, labels=labels,
+                                  cand_labels=_rows(rows, lo, hi), cand_guidance=_rows(guidance, lo, hi), n_seg=K)
         self.nfes += n
         self.last_scores = scores.view(K, N)
         idx, val = _topk_device(scores, 1, n_seg=K)
         ids, vals = idx.tolist(), val.tolist()
         self.last_guidance = _winner_guidance(guidance, ids)
-        best = torch.full((K, *noise_shape), float('nan'), dtype=torch.float32, device=dev)
+        self.last_index = [own[0] for own in _per_query(ids, K, N)]
+        best = torch.full((K,) + shape, float('nan'), dtype=torch.float32, device=dev)
         for q, i in enumerate(ids):
-            if i < 0:
-                continue
-            if cand_noise is not None:
-                best[q] = cand_noise[i].to(dev, torch.float32)
-            else:  # every rank regenerates the winner from its key: no broadcast needed
-                best[q] = philox_normal((1,) + tuple(noise_shape), seed, i, TAG_X_T, dev)[0]
-        return best, vals, [i - q * N if i >= 0 else -1 for q, i in enumerate(ids)]
+            if i >= 0:   # every rank regenerates the winner from its key (or its row): no broadcast needed
+                best[q] = _x_T(cand, seed, i, i + 1, shape, dev)[0]
+        return best, vals
 
     def reset_nfes(self):
         self.nfes = 0
@@ -639,7 +685,8 @@ class ZeroOrderSearch:
                 else:
                     local = current.new_empty((0, *current.shape))
                 with torch.no_grad():
-                    scores = _score_population(local, lo + it * K, K, denoise_fn, ver, kwargs, seed=seed)
+                    _, scores = _evaluate(local, lo + it * K, K, denoise_fn, ver, t_start=denoise_fn.sampler.T - 1,
+                                          seed=seed, labels=kwargs.get("labels"))
                 self.nfes += K
                 it_scores = [float(s) for s in scores.tolist()]
                 idx, it_best = argmax_first(scores)
@@ -687,7 +734,8 @@ class PathSearch:
         variations = kwargs.pop("variations", None)   # [n_paths, *shape] injected N(0,1) draws
         seed = kwargs.pop("seed", None)
         restart = bool(kwargs.pop("restart", False))
-        ver = _population_mode(denoise_fn, verifier_fn)
+        ver = _require_population(denoise_fn, verifier_fn, "PathSearch with restart=True") if restart else \
+            _population_mode(denoise_fn, verifier_fn)
         best_noise, best_score = initial_noise.clone(), float('-inf')
         history: Dict[str, Any] = {'scores': [], 'injection_points': []}
         P = self.n_paths
@@ -695,8 +743,6 @@ class PathSearch:
         if isinstance(denoise_fn, SamplerDenoiser):
             denoise_fn.reset_calls()
         if ver is None:
-            if restart:
-                raise ValueError("restart=True needs an its_b200 SamplerDenoiser (population mode)")
             for p in range(P):
                 var = variations[p].to(initial_noise) if variations is not None else torch.randn_like(initial_noise)
                 perturbed = initial_noise + var * self.noise_scale
@@ -715,11 +761,10 @@ class PathSearch:
         lo, hi = _shard(P, rank, world)
         B = initial_noise.shape[0]
         base = initial_noise
-        t_start = None
+        T = denoise_fn.sampler.T
+        t_start = T - 1
         if restart:
             # pivot trajectory T-1 .. injection_step (exclusive) on every rank, unclipped
-            smp = denoise_fn.sampler
-            T = smp.T
             if not (0 < self.injection_step < T):
                 raise ValueError("injection_step must lie in (0, T)")
             base = denoise_fn.denoise_candidates(initial_noise.unsqueeze(0), 0, labels=kwargs.get("labels"), seed=seed,
@@ -735,7 +780,8 @@ class PathSearch:
                                  base=base.reshape(-1), scale=self.noise_scale)
 
         with torch.no_grad():
-            scores = _score_population(perturbed(lo, hi), lo, P, denoise_fn, ver, kwargs, t_start=t_start, seed=seed)
+            _, scores = _evaluate(perturbed(lo, hi), lo, P, denoise_fn, ver, t_start=t_start, seed=seed,
+                                  labels=kwargs.get("labels"))
         self.nfes += P
         history['scores'] = [float(s) for s in scores.tolist()]
         history['injection_points'] = [self.injection_step] * P
@@ -809,24 +855,13 @@ class SearchOverPaths:
     def search(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
                device: str = 'cuda', verbose: Optional[bool] = None,
                **kwargs) -> Tuple[torch.Tensor, float, Dict[str, Any]]:
-        cand_noise = kwargs.pop("candidate_noise", None)
         fwd_noise = kwargs.pop("forward_noise", None)
-        seed = kwargs.pop("seed", None)
-        guidance = kwargs.pop("guidance", None)
-        ver, rounds = self._schedule(denoise_fn, verifier_fn)
-        guidance = _guidance(guidance, 1, int(self.n_beams), denoise_fn, "SearchOverPaths", device, batch=False)
-        if fwd_noise is not None and len(fwd_noise) < len(rounds):
-            raise ValueError(f"forward_noise has {len(fwd_noise)} rounds, the schedule {len(rounds)}")
-        images, best, h = self._population(tuple(noise_shape), denoise_fn, ver, rounds, 1, labels=kwargs.get("labels"),
-                                           query_labels=None, cand_noise=cand_noise, fwd_noise=fwd_noise, seed=seed,
-                                           device=device, guidance=guidance)
-        history = {'rounds': h['rounds'], 'scores': h['scores'][0], 'survivors': h['survivors'][0],
-                   'lineage': h['lineage'][0], 'unet_image_steps': h['unet_image_steps']}
-        if guidance is not None:
-            history['lineage_guidance'] = h['lineage_guidance'][0]
-            self.last_guidance = self.last_guidance[0]
-        self.last_index = history['lineage']['path']
-        return images[0], best[0], history
+        images, best, history = self._search(
+            noise_shape, denoise_fn, verifier_fn, 1, labels=kwargs.get("labels"),
+            candidate_noise=_one(kwargs.pop("candidate_noise", None)),
+            forward_noise=None if fwd_noise is None else [_one(f) for f in fwd_noise], seed=kwargs.pop("seed", None),
+            device=device, guidance=kwargs.pop("guidance", None), batch=False)
+        return images[0], best[0], _unwrap(self, history)
 
     def search_batch(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
                      n_queries: int, *, labels: Optional[torch.Tensor] = None,
@@ -848,49 +883,34 @@ class SearchOverPaths:
         within-query ids; 'unet_image_steps' is the whole batch's.  `last_index` is the list of the winners' initial
         path ids, `last_guidance` of their weights.  A query whose children cannot be ranked raises ValueError naming
         the query and the round."""
-        K = _check_queries(n_queries, noise_shape, labels)
-        ver, rounds = self._schedule(denoise_fn, verifier_fn)
-        shape = tuple(noise_shape)
-        N, NM = int(self.n_beams), int(self.n_beams) * int(self.n_children)
+        return self._search(noise_shape, denoise_fn, verifier_fn, n_queries, query_labels=labels,
+                            candidate_noise=candidate_noise, forward_noise=forward_noise, seed=seed, device=device,
+                            guidance=guidance)
+
+    def _search(self, noise_shape, denoise_fn, verifier_fn, K: int, *, labels=None, query_labels=None,
+                candidate_noise=None, forward_noise=None, seed=None, device='cuda', guidance=None,
+                batch: bool = True) -> Tuple[torch.Tensor, List[float], Dict[str, Any]]:
+        """`search_batch`, and `search` with one query: K queries as one population sharded over the ranks.
+        `labels`: shared labels of every member (a single search's); `query_labels`: one label row per query
+        (`search_batch`'s `labels`); `guidance` ([N], or with `batch` [K, N]): the initial paths' weights, which
+        every child inherits from its parent (re-indexed by the same device survivor ids the expansion reads).
+        Every argument, and the parameters against sampler.T, is checked before any device work."""
+        K = _check_queries(K, noise_shape, query_labels)
+        ver = _require_population(denoise_fn, verifier_fn, "SearchOverPaths")
+        N, M = int(self.n_beams), int(self.n_children)
+        if N < 1 or M < 1:
+            raise ValueError(f"n_beams={N} and n_children={M} must be >= 1")
+        smp = denoise_fn.sampler
+        T = smp.T
+        rounds = path_rounds(T, self.start_step, self.delta_f, self.delta_b)
+        NM, shape = N * M, tuple(noise_shape)
         _check_shape("candidate_noise", candidate_noise, (K, N) + shape)
-        guidance = _guidance(guidance, K, N, denoise_fn, "SearchOverPaths", device, batch=True)
-        fwd = None
+        guidance = _guidance(guidance, K, N, denoise_fn, "SearchOverPaths", device, batch)
         if forward_noise is not None:
             if len(forward_noise) < len(rounds):
                 raise ValueError(f"forward_noise has {len(forward_noise)} rounds, the schedule {len(rounds)}")
             for r in range(len(rounds)):
                 _check_shape(f"forward_noise[{r}]", forward_noise[r], (K, NM) + shape)
-            fwd = [forward_noise[r].reshape((K * NM,) + shape) for r in range(len(rounds))]
-        images, best, history = self._population(
-            shape, denoise_fn, ver, rounds, K, labels=None, query_labels=labels,
-            cand_noise=None if candidate_noise is None else candidate_noise.reshape((K * N,) + shape),
-            fwd_noise=fwd, seed=seed, device=device, guidance=guidance)
-        self.last_index = [lin['path'] for lin in history['lineage']]
-        return images, best, history
-
-    def _schedule(self, denoise_fn, verifier_fn) -> Tuple[Any, List[Tuple[int, int, int]]]:
-        """(kernel verifier, round schedule) after checking the mode and the parameters against sampler.T."""
-        ver = _population_mode(denoise_fn, verifier_fn)
-        if ver is None:
-            raise ValueError("SearchOverPaths needs an its_b200 SamplerDenoiser and a kernel verifier's .score "
-                             "(population mode)")
-        N, M = int(self.n_beams), int(self.n_children)
-        if N < 1 or M < 1:
-            raise ValueError(f"n_beams={N} and n_children={M} must be >= 1")
-        return ver, path_rounds(denoise_fn.sampler.T, self.start_step, self.delta_f, self.delta_b)
-
-    def _population(self, shape: Tuple[int, ...], denoise_fn: SamplerDenoiser, ver, rounds, K: int, *, labels,
-                    query_labels, cand_noise, fwd_noise, seed, device, guidance=None):
-        """K queries as one population sharded over the ranks (query q's path i is global path q*N + i, its child c
-        global child q*N*M + c).  `labels`: shared labels of every member; `query_labels` ([K] or [K, B]): one
-        label row per query; `guidance` ([K*N] or None): the initial paths' weights, which every child inherits
-        from its parent (re-indexed by the same device survivor ids the expansion reads).  Sets `last_guidance`.
-        Returns (best images [K, *shape], best scores, history with per-query 'scores',
-        'survivors' and 'lineage' in within-query ids)."""
-        N, M = int(self.n_beams), int(self.n_children)
-        NM = N * M
-        smp = denoise_fn.sampler
-        T = smp.T
         dist, rank, world = _dist()
         dev = torch.device(device)
         seed = _shared_seed(seed, dev)
@@ -901,19 +921,15 @@ class SearchOverPaths:
         path_labels, child_labels = _label_rows(query_labels, K, N, B, dev), _label_rows(query_labels, K, NM, B, dev)
         history: Dict[str, Any] = {'rounds': [], 'scores': [[] for _ in range(K)],
                                    'survivors': [[] for _ in range(K)]}
-        self.last_guidance = None
-        g_rows, g_rounds = guidance, []               # weight of each row of `parents`; children's weights per round
+        g_rows = guidance                             # weight of each row of `parents`
+        g_rounds = None if guidance is None else []   # children's weights per round
         steps = 0                                     # UNet steps x candidates
         with torch.no_grad():
             # stage 0: K*N paths from x_T down to the states at step start_step
             n_p = K * N
             lo, hi = _shard(n_p, rank, world)
-            if cand_noise is not None:
-                local = cand_noise[lo:hi].to(dev, torch.float32)
-            elif hi > lo:
-                local = philox_normal((hi - lo,) + shape, seed, lo, TAG_X_T, dev)
-            else:
-                local = torch.empty((0,) + shape, device=dev)
+            cand = None if candidate_noise is None else candidate_noise.reshape((n_p,) + shape)
+            local = _x_T(cand, seed, lo, hi, shape, dev)
             s0 = rounds[0][0]
             if s0 < T - 1 and hi > lo:
                 local = denoise_fn.denoise_candidates(local, lo, labels=labels, seed=seed, t_stop=s0 + 1,
@@ -931,32 +947,24 @@ class SearchOverPaths:
                     g_rows = g_rows.index_select(0, parent_idx.long()).repeat_interleave(M)
                     g_rounds.append(g_rows.tolist())
                 if hi > lo:
-                    z = None if fwd_noise is None else fwd_noise[r][lo:hi]
+                    z = None if forward_noise is None else forward_noise[r].reshape((n_c,) + shape)[lo:hi]
                     kids = path_expand(parents.reshape(parents.shape[0], -1), parent_idx, M, lo, hi - lo, a, b,
                                        z=None if z is None else z.reshape(hi - lo, -1), seed=seed,
                                        cand_id0=(r + 1) * ROUND_STRIDE, tag=TAG_FORWARD).view((hi - lo,) + shape)
-                    states, x0 = denoise_fn.denoise_segment(kids, lo, t_start=sp, t_stop=e, labels=labels, seed=seed,
-                                                            cand_offset=(r + 1) * ROUND_STRIDE, x0=True,
-                                                            cand_labels=_rows(child_labels, lo, hi),
-                                                            cand_guidance=_rows(g_rows, lo, hi))
-                    judged = x0 if e > 0 else states   # the last round scores the finished, clipped samples
-                    local_scores = _score_candidates(ver, judged.reshape(-1, *shape[1:]), B, denoise_fn, labels,
-                                                     _rows(child_labels, lo, hi))
                 else:
-                    states = torch.empty((0,) + shape, device=dev)
-                    local_scores = _no_scores(ver, dev)
+                    kids = torch.empty((0,) + shape, device=dev)
+                states, scores = _evaluate(kids, lo, n_c, denoise_fn, ver, t_start=sp, t_stop=e,
+                                           cand_offset=(r + 1) * ROUND_STRIDE, x0=True, seed=seed, labels=labels,
+                                           cand_labels=_rows(child_labels, lo, hi),
+                                           cand_guidance=_rows(g_rows, lo, hi), n_seg=K)
                 steps += n_c * (sp - e + 1)
-                scores = _combine(ver, _gather_scores(local_scores, n_c), K)
                 history['rounds'].append((s, sp, e))
                 for q, row in enumerate(scores.view(K, NM).tolist()):
                     history['scores'][q].append(row)
                 parents = _gather_states(states.contiguous(), n_c)
                 # survivors (k = N per query) or the winner (k = 1): flat child ids, passed on as parents as they are
                 parent_idx, best = _topk_device(scores, N if e > 0 else 1, n_seg=K)
-                ids = parent_idx.tolist()
-                k = len(ids) // K
-                for q in range(K):
-                    own = [i - q * NM if i >= 0 else -1 for i in ids[q * k:(q + 1) * k]]
+                for q, own in enumerate(_per_query(parent_idx.tolist(), K, NM)):
                     if min(own) >= 0:
                         history['survivors'][q].append(own)
                     elif e > 0:
@@ -966,21 +974,10 @@ class SearchOverPaths:
                         raise ValueError(f"{_query(K, q)}last round: none of the {NM} finished samples has a score "
                                          "that can be ranked")
         # lineage of each winner: child id in every round, back to its initial path
-        history['lineage'] = []
-        for surv in history['survivors']:
-            child = surv[-1][0]
-            lineage = [child]
-            for ids in reversed(surv[:-1]):
-                child = ids[child // M]
-                lineage.append(child)
-            lineage.reverse()
-            history['lineage'].append({'path': lineage[0] // M, 'children': lineage})
-        if guidance is not None:
-            history['lineage_guidance'] = [[g_rounds[r][q * NM + c] for r, c in enumerate(lin['children'])]
-                                           for q, lin in enumerate(history['lineage'])]
-            self.last_guidance = [lg[-1] for lg in history['lineage_guidance']]
-        history['unet_image_steps'] = steps * B * (2 if getattr(smp, "guided", False) else 1)
-        self.nfes += steps
+        lineages = [_lineage(surv[-1][0], surv[:-1], M) for surv in history['survivors']]
+        history['lineage'] = [{'path': line[0] // M, 'children': line} for line in lineages]
+        self.last_index = [lin['path'] for lin in history['lineage']]
+        _finish(self, history, lineages, g_rounds, NM, steps, B, smp)
         return parents[parent_idx.long()].clone(), best.tolist(), history
 
     def reset_nfes(self):
@@ -1042,23 +1039,11 @@ class FKSteering:
     def search(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
                device: str = 'cuda', verbose: Optional[bool] = None,
                **kwargs) -> Tuple[torch.Tensor, float, Dict[str, Any]]:
-        cand_noise = kwargs.pop("candidate_noise", None)
-        seed = kwargs.pop("seed", None)
-        guidance = kwargs.pop("guidance", None)
-        shape = tuple(noise_shape)
-        ver, segments = self._schedule(denoise_fn, verifier_fn)
-        _check_shape("candidate_noise", cand_noise, (int(self.n_particles),) + shape)
-        guidance = _guidance(guidance, 1, int(self.n_particles), denoise_fn, "FKSteering", device, batch=False)
-        images, best, h = self._population(shape, denoise_fn, ver, segments, 1, labels=kwargs.get("labels"),
-                                           query_labels=None, cand_noise=cand_noise, seed=seed, device=device,
-                                           guidance=guidance)
-        history = {'segments': h['segments'], 'scores': h['scores'][0], 'ancestors': h['ancestors'][0],
-                   'ess': h['ess'][0], 'lineage': h['lineage'][0], 'unet_image_steps': h['unet_image_steps']}
-        if guidance is not None:
-            history['lineage_guidance'] = h['lineage_guidance'][0]
-            self.last_guidance = self.last_guidance[0]
-        self.last_index = history['lineage'][0]
-        return images[0], best[0], history
+        images, best, history = self._search(
+            noise_shape, denoise_fn, verifier_fn, 1, labels=kwargs.get("labels"),
+            candidate_noise=_one(kwargs.pop("candidate_noise", None)), seed=kwargs.pop("seed", None), device=device,
+            guidance=kwargs.pop("guidance", None), batch=False)
+        return images[0], best[0], _unwrap(self, history)
 
     def search_batch(self, noise_shape: Tuple[int, ...], denoise_fn: Callable, verifier_fn: Callable,
                      n_queries: int, *, labels: Optional[torch.Tensor] = None,
@@ -1080,43 +1065,32 @@ class FKSteering:
         within-query ids; 'unet_image_steps' is the whole batch's.  `last_index` is the list of the winners' x_T ids,
         `last_guidance` of their weights.  A query none of whose particles can
         be weighted raises ValueError naming the query and the resampling round."""
-        K = _check_queries(n_queries, noise_shape, labels)
-        shape = tuple(noise_shape)
-        ver, segments = self._schedule(denoise_fn, verifier_fn)
-        N = int(self.n_particles)
-        _check_shape("candidate_noise", candidate_noise, (K, N) + shape)
-        guidance = _guidance(guidance, K, N, denoise_fn, "FKSteering", device, batch=True)
-        images, best, history = self._population(
-            shape, denoise_fn, ver, segments, K, labels=None, query_labels=labels,
-            cand_noise=None if candidate_noise is None else candidate_noise.reshape((K * N,) + shape),
-            seed=seed, device=device, guidance=guidance)
-        self.last_index = [lin[0] for lin in history['lineage']]
-        return images, best, history
+        return self._search(noise_shape, denoise_fn, verifier_fn, n_queries, query_labels=labels,
+                            candidate_noise=candidate_noise, seed=seed, device=device, guidance=guidance)
 
-    def _schedule(self, denoise_fn, verifier_fn) -> Tuple[Any, List[Tuple[int, int]]]:
-        """(kernel verifier, segment schedule) after checking the mode and the parameters against sampler.T."""
+    def _search(self, noise_shape, denoise_fn, verifier_fn, K: int, *, labels=None, query_labels=None,
+                candidate_noise=None, seed=None, device='cuda', guidance=None,
+                batch: bool = True) -> Tuple[torch.Tensor, List[float], Dict[str, Any]]:
+        """`search_batch`, and `search` with one query: K queries of N particles as one population sharded over the
+        ranks.  `labels`: shared labels of every particle (a single search's); `query_labels`: one label row per
+        query (`search_batch`'s `labels`); `guidance` ([N], or with `batch` [K, N]): the particles' weights, which
+        follow their ancestors (`index_select` with the same device ancestor ids as the states).  Every argument,
+        and the parameters against sampler.T, is checked before any device work."""
+        K = _check_queries(K, noise_shape, query_labels)
         _refuse_ranks(verifier_fn, "FKSteering", "it weights particles by the change of their reward between "
                       "resamplings")
-        ver = _population_mode(denoise_fn, verifier_fn)
-        if ver is None:
-            raise ValueError("FKSteering needs an its_b200 SamplerDenoiser and a kernel verifier's .score "
-                             "(population mode)")
-        if int(self.n_particles) < 1:
+        ver = _require_population(denoise_fn, verifier_fn, "FKSteering")
+        N = int(self.n_particles)
+        if N < 1:
             raise ValueError(f"n_particles={self.n_particles} must be >= 1")
         if not (math.isfinite(float(self.lam)) and float(self.lam) >= 0.0):
             raise ValueError(f"lam={self.lam} must be finite and >= 0")
-        return ver, fk_segments(denoise_fn.sampler.T, self.start_step, self.resample_interval)
-
-    def _population(self, shape: Tuple[int, ...], denoise_fn: SamplerDenoiser, ver, segments, K: int, *, labels,
-                    query_labels, cand_noise, seed, device, guidance=None):
-        """K queries of N particles as one population sharded over the ranks (query q's particle j is global
-        particle q*N + j).  `labels`: shared labels of every particle; `query_labels` ([K] or [K, B]): one label row
-        per query; `guidance` ([K*N] or None): the particles' weights, which follow their ancestors (`index_select`
-        with the same device ancestor ids as the states).  Sets `last_guidance`.  Returns (best images [K, *shape], best scores, history with per-query 'scores', 'ancestors',
-        'ess' and 'lineage' in within-query ids)."""
-        N = int(self.n_particles)
-        n = K * N
         smp = denoise_fn.sampler
+        segments = fk_segments(smp.T, self.start_step, self.resample_interval)
+        shape = tuple(noise_shape)
+        _check_shape("candidate_noise", candidate_noise, (K, N) + shape)
+        guidance = _guidance(guidance, K, N, denoise_fn, "FKSteering", device, batch)
+        n = K * N
         dist, rank, world = _dist()
         dev = torch.device(device)
         seed = _shared_seed(seed, dev)
@@ -1129,38 +1103,24 @@ class FKSteering:
                                    'ancestors': [[] for _ in range(K)], 'ess': [[] for _ in range(K)]}
         steps = 0                                     # UNet steps x particles
         carried = None
-        g, g_segments = guidance, []                  # particle weights now, and in every segment
-        self.last_guidance = None
+        g = guidance                                  # particle weights now,
+        g_segments = None if guidance is None else []   # and in every segment
         with torch.no_grad():
-            if cand_noise is not None:
-                local = cand_noise[lo:hi].to(dev, torch.float32)
-            elif hi > lo:
-                local = philox_normal((hi - lo,) + shape, seed, lo, TAG_X_T, dev)
-            else:
-                local = torch.empty((0,) + shape, device=dev)
+            cand = None if candidate_noise is None else candidate_noise.reshape((n,) + shape)
+            local = _x_T(cand, seed, lo, hi, shape, dev)
             for r, (t_start, t_stop) in enumerate(segments):
-                last = t_stop == 0
                 if g is not None:
                     g_segments.append(g.tolist())
-                if hi > lo:
-                    local, x0 = denoise_fn.denoise_segment(local, lo, t_start=t_start, t_stop=t_stop, labels=labels,
-                                                           seed=seed, cand_offset=r * ROUND_STRIDE, x0=True,
-                                                           cand_labels=_rows(rows, lo, hi),
-                                                           cand_guidance=_rows(g, lo, hi))
-                    judged = local if last else x0    # the last segment scores the finished, clipped samples
-                    local_scores = _score_candidates(ver, judged.reshape(-1, *shape[1:]), B, denoise_fn, labels,
-                                                     _rows(rows, lo, hi))
-                else:
-                    local_scores = torch.empty(0, dtype=torch.float32, device=dev)
+                local, scores = _evaluate(local, lo, n, denoise_fn, ver, t_start=t_start, t_stop=t_stop,
+                                          cand_offset=r * ROUND_STRIDE, x0=True, seed=seed, labels=labels,
+                                          cand_labels=_rows(rows, lo, hi), cand_guidance=_rows(g, lo, hi), n_seg=K)
                 steps += n * (t_start - t_stop + 1)
-                scores = _gather_scores(local_scores, n)
                 states = _gather_states(local.contiguous(), n)
-                if last:
+                if t_stop == 0:
                     break
                 anc, carried, ess = resample_systematic(scores, carried, self.lam, K, seed, r)
-                ids, vals, ess_q = anc.tolist(), scores.view(K, N).tolist(), ess.tolist()
-                for q in range(K):
-                    own = [i - q * N if i >= 0 else -1 for i in ids[q * N:(q + 1) * N]]
+                ids, vals, ess_q = _per_query(anc.tolist(), K, N), scores.view(K, N).tolist(), ess.tolist()
+                for q, own in enumerate(ids):
                     if own[0] < 0:
                         raise ValueError(f"{_query(K, q)}resampling round {r}: none of the {N} particles has a "
                                          "finite score to weight")
@@ -1171,25 +1131,15 @@ class FKSteering:
                 if g is not None:
                     g = g.index_select(0, anc.long())
             idx, best = _topk_device(scores, 1, n_seg=K)
-            winners = idx.tolist()
+            winners = _per_query(idx.tolist(), K, N)
         history['lineage'] = []
-        for q, i in enumerate(winners):
-            if i < 0:
+        for q, own in enumerate(winners):
+            if own[0] < 0:
                 raise ValueError(f"{_query(K, q)}last segment: none of the {N} finished samples has a score that can "
                                  "be ranked")
-            j = i - q * N
-            lineage = [j]
-            for own in reversed(history['ancestors'][q]):
-                j = own[j]
-                lineage.append(j)
-            lineage.reverse()
-            history['lineage'].append(lineage)
-        if guidance is not None:
-            history['lineage_guidance'] = [[g_segments[r][q * N + j] for r, j in enumerate(lin)]
-                                           for q, lin in enumerate(history['lineage'])]
-            self.last_guidance = [lg[-1] for lg in history['lineage_guidance']]
-        history['unet_image_steps'] = steps * B * (2 if getattr(smp, "guided", False) else 1)
-        self.nfes += steps
+            history['lineage'].append(_lineage(own[0], history['ancestors'][q]))
+        self.last_index = [line[0] for line in history['lineage']]
+        _finish(self, history, history['lineage'], g_segments, N, steps, B, smp)
         return states.index_select(0, idx.long()), best.tolist(), history
 
     def reset_nfes(self):

@@ -323,6 +323,8 @@ def test_unrankable_query(cuda_dev):
     assert bad.last_index[1] == -1 and b_scores[1] == -math.inf and torch.isnan(b_best[1]).all()
     for q in (0, 2):
         assert bad.last_index[q] == rs.last_index[q] and b_scores[q] == scores[q] and torch.equal(b_best[q], best[q])
+    assert bad.search(shape, _den(smp, cuda_dev), _nan_query_verifier(4, 0).score, device=str(cuda_dev),
+                      seed=12) == (None, -math.inf) and bad.last_index == -1
     NM = cfg["n_beams"] * cfg["n_children"]
     with pytest.raises(ValueError, match="query 2, round 0: only 0 of %d children" % NM):
         _sop(cfg).search_batch(shape, _den(smp, cuda_dev), _nan_query_verifier(NM, 2).score, 3, seed=12, device=str(cuda_dev))
